@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA engine
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU arithmetic (oracle port)
+  python bench.py ... --dump-outputs DIR                   # also save the last timed step's outputs as .npy
 
 A "step" is one dspb_process call over one batch of synthetic input: C channels x n samples per channel
 (n = blocks_per_step device blocks), state carried across steps.  `value` is measured with inputs and outputs
@@ -63,7 +64,13 @@ def parse_args():
     ap.add_argument("--no-scan-side", action="store_true", help="skip the iir_mode=1 side measurement")
     ap.add_argument("--no-weak", action="store_true", help="skip the weak-scaling side measurement of a strong N>1 run")
     ap.add_argument("--gather", action="store_true", help="also time an NCCL gather of the outputs to rank 0")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's outputs of the last timed step as DIR/output<i>.npy (float32), to compare two builds "
+                         "(bench_outputs/ is ignored by git)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the CUDA engine's outputs: it needs --impl b200")
+    return args
 
 
 DEFAULT_CHANNELS = {"config1": 2, "config2": 256, "config2_one_pole": 256, "config3": 1024, "config4": 4096, "config5": 8192, "target": 4096}
@@ -319,6 +326,25 @@ def parity_check(args, spec, eng, x_dev, n, ch_offset):
             "pass": bool(exact or (rel <= 1e-5 and dbfs <= -100.0)), "tolerance": "1e-5 peak-relative and -100 dBFS rms (north_star)"}
 
 
+DUMP_BYTES = 32 * 2**20
+
+
+def dump_outputs(path, ys):
+    """Writes the output arrays `ys` ([C, n] device tensors) as path/output<i>.npy.  When they exceed DUMP_BYTES in all,
+    a fixed seeded sample of whole channels (the same rows of every output) is written instead, cut to fewer samples only
+    if a single channel per output is already too large.  The bench input is seeded too, so equal arguments give files
+    that two builds can be compared on."""
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    C, n = ys[0].shape
+    rows = max(1, min(C, DUMP_BYTES // (4 * n * len(ys))))
+    cols = min(n, DUMP_BYTES // (4 * rows * len(ys)))
+    sel = torch.from_numpy(np.sort(np.random.default_rng(0).choice(C, rows, replace=False))).to(ys[0].device)
+    for i, y in enumerate(ys):
+        np.save(os.path.join(path, f"output{i}.npy"), y.index_select(0, sel)[:, :cols].cpu().numpy())
+
+
 def timed_steps(eng, x_dev, y_dev, n, steps, stream, barrier):
     import torch
 
@@ -408,6 +434,8 @@ def main():
     eng.profile(False)
     plan = eng.plan_steps()
     (ms,) = allmax([ms])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, y_dev)   # before any later section overwrites y_dev
 
     # ---- sustained: >= sustain_seconds of back-to-back steps (the 20-step figure is a burst at boost clocks) -------
     sustained = None

@@ -1,8 +1,14 @@
-"""bench.py contract checks that need no GPU: the reference arm (the oracle port on the host cores) runs here."""
+"""bench.py contract checks: the reference arm (the oracle port on the host cores) needs no GPU; --dump-outputs does."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
+
+from dsp_stuff_b200 import signals as S
+from tests.util import assert_bit_exact
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -41,3 +47,24 @@ def test_strong_scaling_shards_are_what_both_arms_report():
     assert d["config"]["channels"] == 4096 and d["config"]["channels_per_gpu"] == 512 and d["scaling"] == "strong"
     d = run_bench("--impl", "reference", "--gpus", "8", "--steps", "1", "--warmup", "0", "--scaling", "weak", env={"RANK": "0", "WORLD_SIZE": "8"})
     assert d["config"]["channels"] == 8 * 4096 and d["config"]["channels_per_gpu"] == 4096 and d["scaling"] == "weak"
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_last_timed_step(tmp_path):
+    """--steps K --warmup 3: the dumped array is the engine's output of its 3 + K-th call on the seeded bench input."""
+    from dsp_stuff_b200.engine import Engine
+
+    C, n, steps = 8, 2048, 4
+    d = run_bench("--workload", "config3", "--channels", str(C), "--blocks-per-step", "2", "--steps", str(steps), "--warmup", "3",
+                  "--no-cpu-baseline", "--no-e2e", "--no-parity", "--no-block-calls", "--no-scan-side", "--sustain-seconds", "0",
+                  "--dump-outputs", str(tmp_path))
+    assert d["steps"] == steps and d["warmup"] == 3
+    assert sorted(os.listdir(tmp_path)) == ["output0.npy"]
+    got = np.load(tmp_path / "output0.npy")
+    assert got.dtype == np.float32 and got.shape == (C, n)
+    e = Engine(C, block=1024, max_samples=n)
+    S.config3().apply(e)
+    x = S.noise(C, n, seed=42)
+    for _ in range(3 + steps):
+        y = e.process(x)[0]
+    assert_bit_exact(got, y, "dumped output vs the engine's last call")

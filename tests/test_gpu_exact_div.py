@@ -12,7 +12,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 def test_div_const_matches_ieee_for_every_f32_dividend(tmp_path):
     exe = str(tmp_path / "div_exhaustive")
-    subprocess.check_call(["nvcc", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-o", exe,
+    from dsp_stuff_b200.build import _nvcc   # the compiler the library is built with, also when nvcc is not on PATH
+
+    subprocess.check_call([_nvcc(), "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-o", exe,
                            os.path.join(ROOT, "tests", "cuda", "div_exhaustive.cu")])
     nf = np.float32(0.0001)
     divisors = []
