@@ -133,6 +133,8 @@ struct Node {
     int64_t id;
     int type;
     std::vector<float> f32;   // by ParamDef index
+    std::vector<std::vector<float>> f32_pc;  // by ParamDef index: per-channel values (dspb_node_set_f32_channels), empty = shared;
+                                             // f32 then holds channel 0's value
     std::vector<int> enums;   // by EnumDef index
     // biquad: normalised coefficients (regenerate_filter, nodes/biquad.rs:62-76)
     float bq[5] = {0.758f, 0.f, 0.f, -0.24f, 0.f};  // b0 b1 b2 a1 a2 (initial_filter, biquad.rs:48-55)
@@ -175,6 +177,8 @@ struct Step {
     std::vector<Bind> binds;             // parallel to prog.bufs
     std::vector<int> ring_nodes;         // parallel to prog.rings
     std::vector<int> nodes;              // STEP_FUSED: the nodes (engine indices) whose ops this segment holds, in order
+    std::vector<float> pc_host;          // STEP_FUSED: per-channel parameter table [C x pc_k] (plan.h Program::pc), or empty
+    int pc_k = 0;
     std::string text;                    // human-readable listing
 };
 
@@ -190,6 +194,7 @@ struct dspb_engine {
     std::vector<std::vector<std::vector<int>>> in_links, out_links;
     std::vector<Step> steps;
     std::vector<std::unique_ptr<DevBuf>> scratch;  // [C x max_samples] intermediates crossing steps
+    std::vector<std::unique_ptr<DevBuf>> pc_tabs;  // per step: its per-channel parameter table on the device (or null)
     // host-memory mode staging
     std::vector<std::unique_ptr<DevBuf>> h_in, h_out;
     cudaStream_t s_h2d = nullptr, s_cmp = nullptr, s_d2h = nullptr;
@@ -331,13 +336,43 @@ int64_t reverb_delay(float seconds, int sample_rate, int granule) {
     return round_up(num, granule);
 }
 
-void biquad_regenerate(Node& n) {  // BiQuad::regenerate_filter, nodes/biquad.rs:62-76 (f32 divisions)
-    const float a0 = n.f32[0];
-    n.bq[3] = n.f32[1] / a0;  // a1
-    n.bq[4] = n.f32[2] / a0;  // a2
-    n.bq[0] = n.f32[3] / a0;  // b0
-    n.bq[1] = n.f32[4] / a0;  // b1
-    n.bq[2] = n.f32[5] / a0;  // b2
+// BiQuad::regenerate_filter, nodes/biquad.rs:62-76 (f32 divisions): sliders a0 a1 a2 b0 b1 b2 -> bq = b0 b1 b2 a1 a2
+void biquad_coefs(const float* f, float* bq) {
+    const float a0 = f[0];
+    bq[3] = f[1] / a0;  // a1
+    bq[4] = f[2] / a0;  // a2
+    bq[0] = f[3] / a0;  // b0
+    bq[1] = f[4] / a0;  // b1
+    bq[2] = f[5] / a0;  // b2
+}
+void biquad_regenerate(Node& n) { biquad_coefs(n.f32.data(), n.bq); }
+float calc_gain(float frames) { return frames == 0.0f ? 0.0f : std::exp(-1.0f / frames); }  // dasp calc_gain
+
+// The values op `which` of a node of type `type` reads, in plan.h op_pc_cols order (p[0], p[1], ...; the biquad's a2 last),
+// from the node's slider values f (ParamDef order) with the reference's host arithmetic.  Both the shared Op fields and every
+// row of a per-channel table come from here.  which: 0, or the gate's second op (1: the compare).
+void op_values(int type, int which, const float* f, float* v) {
+    switch (type) {
+        case T_GAIN: case T_DISTORT: case T_MIX: v[0] = f[0]; break;
+        case T_OVERDRIVE: v[0] = f[0]; v[1] = f[1]; v[2] = f[2]; break;
+        case T_CHEBY:  // level.tanh(): libm tanhf, as the reference host would
+            v[0] = f[0]; v[1] = f[1]; v[2] = std::tanh(f[0]); v[3] = std::tanh(f[1]); break;
+        case T_BIQUAD: biquad_coefs(f, v); break;
+        case T_LOWPASS: case T_HIGHPASS: v[0] = f[0]; v[1] = 1.0f - f[0]; break;
+        case T_REVERB: v[0] = f[1]; break;  // decay (seconds sets the ring length: shared)
+        case T_ENVELOPE: v[0] = calc_gain(f[0]); v[1] = calc_gain(f[1]); break;
+        case T_SIGGEN: v[0] = f[0]; v[1] = f[1]; break;
+        case T_GATE:
+            if (which == 0) { v[0] = calc_gain(f[1]); v[1] = calc_gain(f[2]); }
+            else v[0] = f[0];
+            break;
+    }
+}
+// op_values into the shared Op fields
+void set_op_values(Op& op, const float* v) {
+    const int n = op_pc_cols(op.code);
+    for (int k = 0; k < n && k < 4; k++) op.p[k] = v[k];
+    if (n > 4) op.a2 = v[4];
 }
 
 bool is_stateful(int type) {
@@ -379,6 +414,7 @@ struct Lowerer {
     std::vector<int> node_step;                   // step index in which a node's ops are emitted
     std::set<int> fused_sinks;                    // output terminals written directly by a FIR step
     std::vector<ScanTab> scan_tabs;               // scan tables of the current fused step (Op::mode = index + 1)
+    std::vector<std::vector<float>> pc_cols;      // per-channel table of the current fused step, column by column
     std::string err;
     // A graph region between two FIR nodes normally becomes ONE fused segment.  When it exceeds what one Program holds
     // (ops, global buffers, states, rings, virtual vregs, shared memory) the segment is closed in front of a node and the
@@ -492,6 +528,35 @@ struct Lowerer {
         emit(o, "v" + std::to_string(id) + " = acc                    ; " + what);
         return id;
     }
+    // Per-channel parameters of the op node `ni` is about to emit: when one of `fields` (a bitmask over its ParamDef indices)
+    // holds per-channel values that no linked control port overrides (lib.rs:122-161), the op gets op_pc_cols columns in
+    // this segment's table, row c = op_values of channel c's sliders -- the function that gave the op its shared values.
+    // Returns the listing marker ("" = shared parameters).
+    std::string per_channel(Op& op, int ni, int which, unsigned fields) {
+        const Node& nd = *e.nodes[ni];
+        const NodeType& nt = kNodeTypes[nd.type];
+        std::string names;
+        for (size_t p = 0; p < nt.params.size(); p++) {
+            if (!((fields >> p) & 1) || nd.f32_pc[p].empty()) continue;
+            const int port = nt.params[p].ctl_port;
+            if (port >= 0 && !e.in_links[ni][port].empty()) continue;
+            names += std::string(names.empty() ? "" : ",") + nt.params[p].name;
+        }
+        if (names.empty()) return "";
+        const int k = op_pc_cols(op.code), col = (int)pc_cols.size();
+        if (col + k > kMaxPcCols) { overflow("segment has more per-channel parameters than one table holds"); return ""; }
+        const int C = e.cfg.channels;
+        pc_cols.resize(col + k, std::vector<float>(C));
+        std::vector<float> f(nd.f32);
+        float v[5] = {0, 0, 0, 0, 0};
+        for (int c = 0; c < C; c++) {
+            for (size_t p = 0; p < f.size(); p++) f[p] = nd.f32_pc[p].empty() ? nd.f32[p] : nd.f32_pc[p][c];
+            op_values(nd.type, which, f.data(), v);
+            for (int q = 0; q < k; q++) pc_cols[col + q][c] = v[q];
+        }
+        op.pad = (uint8_t)((op.pad & 1) | ((col + 1) << 1));
+        return " per-channel[" + names + "]";
+    }
     void close_fused();
     int lower();
     int finish_vregs(Step& st, std::vector<Op>& o, std::vector<std::string>& t);
@@ -591,7 +656,7 @@ int Lowerer::finish_vregs(Step& st, std::vector<Op>& o, std::vector<std::string>
 }
 
 void Lowerer::close_fused() {
-    if (ops.empty() || !err.empty()) { cur = Step(); ops.clear(); txt.clear(); cur_nodes.clear(); next_vreg = 0; return; }
+    if (ops.empty() || !err.empty()) { cur = Step(); ops.clear(); txt.clear(); cur_nodes.clear(); pc_cols.clear(); next_vreg = 0; return; }
     cur.kind = STEP_FUSED;
     finish_vregs(cur, ops, txt);
     if ((int)ops.size() > kMaxOps - 1) {  // the folded program does not fit: cut the segment in the middle and lower again
@@ -632,6 +697,14 @@ void Lowerer::close_fused() {
         if (c == OP_COMB) min_ring = std::min(min_ring, e.nodes[cur.ring_nodes[ops[i].aux & 0xff]]->D);
     }
     scan_tabs.clear();
+    cur.pc_k = (int)pc_cols.size();
+    if (cur.pc_k) {  // row-major [C x K]: row = absolute channel
+        const int C = e.cfg.channels;
+        cur.pc_host.assign((size_t)C * cur.pc_k, 0.0f);
+        for (int k = 0; k < cur.pc_k; k++)
+            for (int c = 0; c < C; c++) cur.pc_host[(size_t)c * cur.pc_k + k] = pc_cols[k][c];
+    }
+    pc_cols.clear();
     // Tile geometry: G channels x S = 4096/G samples per CTA.  S may not exceed the shortest comb
     // delay (a tile must never read a ring slot it writes itself); recurrences run lane = channel,
     // so they want G large, but the grid wants >= ~1.7 CTAs per SM (148 SMs).
@@ -706,6 +779,10 @@ void Lowerer::close_fused() {
     snprintf(hdr, sizeof hdr, "fused segment: G=%d channels x S=%d samples per CTA, %d ops, %d smem vregs, %d prefetch slots, alg_bytes=%d\n", G,
              S, P.n_ops, P.n_vregs, P.n_prefetch, alg);
     cur.text = hdr;
+    if (cur.pc_k) {
+        cur.text.pop_back();
+        cur.text += ", per-channel table " + std::to_string(cur.pc_k) + " column(s)\n";
+    }
     for (size_t i = 0; i < txt.size(); i++) cur.text += "    " + txt[i] + "\n";
     {   // the lowered program as the kernel sees it (physical shared-memory slots, prefetch flags): "op<code>:..." per op
         std::string m = "    lowered:";
@@ -716,6 +793,7 @@ void Lowerer::close_fused() {
             if (op_reads_vreg_field(o.code) || o.code == OP_SAVEV) k += snprintf(b + k, sizeof b - k, ":v%d", o.vreg == 0xFF ? -1 : (int)o.vreg);
             for (int q = 0; q < 3; q++)
                 if (o.pflags & (1 << q)) k += snprintf(b + k, sizeof b - k, ":p%d=v%d", q, (int)o.pv[q]);
+            if (op_pc_col(o) >= 0) k += snprintf(b + k, sizeof b - k, ":c%d", op_pc_col(o));  // per-channel table column
             if (o.code == OP_LOADG || o.code == OP_ADDG || o.code == OP_COPYG || o.code == OP_STOREG) k += snprintf(b + k, sizeof b - k, ":g%d%s", (int)o.buf, o.aux ? "*" : "");
             m += b;
         }
@@ -899,27 +977,35 @@ int Lowerer::lower() {
                 emit_avg(ni, 1);
                 int vb = temp_save(tag + ".b");
                 Op op = mk(nd.type == T_ADD ? OP_ADD : OP_MIX);
-                if (nd.type == T_MIX) ctl_param(op, 0, 0);
+                std::string pcm;
+                if (nd.type == T_MIX) {
+                    ctl_param(op, 0, 0);
+                    pcm = per_channel(op, ni, 0, 1u);
+                }
                 emit_avg(ni, 0);
                 op.vreg = (uint8_t)vb;
                 emit(op, nd.type == T_ADD ? "acc = acc + v" + std::to_string(vb) + "            ; " + tag
-                                          : "acc = v" + std::to_string(vb) + "*r + acc*(1-r)      ; " + tag);
+                                          : "acc = v" + std::to_string(vb) + "*r + acc*(1-r)" + pcm + "      ; " + tag);
                 values[{ni, 0}] = out_value(0);
             } break;
             case T_GATE: {  // extension: x -> vreg, envelope(x) (nodes/envelope.rs arithmetic) -> compare -> select
                 emit_avg(ni, 0);
                 const int vx = temp_save(tag + ".x");
                 Op env = mk(OP_ENVELOPE);
-                env.p[0] = nd.f32[1] == 0.0f ? 0.0f : std::exp(-1.0f / nd.f32[1]);  // dasp calc_gain
-                env.p[1] = nd.f32[2] == 0.0f ? 0.0f : std::exp(-1.0f / nd.f32[2]);
+                float v[5];
+                op_values(T_GATE, 0, nd.f32.data(), v);
+                set_op_values(env, v);
+                const std::string pce = per_channel(env, ni, 0, 6u);
                 if (alloc_state(env) < 0) return DSPB_ERR_INVALID;
-                char b[160];
-                snprintf(b, sizeof b, "acc = envelope(acc; ga=%g gr=%g) exact, lane=channel  ; %s", env.p[0], env.p[1], tag.c_str());
+                char b[200];
+                snprintf(b, sizeof b, "acc = envelope(acc; ga=%g gr=%g) exact, lane=channel%s  ; %s", env.p[0], env.p[1], pce.c_str(), tag.c_str());
                 emit(env, b);
                 Op g = mk(OP_GATE);
                 g.vreg = (uint8_t)vx;
-                g.p[0] = nd.f32[0];
-                snprintf(b, sizeof b, "acc = acc >= %g ? v%d : 0     ; %s (extension)", nd.f32[0], vx, tag.c_str());
+                op_values(T_GATE, 1, nd.f32.data(), v);
+                set_op_values(g, v);
+                const std::string pcg = per_channel(g, ni, 1, 1u);
+                snprintf(b, sizeof b, "acc = acc >= %g ? v%d : 0%s     ; %s (extension)", nd.f32[0], vx, pcg.c_str(), tag.c_str());
                 emit(g, b);
                 values[{ni, 0}] = out_value(0);
             } break;
@@ -929,63 +1015,74 @@ int Lowerer::lower() {
                 ctl_param(op, 0, 0);  // amplitude
                 ctl_param(op, 1, 1);  // frequency
                 op.p[2] = (float)e.cfg.sample_rate;
+                const std::string pcm = per_channel(op, ni, 0, 3u);
                 if (alloc_state(op) < 0) return DSPB_ERR_INVALID;
-                char b[160];
-                snprintf(b, sizeof b, "acc = signal_gen[%s](amp=%g, freq=%g)  ; %s", nt.enums[0].variants[nd.enums[0]], nd.f32[0], nd.f32[1], tag.c_str());
+                char b[200];
+                snprintf(b, sizeof b, "acc = signal_gen[%s](amp=%g, freq=%g)%s  ; %s", nt.enums[0].variants[nd.enums[0]], nd.f32[0], nd.f32[1],
+                         pcm.c_str(), tag.c_str());
                 emit(op, b);
                 values[{ni, 0}] = out_value(0);
             } break;
             default: {  // single-input effect nodes
                 Op op = mk(OP_END);
-                std::string desc;
+                std::string desc, pcm;
                 char b[320];
                 switch (nd.type) {
                     case T_GAIN:
                         op.code = OP_GAIN;
                         ctl_param(op, 0, 0);
-                        snprintf(b, sizeof b, "acc *= level(%g)", nd.f32[0]);
+                        pcm = per_channel(op, ni, 0, 1u);
+                        snprintf(b, sizeof b, "acc *= level(%g)%s", nd.f32[0], pcm.c_str());
                         break;
                     case T_DISTORT:
                         op.code = OP_DISTORT;
                         op.mode = (uint8_t)nd.enums[0];
                         ctl_param(op, 0, 0);
-                        set_const_div(op, 0, 1, nd.f32[0], e.plan_only);
-                        snprintf(b, sizeof b, "acc = distort[%s](acc, %g)", nt.enums[0].variants[nd.enums[0]], nd.f32[0]);
+                        pcm = per_channel(op, ni, 0, 1u);
+                        // the exact fast division is verified per divisor: per-channel levels divide with IEEE division (dv)
+                        if (pcm.empty()) set_const_div(op, 0, 1, nd.f32[0], e.plan_only);
+                        snprintf(b, sizeof b, "acc = distort[%s](acc, %g)%s", nt.enums[0].variants[nd.enums[0]], nd.f32[0], pcm.c_str());
                         break;
                     case T_OVERDRIVE:
                         op.code = OP_OVERDRIVE;
                         ctl_param(op, 0, 0);
                         ctl_param(op, 1, 1);
                         ctl_param(op, 2, 2);
-                        snprintf(b, sizeof b, "acc = overdrive(acc, %g, %g, %g)", nd.f32[0], nd.f32[1], nd.f32[2]);
+                        pcm = per_channel(op, ni, 0, 7u);
+                        snprintf(b, sizeof b, "acc = overdrive(acc, %g, %g, %g)%s", nd.f32[0], nd.f32[1], nd.f32[2], pcm.c_str());
                         break;
-                    case T_CHEBY:
+                    case T_CHEBY: {
                         op.code = OP_CHEBY;
-                        op.p[0] = nd.f32[0];
-                        op.p[1] = nd.f32[1];
-                        op.p[2] = std::tanh(nd.f32[0]);  // level.tanh(): libm tanhf, as the reference host would
-                        op.p[3] = std::tanh(nd.f32[1]);
-                        snprintf(b, sizeof b, "acc = chebyshev(acc, %g, %g)", nd.f32[0], nd.f32[1]);
-                        break;
+                        float v[5];
+                        op_values(T_CHEBY, 0, nd.f32.data(), v);
+                        set_op_values(op, v);
+                        pcm = per_channel(op, ni, 0, 3u);
+                        snprintf(b, sizeof b, "acc = chebyshev(acc, %g, %g)%s", nd.f32[0], nd.f32[1], pcm.c_str());
+                    } break;
                     case T_BIQUAD:
                     case T_LOWPASS:
                     case T_HIGHPASS: {
                         ScanTab tab;
                         if (nd.type == T_BIQUAD) {
                             op.code = OP_BIQUAD;
-                            for (int i = 0; i < 4; i++) op.p[i] = nd.bq[i];
-                            op.a2 = nd.bq[4];
+                            set_op_values(op, nd.bq);  // regenerated by every setter (biquad_regenerate)
                             tab = make_scan_tab(nd.bq[3], nd.bq[4]);
+                            pcm = per_channel(op, ni, 0, 63u);
                             snprintf(b, sizeof b, "acc = DF1(acc; b=%g,%g,%g a=%g,%g)", nd.bq[0], nd.bq[1], nd.bq[2], nd.bq[3], nd.bq[4]);
                         } else {
                             op.code = nd.type == T_LOWPASS ? OP_LP1 : OP_HP1;
-                            op.p[0] = nd.f32[0];
-                            op.p[1] = 1.0f - nd.f32[0];
+                            float v[5];
+                            op_values(nd.type, 0, nd.f32.data(), v);
+                            set_op_values(op, v);
                             tab = make_scan_tab(-nd.f32[0], 0.0f);  // z[n] = xr[n] + ratio z[n-1]
+                            pcm = per_channel(op, ni, 0, 1u);
                             snprintf(b, sizeof b, "acc = %s(acc; ratio=%g)", nt.cfg_name, nd.f32[0]);
                         }
                         std::string how = " exact, lane=channel";
-                        if (e.cfg.iir_mode == 1) {
+                        if (!pcm.empty()) {
+                            // one scan table per Program, not per channel: per-channel coefficients stay sequential (exact)
+                            how = (e.cfg.iir_mode == 1 ? " exact (per-channel coefficients)" : how) + pcm;
+                        } else if (e.cfg.iir_mode == 1) {
                             char v[96];
                             if (scan_qualifies(op, tab, e.plan_only)) {
                                 // a Program holds kMaxScan scan tables; a fifth qualifying filter would stay sequential and
@@ -1004,19 +1101,22 @@ int Lowerer::lower() {
                         }
                         strncat(b, how.c_str(), sizeof b - strlen(b) - 1);
                     } break;
-                    case T_ENVELOPE:
+                    case T_ENVELOPE: {
                         op.code = OP_ENVELOPE;
-                        op.p[0] = nd.f32[0] == 0.0f ? 0.0f : std::exp(-1.0f / nd.f32[0]);  // dasp calc_gain
-                        op.p[1] = nd.f32[1] == 0.0f ? 0.0f : std::exp(-1.0f / nd.f32[1]);
-                        snprintf(b, sizeof b, "acc = envelope(acc; ga=%g gr=%g) exact, lane=channel", op.p[0], op.p[1]);
-                        break;
+                        float v[5];
+                        op_values(T_ENVELOPE, 0, nd.f32.data(), v);
+                        set_op_values(op, v);
+                        pcm = per_channel(op, ni, 0, 3u);
+                        snprintf(b, sizeof b, "acc = envelope(acc; ga=%g gr=%g) exact, lane=channel%s", op.p[0], op.p[1], pcm.c_str());
+                    } break;
                     case T_REVERB:
                         op.code = OP_COMB;
                         op.p[0] = nd.f32[1];
                         if ((int)cur.ring_nodes.size() >= kMaxRings) { overflow("too many reverb nodes in one segment"); return DSPB_ERR_INVALID; }
+                        pcm = per_channel(op, ni, 0, 2u);
                         op.aux = (uint16_t)cur.ring_nodes.size();
                         cur.ring_nodes.push_back(ni);
-                        snprintf(b, sizeof b, "acc += ring*%g ; ring = acc   (D=%lld)", nd.f32[1], (long long)nd.D);
+                        snprintf(b, sizeof b, "acc += ring*%g ; ring = acc   (D=%lld)%s", nd.f32[1], (long long)nd.D, pcm.c_str());
                         break;
                     default:
                         err = "unhandled node type";
@@ -1130,6 +1230,24 @@ int lower_graph(dspb_engine* e) {
         n_scratch = L.n_scratch;
         break;
     }
+    // Per-channel parameter tables.  Rows up to C + 31 exist (zero) because the last CTA's lanes may run past C with
+    // discarded results.  Lowering runs inside dspb_process, whose kernels go to non-blocking streams: the pageable copy
+    // is waited for here (off the hot path), so a kernel never reads a table the DMA has not finished.
+    e->pc_tabs.resize(e->steps.size());
+    bool uploaded = false;
+    for (size_t i = 0; i < e->steps.size(); i++) {
+        Step& st = e->steps[i];
+        if (st.pc_host.empty()) continue;
+        if (!e->pc_tabs[i]) e->pc_tabs[i] = std::make_unique<DevBuf>();
+        DevBuf& tb = *e->pc_tabs[i];
+        r = tb.alloc(((size_t)e->cfg.channels + 31) * st.pc_k * 4, true, e->plan_only);
+        if (r) return r;
+        if (!e->plan_only) CUDA_TRY(cudaMemcpy(tb.p, st.pc_host.data(), st.pc_host.size() * 4, cudaMemcpyHostToDevice));
+        st.prog.pc = tb.p;
+        st.prog.pc_stride = st.pc_k;
+        uploaded = true;
+    }
+    if (uploaded && !e->plan_only) CUDA_TRY(cudaDeviceSynchronize());
     while ((int)e->scratch.size() < n_scratch) {
         auto b = std::make_unique<DevBuf>();
         r = b->alloc((size_t)e->cfg.channels * e->cfg.max_samples * 4, false, e->plan_only);
@@ -1307,6 +1425,21 @@ int check_ready(dspb_engine* e, int64_t n) {
     return DSPB_OK;
 }
 
+// after_settings_change (lib.rs:560-568) of a slider store, shared or per channel
+int after_settings_change(dspb_engine* e, Node& n) {
+    if (!e->plan_only) CUDA_TRY(cudaSetDevice(e->cfg.device));
+    if (n.type == T_BIQUAD) {  // regenerate_filter: new coefficients + reset_state (per-channel ones: at lowering, op_values)
+        biquad_regenerate(n);
+        if (n.state.p && !e->plan_only) CUDA_TRY(cudaMemsetAsync(n.state.p, 0, n.state.bytes, nullptr));
+    }
+    if (n.type == T_REVERB) {  // refresh_seconds on ANY slider of the node
+        n.D = reverb_delay(n.f32[0], e->cfg.sample_rate, e->cfg.ring_granule);
+        n.ring_dirty = true;
+    }
+    e->lowered = false;
+    return DSPB_OK;
+}
+
 }  // namespace
 
 // =================================================== C ABI =====================================================
@@ -1386,6 +1519,7 @@ int dspb_node_add(dspb_engine* e, const char* cfg_name, int64_t node_id) {
     n->id = node_id;
     n->type = type;
     for (auto& p : kNodeTypes[type].params) n->f32.push_back(p.def);
+    n->f32_pc.resize(n->f32.size());
     for (auto& en : kNodeTypes[type].enums) n->enums.push_back(en.def);
     if (type == T_REVERB) n->D = round_up(128, e->cfg.ring_granule);  // make_buffer(): circular_buffer(128), reverb.rs:44-52
     e->nodes.push_back(std::move(n));
@@ -1402,17 +1536,29 @@ int dspb_node_set_f32(dspb_engine* e, int64_t node_id, const char* field, float 
     if (p < 0) return fail(DSPB_ERR_UNKNOWN_PORT, "node type '%s' has no f32 field '%s'", kNodeTypes[n.type].cfg_name, field);
     DSPB_QUIESCE(e);
     n.f32[p] = value;
-    if (!e->plan_only) CUDA_TRY(cudaSetDevice(e->cfg.device));
-    if (n.type == T_BIQUAD) {  // after_settings_change = regenerate_filter: new coefficients + reset_state
-        biquad_regenerate(n);
-        if (n.state.p && !e->plan_only) CUDA_TRY(cudaMemsetAsync(n.state.p, 0, n.state.bytes, nullptr));
-    }
-    if (n.type == T_REVERB) {  // after_settings_change = refresh_seconds on ANY slider of the node (lib.rs:560-568)
-        n.D = reverb_delay(n.f32[0], e->cfg.sample_rate, e->cfg.ring_granule);
-        n.ring_dirty = true;
-    }
-    e->lowered = false;
-    return DSPB_OK;
+    n.f32_pc[p].clear();  // shared again
+    return after_settings_change(e, n);
+}
+
+int dspb_node_set_f32_channels(dspb_engine* e, int64_t node_id, const char* field, const float* values, int64_t n_values) {
+    if (!e || !field || !values) return fail(DSPB_ERR_INVALID, "null argument");
+    int i = e->find(node_id);
+    if (i < 0) return fail(DSPB_ERR_UNKNOWN_NODE, "unknown node id %lld", (long long)node_id);
+    Node& n = *e->nodes[i];
+    int p = param_index(kNodeTypes[n.type], field);
+    if (p < 0) return fail(DSPB_ERR_UNKNOWN_PORT, "node type '%s' has no f32 field '%s'", kNodeTypes[n.type].cfg_name, field);
+    if (n.type == T_REVERB && p == 0)
+        return fail(DSPB_ERR_INVALID, "reverb.seconds cannot vary per channel: it sets the ring length D, and the ring is one "
+                                      "[C x D] array with one D for every channel (use dspb_node_set_f32)");
+    if (n_values != e->cfg.channels)
+        return fail(DSPB_ERR_INVALID, "n_values %lld != channels %d", (long long)n_values, e->cfg.channels);
+    bool same = true;  // bit for bit: NaN payloads and the sign of zero count
+    for (int64_t c = 1; c < n_values && same; c++) same = memcmp(&values[c], &values[0], 4) == 0;
+    if (same) return dspb_node_set_f32(e, node_id, field, values[0]);
+    DSPB_QUIESCE(e);
+    n.f32_pc[p].assign(values, values + n_values);
+    n.f32[p] = values[0];
+    return after_settings_change(e, n);
 }
 
 int dspb_node_set_enum(dspb_engine* e, int64_t node_id, const char* field, const char* variant) {
@@ -1870,17 +2016,17 @@ int dspb_node_process(dspb_engine* e, int64_t node_id, const float* const* port_
             if ((r = dspb_link(sub, 0, nt.outs[q], 2000 + q, "in"))) return r;
         }
         Node& dst = *sub->nodes[0];
-        dst.f32 = src.f32; dst.enums = src.enums; dst.taps = src.taps; dst.D = src.D;
+        dst.f32 = src.f32; dst.f32_pc = src.f32_pc; dst.enums = src.enums; dst.taps = src.taps; dst.D = src.D;
         memcpy(dst.bq, src.bq, sizeof dst.bq);
         if ((r = dspb_compile(sub))) return r;
     }
     dspb_engine* sub = ne.e;
     Node& dst = *sub->nodes[0];
     // setters on the parent node since the last call: same side effects as on the parent (after_settings_change)
-    if (dst.f32 != src.f32 || dst.enums != src.enums || dst.taps != src.taps || dst.D != src.D) {
-        const bool f32_changed = dst.f32 != src.f32 || dst.D != src.D;
+    if (dst.f32 != src.f32 || dst.f32_pc != src.f32_pc || dst.enums != src.enums || dst.taps != src.taps || dst.D != src.D) {
+        const bool f32_changed = dst.f32 != src.f32 || dst.f32_pc != src.f32_pc || dst.D != src.D;
         const bool taps_changed = dst.taps != src.taps;
-        dst.f32 = src.f32; dst.enums = src.enums; dst.taps = src.taps; dst.D = src.D;
+        dst.f32 = src.f32; dst.f32_pc = src.f32_pc; dst.enums = src.enums; dst.taps = src.taps; dst.D = src.D;
         memcpy(dst.bq, src.bq, sizeof dst.bq);
         CUDA_TRY(cudaSetDevice(e->cfg.device));
         if (f32_changed && dst.type == T_BIQUAD && dst.state.p) CUDA_TRY(cudaMemset(dst.state.p, 0, dst.state.bytes));

@@ -111,6 +111,7 @@ __device__ __forceinline__ void stg_stream(float4* p, float4 v) {
 // ---- sequential cores: only the ops that depend on the previous output ---------------------------------
 struct DF1Core {  // y = (p - a1*y1) - a2*y2, p = b0*x + b1*x1 + b2*x2 precomputed (biquad 0.4.2 DirectForm1::run)
     float a1, a2, y1, y2;
+    __device__ __forceinline__ void from_row(const float* r) { a1 = r[3]; a2 = r[4]; }  // per-channel table: b0 b1 b2 a1 a2
     __device__ __forceinline__ void load(const float4 s) { y1 = s.z; y2 = s.w; }
     __device__ __forceinline__ void save(float4& s) const { s.z = y1; s.w = y2; }
     __device__ __forceinline__ float step(float p) {
@@ -121,12 +122,14 @@ struct DF1Core {  // y = (p - a1*y1) - a2*y2, p = b0*x + b1*x1 + b2*x2 precomput
 };
 struct OnePoleCore {  // z = xr + r*z, xr = x*(1-r) precomputed (nodes/low_pass.rs:37, high_pass.rs:37)
     float r, z;
+    __device__ __forceinline__ void from_row(const float* row) { r = row[0]; }  // per-channel table: ratio, 1 - ratio
     __device__ __forceinline__ void load(const float4 s) { z = s.x; }
     __device__ __forceinline__ void save(float4& s) const { s.x = z; }
     __device__ __forceinline__ float step(float xr) { z = add(xr, mul(r, z)); return z; }
 };
 struct EnvCore {  // dasp_envelope 0.11.0 Detector<f32, Peak<FullWave>>::next, d = |x| precomputed
     float ga, gr, prev;
+    __device__ __forceinline__ void from_row(const float* r) { ga = r[0]; gr = r[1]; }
     __device__ __forceinline__ void load(const float4 s) { prev = s.x; }
     __device__ __forceinline__ void save(float4& s) const { s.x = prev; }
     __device__ __forceinline__ float step(float d) {
@@ -190,8 +193,10 @@ struct TileCtx {
 };
 
 // v (time-parallel, 16 per thread) -> tile; one warp runs `core` lane = channel; tile -> v.
+// pcr != null: per-channel coefficients, the op's columns of table row 0; lane l takes row ch0 + l (ch0: the CTA's first channel).
 template <int G, class Core>
-__device__ __forceinline__ void run_recurrence(Core core, float (&v)[kChunk], const TileCtx& c, float4* st) {
+__device__ __forceinline__ void run_recurrence(Core core, float (&v)[kChunk], const TileCtx& c, float4* st,
+                                               const float* pcr = nullptr, long long pc_stride = 0, int ch0 = 0) {
     using Q = Geo<G>;
     float4* row = reinterpret_cast<float4*>(c.tile + c.g * Q::ROW);
 #pragma unroll
@@ -201,6 +206,7 @@ __device__ __forceinline__ void run_recurrence(Core core, float (&v)[kChunk], co
     const int lane = threadIdx.x & 31;
     if ((threadIdx.x >> 5) == c.rec_warp && lane < G && c.valid_f4 > 0) {  // strictly sequential in time
         float4* r = reinterpret_cast<float4*>(c.tile + lane * Q::ROW);
+        if (pcr) core.from_row(pcr + (long long)(ch0 + lane) * pc_stride);
         float4 s = st[lane];
         core.load(s);
         recurrence_row(core, r, c.valid_f4);
@@ -393,11 +399,31 @@ struct Pf {
 // compile-time constants in the specialised kernels (the switch folds away) and run-time values in
 // the generic interpreter.  pre & 1: acc = 0.0 + acc (first link of a fan-in sum, node.rs:181-183);
 // pre & 2: acc /= nf (node.rs:189-191) with the divisor in p[4], its reciprocal in p[5].
-template <int G>
+// PC: the op may carry per-channel parameters (plan.h Program::pc); false in the compiled specialised chains, whose ops
+// never do (chain_matches), so their code is the shared-parameter code only.
+template <int G, bool PC = false>
 __device__ __forceinline__ void exec_op(const int code, const int mode, const int pre, const int pfc, const Op& op,
                                         const Ctx<G>& c, float (&acc)[kChunk], Pf& pf) {
     const Program& prog = *c.prog;
     const int t = c.t;
+    // scalar parameters: the op's own, or this thread's channel row of the per-channel table (resolved here, once: the code
+    // below is the shared-parameter code run with per-thread values).  Table rows exist for every channel a CTA covers.
+    // prm(i): p[i], prm(4): a2.  Without PC the op's fields are read where they are used, exactly as before.
+    float pcv[5] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
+    const float* pcr = nullptr;  // the op's first column in row 0 (the recurrence lanes pick their own rows)
+    if constexpr (PC) {
+        pcv[0] = op.p[0]; pcv[1] = op.p[1]; pcv[2] = op.p[2]; pcv[3] = op.p[3]; pcv[4] = op.a2;
+        if (op.pad >> 1) {
+            pcr = prog.pc + op_pc_col(op);
+            const float* r = pcr + (long long)c.ch * prog.pc_stride;
+            const int n = op_pc_cols(code);
+            for (int k = 0; k < n; k++) pcv[k] = r[k];
+        }
+    }
+    auto prm = [&](int i) -> float {
+        if constexpr (PC) return pcv[i];
+        else return i < 4 ? op.p[i] : op.a2;
+    };
     if (pre & 1) {
 #pragma unroll
         for (int i = 0; i < kChunk; i++) acc[i] = add(0.0f, acc[i]);
@@ -487,14 +513,14 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
 #pragma unroll
                 for (int i = 0; i < kChunk; i++) acc[i] = mul(acc[i], P[i]);
             } else {
-                const float l = op.p[0];
+                const float l = prm(0);
 #pragma unroll
                 for (int i = 0; i < kChunk; i++) acc[i] = mul(acc[i], l);
             }
         } break;
         case OP_DISTORT: {
             if (!(op.pflags & 1) && mode != Fuzz) {  // scalar level: the common case
-                const float l = op.p[0];
+                const float l = prm(0);       // per-channel: the host clears pad bit 0, so the divisions below are IEEE (dv)
                 if (l < 0.001f) break;  // every shaper returns the sample unchanged (distort.rs:64,...)
                 const ConstDiv dl{l, op.p[1]};
                 const bool fast = op.pad & 1;
@@ -562,7 +588,7 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
             if (op.pflags & 1) load16(c.vregs + (op.pv[0] * kF4) * kThreads + t, kThreads, P);
             else {
 #pragma unroll
-                for (int i = 0; i < kChunk; i++) P[i] = op.p[0];
+                for (int i = 0; i < kChunk; i++) P[i] = prm(0);
             }
             if (mode == Fuzz) {  // nodes/distort.rs:146-172, per 128-sample reference block
                 const float mx = block128_max_abs(acc);
@@ -587,7 +613,7 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
             if (op.pflags & 7) {
                 float B[kChunk], D[kChunk], L[kChunk];
 #pragma unroll
-                for (int i = 0; i < kChunk; i++) { B[i] = op.p[0]; D[i] = op.p[1]; L[i] = op.p[2]; }
+                for (int i = 0; i < kChunk; i++) { B[i] = prm(0); D[i] = prm(1); L[i] = prm(2); }
                 if (op.pflags & 1) load16(c.vregs + (op.pv[0] * kF4) * kThreads + t, kThreads, B);
                 if (op.pflags & 2) load16(c.vregs + (op.pv[1] * kF4) * kThreads + t, kThreads, D);
                 if (op.pflags & 4) load16(c.vregs + (op.pv[2] * kF4) * kThreads + t, kThreads, L);
@@ -596,7 +622,7 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
             } else {
                 const float FRAC_PI_4 = 0.785398163397448309615660845819875721f;
                 const float FRAC_2_PI = 0.636619772367581343075535053490057448f;
-                const float b = op.p[0], dr = op.p[1], l = op.p[2];
+                const float b = prm(0), dr = prm(1), l = prm(2);
                 if (l < 0.001f) break;
                 const float omd = sub(1.0f, dr);
 #pragma unroll
@@ -608,7 +634,7 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
             }
         } break;
         case OP_CHEBY: {
-            const float lp = op.p[0], ln = op.p[1], tp = op.p[2], tn = op.p[3];
+            const float lp = prm(0), ln = prm(1), tp = prm(2), tn = prm(3);
 #pragma unroll
             for (int i = 0; i < kChunk; i++) {
                 const float x = acc[i];
@@ -625,14 +651,14 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
 #pragma unroll
                 for (int i = 0; i < kChunk; i++) acc[i] = add(mul(b[i], R[i]), mul(acc[i], sub(1.0f, R[i])));
             } else {
-                const float r = op.p[0], omr = sub(1.0f, r);
+                const float r = prm(0), omr = sub(1.0f, r);
 #pragma unroll
                 for (int i = 0; i < kChunk; i++) acc[i] = add(mul(b[i], r), mul(acc[i], omr));
             }
         } break;
         case OP_COMB: {
             const RingDesc& r = prog.rings[op.aux & 0xff];
-            const float decay = op.p[0];
+            const float decay = prm(0);
             const int pslot = op.aux >> 8;  // 0 = not staged
             float* rrow = r.base + (long long)c.ch * r.D;
             const bool pfd = pfc < 0 ? pslot != 0 : pfc != 0;
@@ -683,7 +709,7 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
         } break;
         case OP_BIQUAD: {
             // p[n] = b0*x[n] + b1*x[n-1] + b2*x[n-2] in the reference's order, time-parallel
-            const float b0 = op.p[0], b1 = op.p[1], b2 = op.p[2];
+            const float b0 = prm(0), b1 = prm(1), b2 = prm(2);
             float4* st = c.sm_state + op.aux * G;
             c.edge[t] = make_float2(acc[kChunk - 2], acc[kChunk - 1]);
             __syncthreads();
@@ -709,14 +735,14 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
                 break;
             }
             DF1Core core;
-            core.a1 = op.p[3];
-            core.a2 = op.a2;
-            run_recurrence<G>(core, acc, c.tc, st);  // first barrier inside: every thread has read st / edge
+            core.a1 = prm(3);
+            core.a2 = prm(4);
+            run_recurrence<G>(core, acc, c.tc, st, pcr, prog.pc_stride, c.ch - c.g);  // first barrier inside: every thread has read st / edge
             if (c.j == c.j_last) { st[c.g].x = nx1; st[c.g].y = nx2; }
         } break;
         case OP_LP1:
         case OP_HP1: {
-            const float omr = op.p[1];
+            const float omr = prm(1);
             float v[kChunk];
 #pragma unroll
             for (int i = 0; i < kChunk; i++) v[i] = mul(acc[i], omr);
@@ -727,8 +753,8 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
                 break;
             }
             OnePoleCore core;
-            core.r = op.p[0];
-            run_recurrence<G>(core, v, c.tc, c.sm_state + op.aux * G);
+            core.r = prm(0);
+            run_recurrence<G>(core, v, c.tc, c.sm_state + op.aux * G, pcr, prog.pc_stride, c.ch - c.g);
 #pragma unroll
             for (int i = 0; i < kChunk; i++) acc[i] = code == OP_LP1 ? v[i] : sub(acc[i], v[i]);
         } break;
@@ -736,14 +762,14 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
 #pragma unroll
             for (int i = 0; i < kChunk; i++) acc[i] = fabsf(acc[i]);
             EnvCore core;
-            core.ga = op.p[0];
-            core.gr = op.p[1];
-            run_recurrence<G>(core, acc, c.tc, c.sm_state + op.aux * G);
+            core.ga = prm(0);
+            core.gr = prm(1);
+            run_recurrence<G>(core, acc, c.tc, c.sm_state + op.aux * G, pcr, prog.pc_stride, c.ch - c.g);
         } break;
         case OP_GATE: {  // extension: hard noise gate keyed by the envelope already in acc
             float x[kChunk];
             load16(c.vregs + (op.vreg * kF4) * kThreads + t, kThreads, x);
-            const float thr = op.p[0];
+            const float thr = prm(0);
 #pragma unroll
             for (int i = 0; i < kChunk; i++) acc[i] = acc[i] >= thr ? x[i] : 0.0f;
         } break;
@@ -752,7 +778,7 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
             if (op.pflags & 1) load16(c.vregs + (op.pv[0] * kF4) * kThreads + t, kThreads, A);
             else {
 #pragma unroll
-                for (int i = 0; i < kChunk; i++) A[i] = op.p[0];
+                for (int i = 0; i < kChunk; i++) A[i] = prm(0);
             }
             if (mode == 3) {  // Constant: output = amplitude, clock untouched
 #pragma unroll
@@ -782,7 +808,7 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
                 }
                 total_end = run;
             } else {
-                const float step = dv(op.p[1], sr);
+                const float step = dv(prm(1), sr);
                 float run = 0.0f;
                 for (int m = 0; m < pos; m++) run = add(run, step);
 #pragma unroll
@@ -951,7 +977,7 @@ fused_kernel(const __grid_constant__ Program prog, int c_begin, int c_end, long 
         } else {
             for (int ip = 0; ip < prog.n_ops; ip++) {
                 const Op& op = prog.ops[ip];
-                exec_op<G>(op.code, op.mode, op.pre, -1, op, c, acc, pf);
+                exec_op<G, true>(op.code, op.mode, op.pre, -1, op, c, acc, pf);
             }
         }
     }
@@ -1061,6 +1087,9 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
     float* keep = tiles + 2 * G * Q::ROW;
     float4* stage = reinterpret_cast<float4*>(keep + (rcode == OP_HP1 ? 2 * G * Q::ROW : 0));
     float* stp = prog.states[rop.aux];
+    // per-channel coefficients of the recurrence op (interpreter only: chain_matches keeps such ops out of the chains)
+    constexpr bool PC = Chain::n == 0;
+    const bool rpc = PC && op_pc_col(rop) >= 0;
 
     if (t >= n_e) {  // ---------------- R warps ----------------
         constexpr int GP = (G + kNR - 1) / kNR;  // channels per R warp
@@ -1072,6 +1101,7 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
         float4* sout = reinterpret_cast<float4*>(stp) + (ok ? ch : 0);
         if (rcode == OP_BIQUAD) {
             DF1Core core; core.a1 = rop.p[3]; core.a2 = rop.a2;
+            if (PC && rpc && ok) core.from_row(prog.pc + op_pc_col(rop) + (long long)ch * prog.pc_stride);
             // y1, y2 live in .z/.w; the E warps own .x/.y (x1, x2) and write them separately at the end
             float4 s = make_float4(0, 0, 0, 0);
             if (ok) s = *sin;
@@ -1102,9 +1132,11 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
             if (ok) { float* f = reinterpret_cast<float*>(sout); f[2] = core.y1; f[3] = core.y2; }
         } else if (rcode == OP_LP1 || rcode == OP_HP1) {
             OnePoleCore core; core.r = rop.p[0];
+            if (PC && rpc && ok) core.from_row(prog.pc + op_pc_col(rop) + (long long)ch * prog.pc_stride);
             ws_recurrence_warp<G>(core, tiles, sin, sout, lane, ok, n_tiles, T, n_ws);
         } else {
             EnvCore core; core.ga = rop.p[0]; core.gr = rop.p[1];
+            if (PC && rpc && ok) core.from_row(prog.pc + op_pc_col(rop) + (long long)ch * prog.pc_stride);
             ws_recurrence_warp<G>(core, tiles, sin, sout, lane, ok, n_tiles, T, n_ws);
         }
         return;
@@ -1177,7 +1209,7 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
             for (int k = 0; k < kChunk; k++) acc[k] = 0.0f;
             if constexpr (Chain::n > 0) run_static_range<G, Chain, 0, Chain::rec>(prog, c, acc, pf);
             else
-                for (int ip = 0; ip < rec_index; ip++) exec_op<G>(prog.ops[ip].code, prog.ops[ip].mode, prog.ops[ip].pre, -1, prog.ops[ip], c, acc, pf);
+                for (int ip = 0; ip < rec_index; ip++) exec_op<G, true>(prog.ops[ip].code, prog.ops[ip].mode, prog.ops[ip].pre, -1, prog.ops[ip], c, acc, pf);
 #ifdef DSPB_WS_TIMING
             tp1 = clock64();
 #endif
@@ -1189,7 +1221,10 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
             }
             if (rpre & 2) div16(acc, ConstDiv{rop.p[4], rop.p[5]}, rpre & 4);
             if (rcode == OP_BIQUAD) {
-                const float b0 = rop.p[0], b1 = rop.p[1], b2 = rop.p[2];
+                float b0 = rop.p[0], b1 = rop.p[1], b2 = rop.p[2];
+                if constexpr (PC) {
+                    if (rpc) { const float* r = prog.pc + op_pc_col(rop) + (long long)c.ch * prog.pc_stride; b0 = r[0]; b1 = r[1]; b2 = r[2]; }
+                }
                 const float nx1 = acc[kChunk - 1], nx2 = acc[kChunk - 2];
                 float xm1, xm2;
                 if constexpr (Q::TPC <= 32) {
@@ -1230,7 +1265,10 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
                     for (int k = 0; k < kF4; k++)
                         krow[kF4 * c.j + (k ^ sw_of(c.j))] = make_float4(acc[4 * k], acc[4 * k + 1], acc[4 * k + 2], acc[4 * k + 3]);
                 }
-                const float omr = rop.p[1];
+                float omr = rop.p[1];
+                if constexpr (PC) {
+                    if (rpc) omr = prog.pc[op_pc_col(rop) + 1 + (long long)c.ch * prog.pc_stride];
+                }
 #pragma unroll
                 for (int k = 0; k < kChunk; k++) acc[k] = mul(acc[k], omr);
             } else {
@@ -1271,7 +1309,7 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
             }
             if constexpr (Chain::n > 0) run_static_range<G, Chain, Chain::rec + 1, Chain::n>(prog, c, acc, pf);
             else
-                for (int ip = rec_index + 1; ip < prog.n_ops; ip++) exec_op<G>(prog.ops[ip].code, prog.ops[ip].mode, prog.ops[ip].pre, -1, prog.ops[ip], c, acc, pf);
+                for (int ip = rec_index + 1; ip < prog.n_ops; ip++) exec_op<G, true>(prog.ops[ip].code, prog.ops[ip].mode, prog.ops[ip].pre, -1, prog.ops[ip], c, acc, pf);
         }
 #ifdef DSPB_WS_TIMING
         if (blockIdx.x == 0 && t == 0) { long long te3 = clock64(); g_ws_timing[2] += te1 - te0; g_ws_timing[3] += te2 - te1; g_ws_timing[4] += te3 - te2;
@@ -1369,14 +1407,19 @@ fused_kernel_ws2(const __grid_constant__ Program prog, int c_begin, int c_end, l
         float* stp = prog.states[rop.aux];
         float* tl = tiles + st * (2 * G * Q::ROW);
         const int bf = BAR2_FULL + 2 * st, bd = BAR2_DONE + 2 * st;
+        // per-channel coefficients: this lane's channel row (plan.h Program::pc)
+        const float* pr = op_pc_col(rop) >= 0 && ok ? prog.pc + op_pc_col(rop) + (long long)ch * prog.pc_stride : nullptr;
         if (rop.code == OP_BIQUAD) {
             DF1Core core; core.a1 = rop.p[3]; core.a2 = rop.a2;
+            if (pr) core.from_row(pr);
             ws2_rec_loop<G>(core, tl, stp, lane, ch, ok, nt, T, bf, bd, n_ws, true);
         } else if (rop.code == OP_LP1 || rop.code == OP_HP1) {
             OnePoleCore core; core.r = rop.p[0];
+            if (pr) core.from_row(pr);
             ws2_rec_loop<G>(core, tl, stp, lane, ch, ok, nt, T, bf, bd, n_ws, false);
         } else {
             EnvCore core; core.ga = rop.p[0]; core.gr = rop.p[1];
+            if (pr) core.from_row(pr);
             ws2_rec_loop<G>(core, tl, stp, lane, ch, ok, nt, T, bf, bd, n_ws, false);
         }
         return;
@@ -1437,8 +1480,11 @@ fused_kernel_ws2(const __grid_constant__ Program prog, int c_begin, int c_end, l
             for (int k = 0; k < kChunk; k++) acc[k] = add(0.0f, acc[k]);
         }
         if (rop.pre & 2) div16(acc, ConstDiv{rop.p[4], rop.p[5]}, rop.pre & 4);
+        // per-channel parameters: this thread's channel row
+        const float* pr = op_pc_col(rop) >= 0 ? prog.pc + op_pc_col(rop) + (long long)c.ch * prog.pc_stride : nullptr;
         if (rop.code == OP_BIQUAD) {
-            const float b0 = rop.p[0], b1 = rop.p[1], b2 = rop.p[2];
+            float b0 = rop.p[0], b1 = rop.p[1], b2 = rop.p[2];
+            if (pr) { b0 = pr[0]; b1 = pr[1]; b2 = pr[2]; }
             const float nx1 = acc[kChunk - 1], nx2 = acc[kChunk - 2];
             float xm1, xm2;
             if constexpr (Q::TPC <= 32) {
@@ -1473,7 +1519,7 @@ fused_kernel_ws2(const __grid_constant__ Program prog, int c_begin, int c_end, l
                 for (int k = 0; k < kF4; k++)
                     krow[kF4 * c.j + (k ^ sw_of(c.j))] = make_float4(acc[4 * k], acc[4 * k + 1], acc[4 * k + 2], acc[4 * k + 3]);
             }
-            const float omr = rop.p[1];
+            const float omr = pr ? pr[1] : rop.p[1];
 #pragma unroll
             for (int k = 0; k < kChunk; k++) acc[k] = mul(acc[k], omr);
         } else {
@@ -1527,7 +1573,7 @@ fused_kernel_ws2(const __grid_constant__ Program prog, int c_begin, int c_end, l
             } else {
                 fetch(ph - 1, ti, acc);
             }
-            for (int ip = lo[ph]; ip < hi[ph]; ip++) exec_op<G>(prog.ops[ip].code, prog.ops[ip].mode, prog.ops[ip].pre, -1, prog.ops[ip], c, acc, pf);
+            for (int ip = lo[ph]; ip < hi[ph]; ip++) exec_op<G, true>(prog.ops[ip].code, prog.ops[ip].mode, prog.ops[ip].pre, -1, prog.ops[ip], c, acc, pf);
             if (ph < 2) feed(ph == 0 ? rop1 : rop2, ph, ti, acc);
         }
     }
@@ -1687,6 +1733,7 @@ bool chain_matches(const Program& p) {
         const int s = Chain::sig(i);
         const Op& o = p.ops[i];
         if (o.code != (s & 0xff) || o.pre != ((s >> 16) & 0xff) || o.pflags != 0) return false;
+        if (op_pc_col(o) >= 0) return false;  // per-channel parameters: the interpreter (ChainDynamic) runs them
         if (o.code == OP_DISTORT && o.mode != ((s >> 8) & 0xff)) return false;
         if ((o.code == OP_BIQUAD || o.code == OP_LP1 || o.code == OP_HP1) && o.mode != ((s >> 8) & 0xff)) return false;  // exact vs scan
         const bool is_src = o.code == OP_LOADG || o.code == OP_ADDG || o.code == OP_COPYG || o.code == OP_STOREG;

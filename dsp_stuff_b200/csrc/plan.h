@@ -94,11 +94,23 @@ struct Op {
     uint8_t pv[3];    // vregs of tile-valued parameters
     uint8_t buf;      // global buffer index for LOADG/ADDG/STOREG, prefetch slot + 1 in `aux`
     uint16_t aux;     // ring / state slot, or prefetch slot (0 = none, k+1 = slot k)
-    uint8_t pad;      // bit 0: p[1] holds a verified reciprocal of p[0] (exact_math.cuh div_const)
+    uint8_t pad;      // bit 0: p[1] holds a verified reciprocal of p[0] (exact_math.cuh div_const);
+                      // bits 1-7: per-channel parameters, 1 + the column of this op's first value in Program::pc (0 = shared)
     uint8_t pre;      // fan-in prologue folded into this op: 1 = acc = 0.0 + acc; 2 = acc /= p[4]; 4 = p[5] = 1/p[4] usable
     float p[6];       // p[4], p[5]: fan-in divisor and its reciprocal when pre & 2
     float a2;         // biquad: a2 (p[0..3] = b0, b1, b2, a1)
 };
+
+// Per-channel parameters (dspb_node_set_f32_channels).  An op whose `pad >> 1` is k > 0 reads its parameters from row `ch`
+// (the ABSOLUTE channel) of the step's table Program::pc, columns k-1 ... k-2+op_pc_cols(code), in this order: p[0], p[1],
+// ... and, for the biquad, a2 last.  Everything else (fan-in divisor, sample rate, control-port tiles) stays in the Op.
+constexpr int kMaxPcCols = 32;      // columns of one step's table (a segment that needs more is cut)
+__host__ __device__ inline constexpr int op_pc_cols(int code) {
+    return code == OP_BIQUAD ? 5 : code == OP_CHEBY ? 4 : code == OP_OVERDRIVE ? 3
+         : (code == OP_LP1 || code == OP_HP1 || code == OP_ENVELOPE || code == OP_SIGGEN) ? 2
+         : (code == OP_GAIN || code == OP_DISTORT || code == OP_MIX || code == OP_COMB || code == OP_GATE) ? 1 : 0;
+}
+__host__ __device__ inline int op_pc_col(const Op& o) { return (o.pad >> 1) - 1; }  // -1: shared parameters
 
 // Does an op of this code read the shared-memory vreg named by Op::vreg?  (SAVEV writes it; parameter tiles are in pv[].)
 inline constexpr bool op_reads_vreg_field(int code) {
@@ -136,7 +148,11 @@ struct Program {
     int16_t st_buf;        // buffer of the first STOREG (its op has aux = 1): row pointer kept in a register, or -1
     int16_t n_scan;        // scan tables in use
     ScanTab scan[kMaxScan];
+    const float* pc;       // per-channel parameter table [C x pc_stride] f32, row = absolute channel (null: none)
+    int64_t pc_stride;
 };
+// passed by value as a kernel parameter (__grid_constant__): keep it well inside the 4 KB parameter space
+static_assert(sizeof(Program) <= 4096, "Program must stay a kernel parameter");
 
 // ---- launchers (defined in the .cu files) -----------------------------------------------------------
 // Runs `prog` for channels [c_begin, c_end) and samples [0, T) of this call.  G in {1,2,4,8,16,32}.

@@ -55,7 +55,7 @@ ABI_SYMBOLS = [
     "dspb_node_set_f32", "dspb_node_set_enum", "dspb_node_set_taps", "dspb_node_set_impulse_response", "dspb_link",
     "dspb_load_graph_json", "dspb_compile", "dspb_process", "dspb_node_process", "dspb_reset_state",
     "dspb_node_get_i64", "dspb_node_port_index", "dspb_describe_plan", "dspb_profile_enable", "dspb_profile_read",
-    "dspb_fold_stereo", "dspb_dup_stereo", "dspb_resample_dup_stereo", "dspb_sync",
+    "dspb_fold_stereo", "dspb_dup_stereo", "dspb_resample_dup_stereo", "dspb_sync", "dspb_node_set_f32_channels",
 ]
 
 _lib = None
@@ -77,6 +77,7 @@ def load_library(path: Optional[str] = None):
     L.dspb_engine_destroy.restype = None
     L.dspb_node_add.argtypes = [vp, cp, i64]
     L.dspb_node_set_f32.argtypes = [vp, i64, cp, ctypes.c_float]
+    L.dspb_node_set_f32_channels.argtypes = [vp, i64, cp, vp, i64]
     L.dspb_node_set_enum.argtypes = [vp, i64, cp, cp]
     L.dspb_node_set_taps.argtypes = [vp, i64, vp, i64]
     L.dspb_node_set_impulse_response.argtypes = [vp, i64, vp, i64]
@@ -143,6 +144,13 @@ class Engine:
 
     def set_f32(self, node_id: int, field: str, value: float):
         self._ck(self._L.dspb_node_set_f32(self._h, node_id, field.encode(), float(value)))
+
+    def set_f32_channels(self, node_id: int, field: str, values):
+        """One slider value per channel (float32, length `channels`): channel c runs as if set_f32(values[c]) had been
+        called on an engine holding only channel c.  All values bit-identical = set_f32(values[0]); a later set_f32 on
+        the field makes it shared again.  reverb.seconds cannot vary per channel."""
+        v = np.ascontiguousarray(values, dtype=np.float32).reshape(-1)
+        self._ck(self._L.dspb_node_set_f32_channels(self._h, node_id, field.encode(), v.ctypes.data, v.size))
 
     def set_enum(self, node_id: int, field: str, variant: str):
         self._ck(self._L.dspb_node_set_enum(self._h, node_id, field.encode(), variant.encode()))

@@ -1,6 +1,7 @@
-"""Channel sharding across ranks (SURVEY.md section 8e): every channel owns its state, parameters are
-replicated, so the path partitions with no data-path collective.  The only collective is the optional
-gather of output blocks to rank 0."""
+"""Channel sharding across ranks (SURVEY.md section 8e): every channel owns its state, shared parameters are
+replicated and per-channel ones (Engine.set_f32_channels) are sliced: rank r's engine gets values[lo:hi] with
+(lo, hi) = channel_range(r, ...).  So the path partitions with no data-path collective.  The only collective is the
+optional gather of output blocks to rank 0."""
 from __future__ import annotations
 
 from typing import Optional, Tuple

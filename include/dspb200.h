@@ -10,8 +10,10 @@
  * Data model
  *   A graph is instantiated once and run over `channels` independent mono
  *   streams.  All audio is f32, laid out channel-major: buffer[c * n + i] is
- *   sample i of channel c ("[C x n] SoA rows").  Parameters and FIR taps are
- *   shared by all channels; filter/delay/FIR state is per channel.
+ *   sample i of channel c ("[C x n] SoA rows").  Filter/delay/FIR state is per
+ *   channel.  Parameters are shared by all channels unless a field is given one
+ *   value per channel (dspb_node_set_f32_channels); FIR taps, enum fields and
+ *   reverb.seconds are always shared.
  *
  * Threading: one caller thread per engine handle at a time; setters are legal
  * between dspb_process calls and take effect at the next call (the reference
@@ -107,6 +109,23 @@ int dspb_node_add(dspb_engine* e, const char* cfg_name, int64_t node_id);
  * Reverb::refresh_seconds replaces the ring with a zero-filled one (nodes/reverb.rs:55-71).
  * Values are NOT clamped to the slider range (restore() does not clamp either, lib.rs:295-309). */
 int dspb_node_set_f32(dspb_engine* e, int64_t node_id, const char* field, float value);
+
+/* Per-channel slider values: channel c of this engine runs node `node_id` as if dspb_node_set_f32(field, values[c]) had been
+ * called on a one-channel engine holding only channel c.  values: host pointer, n_values == channels.
+ *   - Side effects are those of dspb_node_set_f32: a biquad regenerates its coefficients (per channel) and resets the state
+ *     of every channel; a reverb replaces its ring with a zero-filled one.  Takes effect at the next dspb_process.
+ *   - All values bit-identical (NaN payloads and the sign of zero count): exactly dspb_node_set_f32(values[0]), same plan,
+ *     same kernels, same outputs.
+ *   - A later dspb_node_set_f32 on the same field makes it shared again; other fields are not affected.
+ *   - Every f32 field except reverb.seconds may vary per channel.  reverb.seconds fails with DSPB_ERR_INVALID: it sets the
+ *     ring length D, and the ring is one [C x D] array with one D for all channels.
+ *   - A linked control port (<field>_input, lib.rs:122-161) still overrides the slider: its per-channel values are unused
+ *     while the port is linked.
+ *   - Errors: DSPB_ERR_UNKNOWN_NODE (node id), DSPB_ERR_UNKNOWN_PORT (no such f32 field), DSPB_ERR_INVALID (null pointer,
+ *     n_values != channels, reverb.seconds).
+ *   - Planning engines (device -1) accept the call; dspb_describe_plan marks per-channel parameters ("per-channel[...]").
+ *   - Not stored in saved-graph JSON (one scalar per field there). */
+int dspb_node_set_f32_channels(dspb_engine* e, int64_t node_id, const char* field, const float* values, int64_t n_values);
 
 /* Replaces: the derive-generated select store; `variant` is the Rust enum variant name
  * ("SoftClip", "Balanced", "A", "Sine", ...), the same string serde writes (lib.rs:266-293). */
