@@ -150,7 +150,7 @@ struct Node {
                                     // previous hist_pad samples right behind it -- history carries over without a copy
     int u_ring = 0, u_pos = 0;      // u_ring = round_up(hist_pad + max_samples, 128)
     DevBuf Y;                       // [C x max_samples]
-    std::vector<std::unique_ptr<DevBuf>> fft_work;  // persistent FFT kernel: work counter + per-CTA scratch, one per launch lane
+    std::vector<std::unique_ptr<DevBuf>> fft_work;  // persistent FFT kernels: work counters, one set per launch lane
     DevBuf fdl;                     // short calls (UPC kernel): frequency-domain delay line, [pairs][P][2048] complex
     bool fdl_valid = false;         // the previous call was a UPC call: the FDL holds the P-1 previous block spectra
     bool upc_this_call = false;
@@ -935,7 +935,7 @@ int Lowerer::lower() {
                 if (e.cfg.fir_mode == FIR_FFT || e.cfg.fir_mode == FIR_FFT_PACKED)
                     snprintf(b, sizeof b, "fir step: %s, %zu taps, overlap-save FFT 2^%d%s, two channels per transform, alg_bytes=8\n", tag.c_str(),
                              nd.taps.size(), e.cfg.fir_fft_log2,
-                             e.cfg.fir_mode == FIR_FFT_PACKED ? " (packed f32x2 variant)" : " (+ 2^14 double segments as two sub-transforms, persistent CTAs)");
+                             e.cfg.fir_mode == FIR_FFT_PACKED ? " (packed f32x2 variant)" : " (+ 2^14 double segments in one piece, persistent CTAs)");
                 else if (e.cfg.fir_mode == FIR_TOEPLITZ)
                     snprintf(b, sizeof b, "fir step: %s, %zu taps, Toeplitz-tiled tcgen05 GEMM 128x256x32, split bf16 (3 MMAs per K step), alg_bytes=8\n",
                              tag.c_str(), nd.taps.size());
@@ -1173,6 +1173,14 @@ int ensure_resources(dspb_engine* e) {
             }
             n.fdl_valid = false;
             n.upc_ctr = 0;
+            // work counters of the persistent FFT kernels, one set per launch lane: device-pointer chunk k runs on lane k,
+            // an unchunked call and the host path on lane 0
+            n.fft_work.clear();
+            for (int lane = 0; e->cfg.fir_mode == FIR_FFT && lane < std::max(1, e->dev_chunks); lane++) {
+                n.fft_work.push_back(std::make_unique<DevBuf>());
+                r = n.fft_work.back()->alloc(fir_fft_work_bytes(), true, e->plan_only);
+                if (r) return r;
+            }
             const bool toep = e->cfg.fir_mode == FIR_TOEPLITZ && N <= fir_toeplitz_max_taps();
             if (toep) {
                 r = n.toep_tiles.alloc(fir_toeplitz_tiles_bytes(N), false, e->plan_only);
@@ -1367,23 +1375,14 @@ int run_steps(dspb_engine* e, const float* const* d_in, float* const* d_out, int
             fp.post_nf = s.fir_post_nf;
             fp.u_ring = f.u_ring;
             fp.u_pos = f.u_pos;
-            // work area of the persistent FFT kernel: one per launch lane (lanes run concurrently on their own streams)
-            fp.fft_work = nullptr;
-            if (fp.mode == FIR_FFT) {
-                while ((int)f.fft_work.size() <= lane) {
-                    auto wb = std::make_unique<DevBuf>();
-                    int r = wb->alloc(fir_fft_work_bytes(), true, e->plan_only);
-                    if (r) return r;
-                    f.fft_work.push_back(std::move(wb));
-                }
-                fp.fft_work = f.fft_work[lane]->p;
-            }
+            // work counters of the persistent FFT kernels: lanes run concurrently on their own streams
+            fp.fft_work = fp.mode == FIR_FFT ? f.fft_work[lane]->p : nullptr;
             // short calls (1 or 2 blocks of 1024): uniformly partitioned convolution with a frequency-domain delay line.  Measured
             // at 4096 channels: 62 / 101 / 141 us for 1 / 2 / 3 blocks against 92 - 104 us for the one 8192-point window the
-            // segment kernel needs for any call of up to 4096 samples.  DSPB_FIR_UPC=n: up to n blocks (0 = never).
-            static const int upc_max_blocks = getenv("DSPB_FIR_UPC") ? atoi(getenv("DSPB_FIR_UPC")) : 2;
+            // segment kernel needs for any call of up to 4096 samples.
+            constexpr int kUpcMaxBlocks = 2;
             const int upc_P = fir_upc_partitions(fp.n_taps);
-            f.upc_this_call = fp.mode == FIR_FFT && upc_P > 0 && f.fdl.p && n % kUpcBlock == 0 && n / kUpcBlock <= upc_max_blocks;
+            f.upc_this_call = fp.mode == FIR_FFT && upc_P > 0 && f.fdl.p && n % kUpcBlock == 0 && n / kUpcBlock <= kUpcMaxBlocks;
             if (f.upc_this_call) {
                 fp.upc_fdl = f.fdl.p;
                 fp.upc_prime = f.fdl_valid ? 0 : upc_P - 1;

@@ -17,7 +17,7 @@
 namespace dspb {
 
 int launch_fir_fft(const FirPlan& fp, const float* U, int64_t u_stride, float* Y, int64_t y_stride, int c_begin, int c_end,
-                   int64_t T, int64_t started, cudaStream_t st, int* n_launches);
+                   int64_t T, cudaStream_t st, int* n_launches);
 
 int launch_fir_upc(const FirPlan& fp, const float* U, int64_t u_stride, float* Y, int64_t y_stride, int c_begin, int c_end, int64_t T,
                    cudaStream_t st, int* n_launches);
@@ -94,7 +94,7 @@ int launch_fir(const FirPlan& fp, const float* U, int64_t u_stride, float* Y, in
     }
     int rc = fp.mode == FIR_TOEPLITZ ? launch_fir_toeplitz(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, st, n_launches)
              : (fp.mode == FIR_FFT && fp.upc_fdl) ? launch_fir_upc(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, st, n_launches)
-                                                  : launch_fir_fft(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, started, st, n_launches);
+                                                  : launch_fir_fft(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, st, n_launches);
     if (rc) return rc;
     // Samples that still belong to the warm-up are recomputed exactly by the direct kernel.
     const int64_t warm_end = (int64_t)fp.n_taps - 1 - started;  // call-relative

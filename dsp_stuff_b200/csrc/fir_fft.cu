@@ -8,17 +8,11 @@
 // The last forward pass, the spectrum product and the first inverse pass happen in registers.  The first pass reads the
 // input window straight from global memory and the last pass writes the valid outputs straight back.
 //
-// Segments.  An 8192-point window ("F13") yields V13 = 8192 - (Ne-1) valid outputs -- half of it at 4096 taps.  A
-// 16384-point window ("F14") yields 16384 - (Ne-1) = three quarters, and it is computed with the SAME 64 KB of shared
-// memory as two 8192-point sub-transforms in sequence (one radix-2 decimation-in-frequency step in front):
-//     E[n] = z[n] + z[n+8192]               -> even bins:  e' = IFFT8192(FFT8192(E) .* H[2k])
-//     O[n] = (z[n] - z[n+8192]) W16384^n    -> odd bins:   o' = IFFT8192(FFT8192(O) .* H[2k+1])
-//     y[n] = e'[n] + W16384^-n o'[n],   y[n+8192] = e'[n] - W16384^-n o'[n]
-// e' is parked in a per-CTA scratch slot in global memory between the two halves (each thread reads back exactly
-// the values it wrote; the slots are reused item after item, so they stay L2-resident).  At 4096 taps one F14 item
-// costs ~2.25 F13 items and yields 3x the outputs: 25 % fewer instructions per output sample.
+// Segments.  An 8192-point window yields V13 = 8192 - (Ne-1) valid outputs -- half of it at 4096 taps; a 16384-point
+// window yields V14 = 16384 - (Ne-1), three quarters.  segment_plan cuts a call into 16384-point ("double") segments,
+// which fir_fft_wide_kernel runs, followed by 8192-point ("single") segments, which fir_fft_kernel runs.
 //
-// The kernel is persistent (3 CTAs per SM, 256 threads): CTAs fetch work items (channel pair, segment) from an
+// fir_fft_kernel is persistent (3 CTAs per SM, 256 threads): CTAs fetch work items (channel pair, segment) from an
 // atomic counter in segment-major order within a pair, so the overlapping windows of neighbouring segments meet in L2.
 // The input rows are rings (plan.h FirPlan::u_ring): a call's last N-1 samples are the next call's history in place.
 //
@@ -28,7 +22,6 @@
 
 #include <atomic>
 #include <cmath>
-#include <cstdlib>
 #include <mutex>
 #include <type_traits>
 #include <utility>
@@ -298,25 +291,19 @@ struct FftArgs {
     float* Y;
     long long y_stride;
     const float2* H13;     // spectrum of h for an 8192-point segment, transform order, scaled 1/8192
-    const float2* H14e;    // even / odd bins of the 16384-point spectrum, same order, scaled 1/16384
-    const float2* H14o;
     const float2* Wg;      // compact twiddle table [512 + 32]
     long long T;
     float divisor, post_nf;
     int c_begin, c_end;
-    int n14, n13;          // per channel pair: n14 double segments (V14 outputs each), then n13 single segments (V13 each)
-    long long single_base; // first output sample of the single segments (= double segments in front * V14, whoever ran them)
-    int n_items;           // pairs * (n14 + n13): all double segments first (the costly items), then the single ones
-    int n_heavy;           // pairs * n14
-    int stagger;           // start delay (cycles) per co-resident CTA slot, see fir_fft_kernel
-    unsigned* work;        // [0] next item, [1] CTAs done, [8 + smid] CTAs started on that SM
-    float4* scratch;       // [gridDim.x][kF / 2] e' of the even half, in the last pass's own register order
+    int n13;               // single segments per channel pair (V13 outputs each)
+    long long single_base; // first output sample of the single segments (= the wide kernel's double segments * V14)
+    int n_items;           // pairs * n13
+    unsigned* work;        // [0] next item, [1] CTAs done  (slots 2 / 3 belong to the wide kernel on the same lane)
 };
 
-// MODE 0: plain 8192-point segment.  MODE 1 / 2: even- / odd-bin half of a 16384-point segment.
 // FAST (CTA-uniform): the whole window lies inside this call's samples and does not wrap around the ring, and
 // hist == 4096, so no load is predicated and the valid outputs are exactly the butterfly outputs r >= 4.
-template <int MODE, bool FAST>
+template <bool FAST>
 __device__ __forceinline__ void fwd_pass1(C2<float>* a, const Tw<float>& W, const float* __restrict__ rowA, const float* __restrict__ rowB,
                                           int wb, int R, int lim, int t) {
     constexpr int L = kF / 8, LP = L + L / 16;
@@ -339,27 +326,12 @@ __device__ __forceinline__ void fwd_pass1(C2<float>* a, const Tw<float>& W, cons
     for (int k = 0; k < kF / 8 / kNT / 2; k++) {
         const int j = 2 * (t + kNT * k);
         C2<float> v0[8], v1[8], w[8];
-        C2<float> wj0 = {1.f, 0.f}, wj1 = {1.f, 0.f};
-        if constexpr (MODE == 2) { wj0 = W.at2(j); wj1 = W.at2(j + 1); }
         static_for<8>([&](auto rr) {
             constexpr int r = decltype(rr)::value;
-            const int n = j + r * L;
             float2 xa, xb;
-            load2(n, xa, xb);
-            if constexpr (MODE == 0) {
-                v0[r] = C2<float>{xa.x, xb.x};
-                v1[r] = C2<float>{xa.y, xb.y};
-            } else {
-                float2 ya, yb;
-                load2(n + kF, ya, yb);
-                if constexpr (MODE == 1) {
-                    v0[r] = C2<float>{xa.x + ya.x, xb.x + yb.x};
-                    v1[r] = C2<float>{xa.y + ya.y, xb.y + yb.y};
-                } else {  // (z[n] - z[n+8192]) W16384^(j + 1024 r) = ... W16384^j W16^r
-                    v0[r] = tw<16, r, false, float>(cmul(C2<float>{xa.x - ya.x, xb.x - yb.x}, wj0));
-                    v1[r] = tw<16, r, false, float>(cmul(C2<float>{xa.y - ya.y, xb.y - yb.y}, wj1));
-                }
-            }
+            load2(j + r * L, xa, xb);
+            v0[r] = C2<float>{xa.x, xb.x};
+            v1[r] = C2<float>{xa.y, xb.y};
         });
         C2<float>* p = a + pad(j);  // j is even: j and j + 1 share the padding offset
         twiddles8<1>(W, j, w);
@@ -402,9 +374,9 @@ __device__ __forceinline__ void mid_pass16(C2<float>* a, const C2<float>* __rest
     }
 }
 
-template <int MODE, bool FAST>
+template <bool FAST>
 __device__ __forceinline__ void inv_pass1(const C2<float>* a, const Tw<float>& W, float* __restrict__ outA, float* __restrict__ outB,
-                                          bool hasB, int hist, int lim, float divisor, float post_nf, float4* __restrict__ scr, int t) {
+                                          bool hasB, int hist, int lim, float divisor, float post_nf, int t) {
     constexpr int L = kF / 8, LP = L + L / 16;
     // Epilogue: `* divisor` (fir.rs:187-190, 222) and the fused sink average `(0.0 + y) / nf` collapse into ONE multiplication by
     // divisor / nf (formed in f64 on the host side of this expression, rounded once).  Against the two separately rounded
@@ -432,49 +404,30 @@ __device__ __forceinline__ void inv_pass1(const C2<float>* a, const Tw<float>& W
 #pragma unroll
         for (int s = 1; s < 8; s++) v1[s] = cmulc(p[1 + bitrev3(s) * LP], w[bitrev3(s)]);
         ifft_dit<8>(v1);
-        float4* sc = scr + (k * 8) * kNT + t;  // [k][r][thread]: coalesced, and read back by the thread that wrote it
-        if constexpr (MODE == 1) {
-#pragma unroll
-            for (int r = 0; r < 8; r++) __stcg(sc + r * kNT, make_float4(v0[r].x, v0[r].y, v1[r].x, v1[r].y));
-        } else if constexpr (MODE == 2) {
-            const C2<float> wj0 = W.at2(j), wj1 = W.at2(j + 1);
-            float4 e[8];
-#pragma unroll
-            for (int r = 0; r < 8; r++) e[r] = __ldcg(sc + r * kNT);
-            static_for<8>([&](auto rr) {
-                constexpr int r = decltype(rr)::value;
-                const int n = j + r * L;
-                const C2<float> t0 = tw<16, r, true, float>(cmulc(v0[r], wj0));  // W16384^-(j + 1024 r) o'[n]
-                const C2<float> t1 = tw<16, r, true, float>(cmulc(v1[r], wj1));
-                if (FAST ? r >= 4 : n >= hist) store2(n, e[r].x + t0.x, e[r].z + t1.x, e[r].y + t0.y, e[r].w + t1.y);
-                store2(n + kF, e[r].x - t0.x, e[r].z - t1.x, e[r].y - t0.y, e[r].w - t1.y);
-            });
-        } else {
-            static_for<8>([&](auto rr) {
-                constexpr int r = decltype(rr)::value;
-                const int n = j + r * L;
-                if (FAST ? r >= 4 : (n >= hist && n < lim)) store2(n, v0[r].x, v1[r].x, v0[r].y, v1[r].y);
-            });
-        }
+        static_for<8>([&](auto rr) {
+            constexpr int r = decltype(rr)::value;
+            const int n = j + r * L;
+            if (FAST ? r >= 4 : (n >= hist && n < lim)) store2(n, v0[r].x, v1[r].x, v0[r].y, v1[r].y);
+        });
     }
 }
 
-template <int MODE, bool FAST>
+template <bool FAST>
 __device__ __forceinline__ void transform(C2<float>* a, const Tw<float>& W, const FftArgs& g, const float* rowA, const float* rowB,
-                                          float* outA, float* outB, bool hasB, int wb, int lim, float4* scr, int t) {
-    fwd_pass1<MODE, FAST>(a, W, rowA, rowB, wb, g.u_ring, lim, t);
+                                          float* outA, float* outB, bool hasB, int wb, int lim, int t) {
+    fwd_pass1<FAST>(a, W, rowA, rowB, wb, g.u_ring, lim, t);
     __syncthreads();
     fwd_pass8<kF / 8>(a, W, t);
     __syncthreads();
     fwd_pass8<kF / 64>(a, W, t);
     __syncthreads();
-    mid_pass16(a, reinterpret_cast<const C2<float>*>(MODE == 0 ? g.H13 : MODE == 1 ? g.H14e : g.H14o), t);
+    mid_pass16(a, reinterpret_cast<const C2<float>*>(g.H13), t);
     __syncthreads();
     inv_pass8<kF / 64>(a, W, t);
     __syncthreads();
     inv_pass8<kF / 8>(a, W, t);
     __syncthreads();
-    inv_pass1<MODE, FAST>(a, W, outA, outB, hasB, g.hist, lim, g.divisor, g.post_nf, scr, t);
+    inv_pass1<FAST>(a, W, outA, outB, hasB, g.hist, lim, g.divisor, g.post_nf, t);
 }
 
 __global__ void __launch_bounds__(kNT, 3)
@@ -484,58 +437,29 @@ fir_fft_kernel(const __grid_constant__ FftArgs g) {
     C2<float>* a = reinterpret_cast<C2<float>*>(smem_f2);
     const int t = threadIdx.x;
     const Tw<float> W = load_tables<float>(a + kPadded, g.Wg, t);
-    float4* scr = g.scratch + (size_t)blockIdx.x * (kF / 2);
-    const int V13 = kF - g.hist, V14 = 2 * kF - g.hist;
-    // Persistent CTAs that start together stay in lockstep (every item costs the same), so all three CTAs of an SM
-    // would sit in their global-load pass at the same time and in their FP passes at the same time.  The k-th CTA to
-    // start on an SM waits k * stagger cycles once, which spreads the load phases for the rest of the launch.
-    if (g.stagger > 0) {
-        if (t == 0) {
-            unsigned smid;
-            asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-            const unsigned slot = atomicAdd(g.work + 8 + (smid & 255u), 1u) % 3u;
-            const long long t0 = clock64(), wait = (long long)slot * g.stagger;
-            while (clock64() - t0 < wait) __nanosleep(200);
-        }
-    }
+    const int V13 = kF - g.hist;
     for (;;) {
         __syncthreads();  // the previous item's last pass has read the shared array (and s_item); tables visible
         if (t == 0) s_item = (int)atomicAdd(g.work, 1u);
         __syncthreads();
         const int item = s_item;
         if (item >= g.n_items) break;
-        int pr, sg;
-        if (item < g.n_heavy) { pr = item / g.n14; sg = item - pr * g.n14; }
-        else { const int li = item - g.n_heavy; pr = li / g.n13; sg = g.n14 + (li - pr * g.n13); }
+        const int pr = item / g.n13, sg = item - pr * g.n13;
         const int chA = g.c_begin + 2 * pr, chB = chA + 1;
         const bool hasB = chB < g.c_end;
-        const bool dbl = sg < g.n14;
-        const long long s0 = dbl ? (long long)sg * V14 : g.single_base + (long long)(sg - g.n14) * V13;
+        const long long s0 = g.single_base + (long long)sg * V13;
         const long long w0 = s0 - g.hist;                      // call-relative index of window sample 0 (>= -hist)
-        const int win = dbl ? 2 * kF : kF;
         const long long lim_ll = g.T - w0;                     // window samples >= lim lie beyond this call's input: zeros
-        const int lim = lim_ll > win ? win : (int)lim_ll;
+        const int lim = lim_ll > kF ? kF : (int)lim_ll;
         const int wb = ring_slot(g.u_pos, (int)w0, g.u_ring);  // ring slot of window sample 0
         const float* rowA = g.U + (long long)chA * g.u_stride;
         const float* rowB = g.U + (long long)(hasB ? chB : chA) * g.u_stride;  // odd channel count: B mirrors A, never stored
         float* outA = g.Y + (long long)chA * g.y_stride + w0;
         float* outB = g.Y + (long long)(hasB ? chB : chA) * g.y_stride + w0;
-        const bool fast = g.hist == kF / 2 && lim == win && wb + win <= g.u_ring;
-        if (dbl) {  // lim == win is guaranteed by the launcher (double segments lie fully inside the call)
-            if (fast) {
-                transform<1, true>(a, W, g, rowA, rowB, outA, outB, hasB, wb, lim, scr, t);
-                __syncthreads();
-                transform<2, true>(a, W, g, rowA, rowB, outA, outB, hasB, wb, lim, scr, t);
-            } else {
-                transform<1, false>(a, W, g, rowA, rowB, outA, outB, hasB, wb, lim, scr, t);
-                __syncthreads();
-                transform<2, false>(a, W, g, rowA, rowB, outA, outB, hasB, wb, lim, scr, t);
-            }
-        } else if (fast) {
-            transform<0, true>(a, W, g, rowA, rowB, outA, outB, hasB, wb, lim, scr, t);
-        } else {
-            transform<0, false>(a, W, g, rowA, rowB, outA, outB, hasB, wb, lim, scr, t);
-        }
+        if (g.hist == kF / 2 && lim == kF && wb + kF <= g.u_ring)
+            transform<true>(a, W, g, rowA, rowB, outA, outB, hasB, wb, lim, t);
+        else
+            transform<false>(a, W, g, rowA, rowB, outA, outB, hasB, wb, lim, t);
     }
     // the last CTA out re-arms the work counter for the next launch on this lane (stream-ordered behind this one)
     if (t == 0) {
@@ -543,17 +467,17 @@ fir_fft_kernel(const __grid_constant__ FftArgs g) {
         if (atomicAdd(g.work + 1, 1u) == gridDim.x - 1) {
             g.work[0] = 0;
             g.work[1] = 0;
-            for (int i = 0; i < 256; i++) g.work[8 + i] = 0;
         }
     }
 }
 
 // ======================= 16384-point segments in one piece ("wide" kernel) =======================
-// The double segments above cost 2.9 single ones (measured): two sub-transforms, each with all six shared-memory round
-// trips of the 8192-point pipeline, which is what bounds that kernel (ncu: l1tex data pipe 69 % busy, 79 % of it shared
-// memory).  This kernel keeps a whole 16384-point transform of a channel pair in shared memory (139 KB, one 512-thread
-// CTA per SM, 128 registers per thread) with radices 16 . 32 . 32: FOUR shared-memory round trips per transform instead of
-// six, on 16384 points that yield 12288 outputs per channel instead of 8192 points that yield 4096.
+// A double segment run as two 8192-point sub-transforms (after one radix-2 step) costs 2.9 single segments (measured):
+// each sub-transform has all six shared-memory round trips of the pipeline above, which is what bounds it (ncu: l1tex
+// data pipe 69 % busy, 79 % of it shared memory).  This kernel keeps a whole 16384-point transform of a channel pair in
+// shared memory (139 KB, one 512-thread CTA per SM, 128 registers per thread) with radices 16 . 32 . 32: FOUR
+// shared-memory round trips per transform instead of six, on 16384 points that yield 12288 outputs per channel instead of
+// 8192 points that yield 4096.
 //   pass 1   global -> radix 16 over stride 1024 -> twiddle W16384^(j k) -> shared
 //   pass 2   radix 32 over stride 32 inside each 1024-block -> twiddle W1024^(j k) (table in shared memory) -> shared
 //   middle   radix 32 over 32 contiguous points . spectrum product . inverse radix 32, in registers
@@ -581,7 +505,7 @@ struct WideArgs {
     int c_begin, c_end;
     int n14;               // double segments per channel pair (all lie fully inside the call)
     int n_items;           // pairs * n14
-    unsigned* work;        // [2] next item, [3] CTAs done  (slots 0 / 1 belong to the narrow kernel on the same lane)
+    unsigned* work;        // [2] next item, [3] CTAs done  (slots 0 / 1 belong to fir_fft_kernel on the same lane)
 };
 
 __global__ void __launch_bounds__(kNTW, 1)
@@ -653,8 +577,7 @@ fir_fft_wide_kernel(const __grid_constant__ WideArgs g) {
                 const int nA = g.c_begin + 2 * npr;
                 const int nwb = ring_slot(g.u_pos, (int)((long long)nsg * V14 - g.hist), g.u_ring);
                 // 2 rows x 16384 floats = 1024 lines of 128 bytes: two per thread
-                const int line = t & 511, row = 0;
-                (void)row;
+                const int line = t & 511;
                 int sl = nwb + line * 32;
                 if (sl >= g.u_ring) sl -= g.u_ring;
                 const float* q0 = g.U + (long long)nA * g.u_stride + sl;
@@ -1294,19 +1217,16 @@ __global__ void fir_spectrum_packed_kernel(const double* __restrict__ taps_rev, 
 }
 
 // ---- spectrum of h in the transform's own output order (f64) -----------------------------------------------
-// odd = 0: FFT8192(h) * scale (the bins of an 8192-point segment; with scale 1/16384 the EVEN bins of a 16384-point one,
-// because h[n + 8192] = 0).  odd = 1: FFT8192(h[n] W16384^n) * scale = the ODD bins of the 16384-point spectrum.
+// FFT8192(h) / 8192: the bins of an 8192-point segment, in the order mid_pass16 reads them.
 __global__ void __launch_bounds__(kNT, 1)
-fir_spectrum_kernel(const double* __restrict__ taps_rev, int N, const double2* __restrict__ Wd, float2* __restrict__ Hout, int odd, double scale) {
+fir_spectrum_kernel(const double* __restrict__ taps_rev, int N, const double2* __restrict__ Wd, float2* __restrict__ Hout) {
     extern __shared__ double2 smem_d2[];
     C2<double>* a = reinterpret_cast<C2<double>*>(smem_d2);
     const int t = threadIdx.x;
     const Tw<double> W = load_tables<double>(a + kPadded, Wd, t);
     for (int n = t; n < kF; n += kNT) {
         const double h = n < N ? taps_rev[N - 1 - n] : 0.0;  // h[n] = taps[N-1-n]
-        double sn = 0.0, cs = 1.0;
-        if (odd) sincospi(-(double)n / (double)kF, &sn, &cs);  // W16384^n, exact argument
-        a[pad(n)] = C2<double>{h * cs, h * sn};
+        a[pad(n)] = C2<double>{h, 0.0};
     }
     __syncthreads();
     fwd_pass8<kF>(a, W, t);
@@ -1323,7 +1243,7 @@ fir_spectrum_kernel(const double* __restrict__ taps_rev, int N, const double2* _
         fft_dif<16>(v);
 #pragma unroll
         for (int s = 0; s < 16; s++)  // [k][s / 2][thread] float4 order, see mid_pass16
-            Hout[((k * 8 + (s >> 1)) * kNT + t) * 2 + (s & 1)] = make_float2((float)(v[s].x * scale), (float)(v[s].y * scale));
+            Hout[((k * 8 + (s >> 1)) * kNT + t) * 2 + (s & 1)] = make_float2((float)(v[s].x / kF), (float)(v[s].y / kF));
     }
 }
 
@@ -1369,29 +1289,24 @@ int ensure_tables() {
     return 0;
 }
 
-constexpr int kMaxCtas = 3 * 192;  // persistent grid: 3 CTAs per SM, scratch slots sized for up to 192 SMs
-constexpr size_t kWorkHeader = 2048;  // [0] next, [1] done, [8 .. 264) per-SM start counters
-
 }  // namespace
 
 int fir_fft_max_taps() { return kF / 2 + 1; }
-// H13 | packed-kernel order | H14 even | H14 odd | wide (2 F) | UPC partitions (4 x 2048 = F)
-size_t fir_fft_spectrum_bytes() { return (size_t)7 * kF * sizeof(float2); }
+// H13 (F) | packed-kernel order (F) | wide (2 F) | UPC partitions (4 x 2048 = F)
+size_t fir_fft_spectrum_bytes() { return (size_t)5 * kF * sizeof(float2); }
 int fir_upc_partitions(int n_taps) { return n_taps <= kUMaxP * kUB ? (n_taps + kUB - 1) / kUB : 0; }
 size_t fir_upc_fdl_bytes(int n_taps, int channels) { return (size_t)((channels + 1) / 2) * fir_upc_partitions(n_taps) * kUF * sizeof(float2); }
-size_t fir_fft_work_bytes() { return kWorkHeader + (size_t)kMaxCtas * (kF / 2) * sizeof(float4); }
+// [0] next item, [1] CTAs done of fir_fft_kernel; [2], [3] the same for fir_fft_wide_kernel
+size_t fir_fft_work_bytes() { return 4 * sizeof(unsigned); }
 static int effective_taps(int n) { return (n - 1 + 3) / 4 * 4 + 1; }  // Ne - 1 multiple of 4
 
-// Segment plan of one call: n14 double (16384-point) segments first, then n13 single ones.  A double segment costs
-// about kCost14 single ones (two sub-transforms + the radix-2 step and the scratch round trip) and must lie fully
-// inside the call.  DSPB_FIR_F14=0 disables double segments (the round-1 behaviour).
+// Segment plan of one call: n14 double (16384-point) segments first, the wide kernel's items, then n13 single ones for
+// fir_fft_kernel.  A double segment must lie fully inside the call, and it is used when it costs less per output than
+// single segments at the cost rule kCost14 (one double segment = kCost14 single ones) the plan has used since c4abfd4.
 static void segment_plan(int hist, int64_t T, int* n14, int* n13) {
-    static const int f14_env = getenv("DSPB_FIR_F14") ? atoi(getenv("DSPB_FIR_F14")) : -1;
     constexpr double kCost14 = 2.3;
     const int64_t V13 = kF - hist, V14 = 2 * kF - hist;
-    bool use14 = kCost14 / (double)V14 < 1.0 / (double)V13;
-    if (f14_env == 0) use14 = false;
-    if (f14_env == 1) use14 = true;
+    const bool use14 = kCost14 / (double)V14 < 1.0 / (double)V13;
     int64_t a = use14 ? T / V14 : 0;
     // the rest: single segments, unless one more double segment would be cheaper -- it would not fit, so no
     const int64_t rem = T - a * V14;
@@ -1400,8 +1315,7 @@ static void segment_plan(int hist, int64_t T, int* n14, int* n13) {
 }
 
 int launch_fir_fft(const FirPlan& fp, const float* U, int64_t u_stride, float* Y, int64_t y_stride, int c_begin, int c_end,
-                   int64_t T, int64_t started, cudaStream_t st, int* n_launches) {
-    (void)started;
+                   int64_t T, cudaStream_t st, int* n_launches) {
     if (fp.log2F != kLog2F || fp.n_taps > fir_fft_max_taps() || fp.n_taps < 1) return (int)cudaErrorInvalidValue;
     if (fp.u_ring <= 0 || (fp.u_ring & 127) || fp.hist_pad + T > fp.u_ring) return (int)cudaErrorInvalidValue;
     int rc = ensure_tables();
@@ -1444,22 +1358,18 @@ int launch_fir_fft(const FirPlan& fp, const float* U, int64_t u_stride, float* Y
     g.Y = Y;
     g.y_stride = y_stride;
     g.H13 = fp.H;
-    g.H14e = fp.H + 2 * kF;
-    g.H14o = fp.H + 3 * kF;
     g.Wg = g_tab.Wf;
     g.T = T;
     g.divisor = fp.divisor;
     g.post_nf = fp.post_nf;
     g.c_begin = c_begin;
     g.c_end = c_end;
-    segment_plan(g.hist, T, &g.n14, &g.n13);
+    int n14 = 0;
+    segment_plan(g.hist, T, &n14, &g.n13);
     const long long pairs = (c_end - c_begin + 1) / 2;
-    g.single_base = (long long)g.n14 * (2 * kF - g.hist);
+    g.single_base = (long long)n14 * (2 * kF - g.hist);
     g.work = reinterpret_cast<unsigned*>(fp.fft_work);
-    // Double segments: the wide kernel (a 16384-point transform in one piece, one CTA per SM); DSPB_FIR_WIDE=0 keeps them
-    // in the narrow kernel as two 8192-point sub-transforms.
-    static const bool wide_on = !(getenv("DSPB_FIR_WIDE") && atoi(getenv("DSPB_FIR_WIDE")) == 0);
-    if (wide_on && g.n14 > 0) {
+    if (n14 > 0) {
         static std::atomic<bool> wconf_dev[kMaxDevices];
         std::atomic<bool>& wconf = wconf_dev[current_device_slot()];
         const int wsmem = (kPadW + kTwW) * (int)sizeof(float2);
@@ -1471,31 +1381,27 @@ int launch_fir_fft(const FirPlan& fp, const float* U, int64_t u_stride, float* Y
         WideArgs w;
         w.U = U; w.u_stride = u_stride; w.u_ring = fp.u_ring; w.u_pos = fp.u_pos; w.hist = g.hist;
         w.Y = Y; w.y_stride = y_stride;
-        w.Hw = reinterpret_cast<const float4*>(fp.H + 4 * kF);
+        w.Hw = reinterpret_cast<const float4*>(fp.H + 2 * kF);
         w.Wg = g_tab.Wf;
         w.divisor = fp.divisor; w.post_nf = fp.post_nf;
         w.c_begin = c_begin; w.c_end = c_end;
-        w.n14 = g.n14;
-        const long long wi = pairs * g.n14;
+        w.n14 = n14;
+        const long long wi = pairs * n14;
         if (wi > (1ll << 30)) return (int)cudaErrorInvalidValue;
         w.n_items = (int)wi;
         w.work = g.work;
         const int wgrid = (int)std::min<long long>(wi, g_tab.n_sm);
         fir_fft_wide_kernel<<<wgrid, kNTW, wsmem, st>>>(w);
         if (n_launches) *n_launches += 1;
-        g.n14 = 0;  // the narrow kernel below only runs the single segments behind single_base
-        if (g.n13 == 0) return (int)cudaGetLastError();
     }
-    const long long n_items = pairs * (g.n14 + g.n13);
-    if (n_items <= 0 || n_items > (1ll << 30)) return (int)cudaErrorInvalidValue;
-    g.n_items = (int)n_items;
-    g.n_heavy = (int)(pairs * g.n14);
-    static const int stagger_env = getenv("DSPB_FIR_STAGGER") ? atoi(getenv("DSPB_FIR_STAGGER")) : 0;  // measured: no effect on the steady state, and a start delay is pure loss for short launches
-    g.stagger = stagger_env;
-    g.scratch = reinterpret_cast<float4*>(reinterpret_cast<char*>(fp.fft_work) + kWorkHeader);
-    const int grid = (int)std::min<long long>(n_items, std::min(kMaxCtas, 3 * g_tab.n_sm));
-    fir_fft_kernel<<<grid, kNT, smem, st>>>(g);
-    if (n_launches) *n_launches += 1;
+    if (g.n13 > 0) {
+        const long long n_items = pairs * g.n13;
+        if (n_items > (1ll << 30)) return (int)cudaErrorInvalidValue;
+        g.n_items = (int)n_items;
+        const int grid = (int)std::min<long long>(n_items, 3 * g_tab.n_sm);
+        fir_fft_kernel<<<grid, kNT, smem, st>>>(g);
+        if (n_launches) *n_launches += 1;
+    }
     return (int)cudaGetLastError();
 }
 
@@ -1517,7 +1423,7 @@ int launch_fir_upc(const FirPlan& fp, const float* U, int64_t u_stride, float* Y
     UpcArgs g;
     g.U = U; g.u_stride = u_stride; g.u_ring = fp.u_ring; g.u_pos = fp.u_pos;
     g.Y = Y; g.y_stride = y_stride;
-    g.H = reinterpret_cast<const float4*>(fp.H + 6 * kF);
+    g.H = reinterpret_cast<const float4*>(fp.H + 4 * kF);
     g.fdl = reinterpret_cast<float4*>(fp.upc_fdl);
     g.Wg = g_tab.Wf;
     g.scale = fp.post_nf != 0.0f ? (float)((double)fp.divisor / (double)fp.post_nf) : fp.divisor;
@@ -1539,13 +1445,11 @@ int fir_prepare_spectrum(int log2F, const double* taps_rev_dev, int n_taps, floa
     cudaError_t e = cudaFuncSetAttribute(fir_spectrum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return (int)e;
     cudaStream_t st = (cudaStream_t)stream;
-    fir_spectrum_kernel<<<1, kNT, smem, st>>>(taps_rev_dev, n_taps, g_tab.Wd, H_dev, 0, 1.0 / kF);
+    fir_spectrum_kernel<<<1, kNT, smem, st>>>(taps_rev_dev, n_taps, g_tab.Wd, H_dev);
     fir_spectrum_packed_kernel<<<kH2 / 128, 128, 0, st>>>(taps_rev_dev, n_taps, reinterpret_cast<float4*>(H_dev + kF));
-    fir_spectrum_kernel<<<1, kNT, smem, st>>>(taps_rev_dev, n_taps, g_tab.Wd, H_dev + 2 * kF, 0, 0.5 / kF);
-    fir_spectrum_kernel<<<1, kNT, smem, st>>>(taps_rev_dev, n_taps, g_tab.Wd, H_dev + 3 * kF, 1, 0.5 / kF);
-    fir_spectrum_wide_kernel<<<kN2 / 128, 128, 0, st>>>(taps_rev_dev, n_taps, H_dev + 4 * kF);
+    fir_spectrum_wide_kernel<<<kN2 / 128, 128, 0, st>>>(taps_rev_dev, n_taps, H_dev + 2 * kF);
     if (const int P = fir_upc_partitions(n_taps))
-        fir_spectrum_upc_kernel<<<(P * kUF + 127) / 128, 128, 0, st>>>(taps_rev_dev, n_taps, P, H_dev + 6 * kF);
+        fir_spectrum_upc_kernel<<<(P * kUF + 127) / 128, 128, 0, st>>>(taps_rev_dev, n_taps, P, H_dev + 4 * kF);
     return (int)cudaGetLastError();
 }
 

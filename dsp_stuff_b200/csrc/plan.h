@@ -176,7 +176,7 @@ struct FirPlan {
     int hist_pad;         // history samples kept in U before this call's sample 0 (>= N-1, multiple of 4)
     int u_ring;           // U rows are rings of u_ring samples (multiple of 128, >= hist_pad + T): sample i of this call
     int u_pos;            // (i in [-hist_pad, T)) lives at slot (u_pos + i) mod u_ring
-    void* fft_work;       // FIR_FFT: per-launch-lane work area of the persistent kernel (fir_fft_work_bytes())
+    void* fft_work;       // FIR_FFT: this launch lane's work counters of the persistent kernels (fir_fft_work_bytes())
     // FIR_FFT, short calls: uniformly partitioned convolution (fir_fft.cu fir_upc_kernel)
     void* upc_fdl = nullptr;      // frequency-domain delay line [pairs][P][2048] float2, or null: not eligible
     int upc_prime = 0;            // previous blocks whose spectra must be recomputed from the ring first (0 .. P - 1)
@@ -200,7 +200,7 @@ int launch_fir(const FirPlan& fp, const float* U, int64_t u_stride, float* Y, in
 int fir_prepare_spectrum(int log2F, const double* taps_rev_dev, int n_taps, float2* H_dev, void* stream);
 int fir_fft_max_taps();
 size_t fir_fft_spectrum_bytes();   // H buffer of one tap set (all spectrum tables of the FFT kernels)
-size_t fir_fft_work_bytes();       // one launch lane's work area (work counter + per-CTA scratch)
+size_t fir_fft_work_bytes();       // one launch lane's work area (the persistent kernels' work counters, zeroed once)
 int fir_upc_partitions(int n_taps);                      // 1024-tap partitions of the UPC kernel, 0 = impulse response too long
 size_t fir_upc_fdl_bytes(int n_taps, int channels);
 constexpr int kUpcBlock = 1024;
