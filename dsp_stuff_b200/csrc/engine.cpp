@@ -160,7 +160,59 @@ struct Node {
     int hist_pad = 0;
     int64_t started = 0;            // samples this node has consumed since reset
     bool fir_dirty = true;
+    // Per-channel impulse responses (dspb_node_set_taps_channels); all empty when the taps are shared.  `taps` then holds
+    // set 0 (channel 0's), so taps.size() is the one tap count of every set.
+    std::vector<double> fir_bank;   // [K x N] reversed taps of the K distinct sets, in order of first use by a channel
+    std::vector<int32_t> fir_set;   // [C] set of each channel
+    std::vector<int4> fir_xf;       // transform table {chA, chB or -1, set, 0}, see fir_transforms
+    std::vector<int> fir_xf_group;  // [ceil(C / 32) + 1] index of each 32-channel group's first transform
+    int fir_xf_single = 0;          // transforms that carry one channel
+    DevBuf set_dev, xf_dev;         // fir_set and fir_xf on the device
+    bool fir_pc() const { return !fir_set.empty(); }
 };
+
+// Transform table of per-channel impulse responses.  Two channels share one complex transform only when they use the same set.
+// Transforms are formed inside each aligned group of 32 channels: the group's channels are sorted stably by set (sets in order
+// of first appearance in the group), consecutive channels of one set are paired, and an odd one left over runs alone (B mirrors
+// A and is never stored).  Every launch range [c_begin, c_end) starts on a multiple of 32 and ends on one or at C, so it
+// covers one contiguous slice of the table, the same slice on every call.
+void fir_transforms(Node& n, int C) {
+    n.fir_xf.clear();
+    n.fir_xf_group.clear();
+    n.fir_xf_single = 0;
+    for (int g0 = 0; g0 < C; g0 += 32) {
+        n.fir_xf_group.push_back((int)n.fir_xf.size());
+        const int g1 = std::min(C, g0 + 32);
+        std::vector<int> order;   // sets of the group in order of first appearance
+        for (int c = g0; c < g1; c++)
+            if (std::find(order.begin(), order.end(), n.fir_set[c]) == order.end()) order.push_back(n.fir_set[c]);
+        for (int k : order) {
+            int pending = -1;
+            for (int c = g0; c < g1; c++) {
+                if (n.fir_set[c] != k) continue;
+                if (pending < 0) {
+                    pending = c;
+                } else {
+                    n.fir_xf.push_back(make_int4(pending, c, k, 0));
+                    pending = -1;
+                }
+            }
+            if (pending >= 0) {
+                n.fir_xf.push_back(make_int4(pending, -1, k, 0));
+                n.fir_xf_single++;
+            }
+        }
+    }
+    n.fir_xf_group.push_back((int)n.fir_xf.size());
+}
+
+void copy_fir_pc(Node& dst, const Node& src) {  // dspb_node_process: per-channel impulse responses carry over to the sub-engine
+    dst.fir_bank = src.fir_bank;
+    dst.fir_set = src.fir_set;
+    dst.fir_xf = src.fir_xf;
+    dst.fir_xf_group = src.fir_xf_group;
+    dst.fir_xf_single = src.fir_xf_single;
+}
 
 struct Link { int src, sport, dst, dport; };
 
@@ -942,6 +994,16 @@ int Lowerer::lower() {
                 else
                     snprintf(b, sizeof b, "fir step: %s, %zu taps, direct f64 sum in reference order, alg_bytes=8\n", tag.c_str(), nd.taps.size());
                 fs.text = b;
+                if (nd.fir_pc()) {
+                    fs.text.pop_back();
+                    const int K = (int)(nd.fir_bank.size() / nd.taps.size());
+                    if (e.cfg.fir_mode == FIR_FFT && (int)nd.taps.size() <= fir_fft_max_taps())   // fir_mode 2 / 3 hold no per-channel taps
+                        snprintf(b, sizeof b, ", per-channel taps: %d sets, %zu transforms (%d single-channel)\n", K, nd.fir_xf.size(),
+                                 nd.fir_xf_single);
+                    else
+                        snprintf(b, sizeof b, ", per-channel taps: %d sets\n", K);
+                    fs.text += b;
+                }
                 if (fs.fir_out_term >= 0) {
                     fs.text.pop_back();
                     fs.text += ", epilogue (0.0 + y)/1.00010002 -> output terminal " + std::to_string(fs.fir_out_term) + "\n";
@@ -1162,13 +1224,21 @@ int ensure_resources(dspb_engine* e) {
             if (r) return r;
             r = n.Y.alloc((size_t)C * maxn * 4, false, e->plan_only);
             if (r) return r;
-            r = n.H.alloc(fir_fft_spectrum_bytes(), false, e->plan_only);  // every spectrum table of the FFT kernels
+            // per-channel impulse responses: K sets of spectra and taps, set k at H + k * fir_fft_spectrum_bytes()
+            const bool pc = n.fir_pc();
+            const int K = pc ? (int)(n.fir_bank.size() / N) : 1;
+            const double* taps_host = pc ? n.fir_bank.data() : n.taps.data();
+            r = n.H.alloc(K * fir_fft_spectrum_bytes(), false, e->plan_only);  // every spectrum table of the FFT kernels
             if (r) return r;
             (void)F;
-            r = n.taps_dev.alloc((size_t)N * 8, false, e->plan_only);
+            r = n.taps_dev.alloc((size_t)K * N * 8, false, e->plan_only);
             if (r) return r;
-            if (upc_P) {
-                r = n.fdl.alloc(fir_upc_fdl_bytes(N, C), true, e->plan_only);
+            r = n.set_dev.alloc(pc ? (size_t)C * 4 : 0, false, e->plan_only);
+            if (r) return r;
+            r = n.xf_dev.alloc(pc ? n.fir_xf.size() * sizeof(int4) : 0, false, e->plan_only);
+            if (r) return r;
+            if (upc_P) {  // one delay line per transform
+                r = n.fdl.alloc(fir_upc_fdl_bytes(N, pc ? (int)n.fir_xf.size() : (C + 1) / 2), true, e->plan_only);
                 if (r) return r;
             }
             n.fdl_valid = false;
@@ -1189,12 +1259,17 @@ int ensure_resources(dspb_engine* e) {
                 if (r) return r;
             }
             if (!e->plan_only) {
-                CUDA_TRY(cudaMemcpy(n.taps_dev.p, n.taps.data(), (size_t)N * 8, cudaMemcpyHostToDevice));
+                CUDA_TRY(cudaMemcpy(n.taps_dev.p, taps_host, (size_t)K * N * 8, cudaMemcpyHostToDevice));
+                if (pc) {
+                    CUDA_TRY(cudaMemcpy(n.set_dev.p, n.fir_set.data(), (size_t)C * 4, cudaMemcpyHostToDevice));
+                    CUDA_TRY(cudaMemcpy(n.xf_dev.p, n.fir_xf.data(), n.fir_xf.size() * sizeof(int4), cudaMemcpyHostToDevice));
+                }
                 if (toep) {
                     int rc = fir_toeplitz_prepare(reinterpret_cast<const double*>(n.taps_dev.p), N, n.toep_tiles.p, nullptr);
                     if (rc) return fail(DSPB_ERR_CUDA, "fir_toeplitz_prepare: %s", cudaGetErrorString((cudaError_t)rc));
                 } else if (N <= fir_fft_max_taps()) {  // longer impulse responses run on the exact direct path
-                    int rc = fir_prepare_spectrum(e->cfg.fir_fft_log2, reinterpret_cast<const double*>(n.taps_dev.p), N, reinterpret_cast<float2*>(n.H.p), nullptr);
+                    int rc = fir_prepare_spectrum(e->cfg.fir_fft_log2, reinterpret_cast<const double*>(n.taps_dev.p), N, K,
+                                                  reinterpret_cast<float2*>(n.H.p), nullptr);
                     if (rc) return fail(DSPB_ERR_CUDA, "fir_prepare_spectrum: %s", cudaGetErrorString((cudaError_t)rc));
                 }
                 CUDA_TRY(cudaDeviceSynchronize());
@@ -1377,6 +1452,16 @@ int run_steps(dspb_engine* e, const float* const* d_in, float* const* d_out, int
             fp.u_pos = f.u_pos;
             // work counters of the persistent FFT kernels: lanes run concurrently on their own streams
             fp.fft_work = fp.mode == FIR_FFT ? f.fft_work[lane]->p : nullptr;
+            if (f.fir_pc()) {  // per-channel impulse responses: the transform-table slice of channels [c0, c1)
+                if (c0 % 32 || (c1 % 32 && c1 != e->cfg.channels))
+                    return fail(DSPB_ERR_INVALID, "per-channel taps: launch range [%d, %d) is not aligned to 32 channels", c0, c1);
+                const int x0 = f.fir_xf_group[c0 / 32], x1 = f.fir_xf_group[(c1 + 31) / 32];
+                fp.set_index = reinterpret_cast<const int*>(f.set_dev.p);
+                fp.xf = reinterpret_cast<const int4*>(f.xf_dev.p) + x0;
+                fp.n_xf = x1 - x0;
+                fp.xf0 = x0;
+                fp.h_stride = (int64_t)(fir_fft_spectrum_bytes() / sizeof(float2));
+            }
             // short calls (1 or 2 blocks of 1024): uniformly partitioned convolution with a frequency-domain delay line.  Measured
             // at 4096 channels: 62 / 101 / 141 us for 1 / 2 / 3 blocks against 92 - 104 us for the one 8192-point window the
             // segment kernel needs for any call of up to 4096 samples.
@@ -1588,6 +1673,11 @@ int dspb_node_set_taps(dspb_engine* e, int64_t node_id, const double* taps, int6
     if (n.type != T_FIR) return fail(DSPB_ERR_INVALID, "node %lld is not a fir", (long long)node_id);
     DSPB_QUIESCE(e);
     n.taps.assign(taps, taps + n_taps);
+    n.fir_bank.clear();  // shared again
+    n.fir_set.clear();
+    n.fir_xf.clear();
+    n.fir_xf_group.clear();
+    n.fir_xf_single = 0;
     n.fir_dirty = true;
     e->lowered = false;
     return DSPB_OK;
@@ -1598,6 +1688,64 @@ int dspb_node_set_impulse_response(dspb_engine* e, int64_t node_id, const double
     std::vector<double> rev(h, h + n);
     std::reverse(rev.begin(), rev.end());  // taps.reverse(), nodes/fir.rs:163-168
     return dspb_node_set_taps(e, node_id, rev.data(), n);
+}
+
+int dspb_node_set_taps_channels(dspb_engine* e, int64_t node_id, const double* taps, int64_t n_sets, int64_t n_taps,
+                                const int32_t* set_index, int64_t n_channels) {
+    if (!e) return fail(DSPB_ERR_INVALID, "null engine");
+    int i = e->find(node_id);
+    if (i < 0) return fail(DSPB_ERR_UNKNOWN_NODE, "unknown node id %lld", (long long)node_id);
+    Node& n = *e->nodes[i];
+    if (n.type != T_FIR) return fail(DSPB_ERR_INVALID, "node %lld is not a fir", (long long)node_id);
+    if (!taps || !set_index) return fail(DSPB_ERR_INVALID, "null argument");
+    if (n_sets < 1 || n_taps < 1) return fail(DSPB_ERR_INVALID, "n_sets %lld and n_taps %lld must be >= 1", (long long)n_sets, (long long)n_taps);
+    const int C = e->cfg.channels;
+    if (n_channels != C) return fail(DSPB_ERR_INVALID, "n_channels %lld != channels %d", (long long)n_channels, C);
+    for (int c = 0; c < C; c++)
+        if (set_index[c] < 0 || set_index[c] >= n_sets)
+            return fail(DSPB_ERR_INVALID, "set_index[%d] = %d is outside [0, %lld)", c, (int)set_index[c], (long long)n_sets);
+    // Deduplicate: bit-identical rows (memcmp) are one set, unused rows are dropped, sets are numbered in order of first use.
+    const size_t row_bytes = (size_t)n_taps * sizeof(double);
+    std::vector<int32_t> remap(n_sets, -1), set(C);
+    std::vector<int64_t> kept;                          // original row of each set
+    std::map<uint64_t, std::vector<int>> by_hash;       // FNV-1a of a row's bytes -> sets with that hash
+    for (int c = 0; c < C; c++) {
+        const int32_t s = set_index[c];
+        if (remap[s] < 0) {
+            const unsigned char* row = reinterpret_cast<const unsigned char*>(taps + (size_t)s * n_taps);
+            uint64_t h = 1469598103934665603ull;
+            for (size_t b = 0; b < row_bytes; b++) h = (h ^ row[b]) * 1099511628211ull;
+            auto& cand = by_hash[h];
+            for (int k : cand)
+                if (!memcmp(row, taps + (size_t)kept[k] * n_taps, row_bytes)) { remap[s] = k; break; }
+            if (remap[s] < 0) {
+                remap[s] = (int32_t)kept.size();
+                cand.push_back(remap[s]);
+                kept.push_back(s);
+            }
+        }
+        set[c] = remap[s];
+    }
+    if (kept.size() == 1) return dspb_node_set_taps(e, node_id, taps + (size_t)kept[0] * n_taps, n_taps);  // every channel alike
+    if (e->cfg.fir_mode != FIR_FFT && e->cfg.fir_mode != FIR_DIRECT)
+        return fail(DSPB_ERR_INVALID, "per-channel taps need fir_mode 0 or 1 (FFT or direct); this engine has fir_mode %d", e->cfg.fir_mode);
+    DSPB_QUIESCE(e);
+    n.fir_bank.resize(kept.size() * (size_t)n_taps);
+    for (size_t k = 0; k < kept.size(); k++) memcpy(n.fir_bank.data() + k * n_taps, taps + (size_t)kept[k] * n_taps, row_bytes);
+    n.taps.assign(n.fir_bank.begin(), n.fir_bank.begin() + n_taps);
+    n.fir_set = std::move(set);
+    fir_transforms(n, C);
+    n.fir_dirty = true;
+    e->lowered = false;
+    return DSPB_OK;
+}
+
+int dspb_node_set_impulse_response_channels(dspb_engine* e, int64_t node_id, const double* h, int64_t n_sets, int64_t n_taps,
+                                            const int32_t* set_index, int64_t n_channels) {
+    if (!h || n_sets < 1 || n_taps < 1) return fail(DSPB_ERR_INVALID, "bad impulse responses");
+    std::vector<double> rev(h, h + n_sets * n_taps);
+    for (int64_t k = 0; k < n_sets; k++) std::reverse(rev.begin() + k * n_taps, rev.begin() + (k + 1) * n_taps);  // per row, like the WAV loader
+    return dspb_node_set_taps_channels(e, node_id, rev.data(), n_sets, n_taps, set_index, n_channels);
 }
 
 int dspb_link(dspb_engine* e, int64_t src_node, const char* out_port, int64_t dst_node, const char* in_port) {
@@ -2016,16 +2164,18 @@ int dspb_node_process(dspb_engine* e, int64_t node_id, const float* const* port_
         }
         Node& dst = *sub->nodes[0];
         dst.f32 = src.f32; dst.f32_pc = src.f32_pc; dst.enums = src.enums; dst.taps = src.taps; dst.D = src.D;
+        copy_fir_pc(dst, src);
         memcpy(dst.bq, src.bq, sizeof dst.bq);
         if ((r = dspb_compile(sub))) return r;
     }
     dspb_engine* sub = ne.e;
     Node& dst = *sub->nodes[0];
     // setters on the parent node since the last call: same side effects as on the parent (after_settings_change)
-    if (dst.f32 != src.f32 || dst.f32_pc != src.f32_pc || dst.enums != src.enums || dst.taps != src.taps || dst.D != src.D) {
+    const bool taps_changed = dst.taps != src.taps || dst.fir_bank != src.fir_bank || dst.fir_set != src.fir_set;
+    if (dst.f32 != src.f32 || dst.f32_pc != src.f32_pc || dst.enums != src.enums || taps_changed || dst.D != src.D) {
         const bool f32_changed = dst.f32 != src.f32 || dst.f32_pc != src.f32_pc || dst.D != src.D;
-        const bool taps_changed = dst.taps != src.taps;
         dst.f32 = src.f32; dst.f32_pc = src.f32_pc; dst.enums = src.enums; dst.taps = src.taps; dst.D = src.D;
+        copy_fir_pc(dst, src);
         memcpy(dst.bq, src.bq, sizeof dst.bq);
         CUDA_TRY(cudaSetDevice(e->cfg.device));
         if (f32_changed && dst.type == T_BIQUAD && dst.state.p) CUDA_TRY(cudaMemset(dst.state.p, 0, dst.state.bytes));

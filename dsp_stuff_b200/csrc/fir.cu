@@ -30,12 +30,15 @@ namespace {
 constexpr int kDirectTile = 256;
 
 // One thread per output sample; the CTA's input window lives in shared memory.
+// PC: per-channel impulse responses, channel ch reads the reversed taps of its set, taps + set_index[ch] * N.
+template <bool PC>
 __global__ void __launch_bounds__(kDirectTile)
 fir_direct_kernel(const float* __restrict__ U, long long u_stride, int hist_pad, int u_ring, int u_pos, float* __restrict__ Y, long long y_stride,
                   const double* __restrict__ taps, int N, long long T, long long started, float divisor, float post_nf,
-                  int c_begin, long long n_begin, long long n_end) {
+                  int c_begin, long long n_begin, long long n_end, const int* __restrict__ set_index) {
     extern __shared__ float xw[];  // [kDirectTile + N - 1]
     const int ch = c_begin + blockIdx.y;
+    if constexpr (PC) taps += (long long)set_index[ch] * N;
     const long long tile0 = n_begin + (long long)blockIdx.x * kDirectTile;
     const long long w0 = tile0 - (N - 1);  // call-relative index of xw[0]; >= -hist_pad
     const float* row = U + (long long)ch * u_stride;  // a ring of u_ring samples, call sample n at slot (u_pos + n) mod u_ring
@@ -67,10 +70,13 @@ int launch_fir_direct(const FirPlan& fp, const float* U, int64_t u_stride, float
                       int64_t T, int64_t started, int64_t n_begin, int64_t n_end, cudaStream_t st) {
     const int N = fp.n_taps;
     const size_t smem = (size_t)(kDirectTile + N - 1) * 4;
-    static std::atomic<size_t> configured_dev[kMaxDevices];  // per device: the opt-in is a per-device function attribute
-    std::atomic<size_t>& configured = configured_dev[current_device_slot()];
+    const bool pc = fp.set_index != nullptr;
+    auto kernel = pc ? fir_direct_kernel<true> : fir_direct_kernel<false>;
+    // per device and instantiation: the opt-in is a per-device function attribute
+    static std::atomic<size_t> configured_dev[kMaxDevices][2];
+    std::atomic<size_t>& configured = configured_dev[current_device_slot()][pc];
     if (smem > 48 * 1024 && smem > configured.load(std::memory_order_acquire)) {
-        cudaError_t e = cudaFuncSetAttribute(fir_direct_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
         configured.store(smem, std::memory_order_release);
     }
@@ -79,8 +85,8 @@ int launch_fir_direct(const FirPlan& fp, const float* U, int64_t u_stride, float
     const long long tiles = (n_end - n_begin + kDirectTile - 1) / kDirectTile;
     for (int c = 0; c < C; c += 65535) {  // gridDim.y limit
         dim3 grid((unsigned)tiles, (unsigned)std::min(65535, C - c));
-        fir_direct_kernel<<<grid, kDirectTile, smem, st>>>(U, u_stride, fp.hist_pad, fp.u_ring, fp.u_pos, Y, y_stride, fp.taps, N, T, started,
-                                                          fp.divisor, fp.post_nf, c_begin + c, n_begin, n_end);
+        kernel<<<grid, kDirectTile, smem, st>>>(U, u_stride, fp.hist_pad, fp.u_ring, fp.u_pos, Y, y_stride, fp.taps, N, T, started,
+                                               fp.divisor, fp.post_nf, c_begin + c, n_begin, n_end, fp.set_index);
     }
     return (int)cudaGetLastError();
 }
@@ -92,6 +98,7 @@ int launch_fir(const FirPlan& fp, const float* U, int64_t u_stride, float* Y, in
         if (n_launches) *n_launches += 1;
         return launch_fir_direct(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, started, 0, T, st);
     }
+    if (fp.mode == FIR_TOEPLITZ && fp.set_index) return (int)cudaErrorInvalidValue;  // shared taps only
     int rc = fp.mode == FIR_TOEPLITZ ? launch_fir_toeplitz(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, st, n_launches)
              : (fp.mode == FIR_FFT && fp.upc_fdl) ? launch_fir_upc(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, st, n_launches)
                                                   : launch_fir_fft(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, st, n_launches);

@@ -20,6 +20,7 @@
 // parity bar against the reference's f64 accumulation (tests/test_gpu_fir.py).
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <atomic>
 #include <cmath>
 #include <mutex>
@@ -299,6 +300,10 @@ struct FftArgs {
     long long single_base; // first output sample of the single segments (= the wide kernel's double segments * V14)
     int n_items;           // pairs * n13
     unsigned* work;        // [0] next item, [1] CTAs done  (slots 2 / 3 belong to the wide kernel on the same lane)
+    // per-channel impulse responses only (template PC = true): a "pair" is an entry of the transform table, whose set k
+    // reads its spectrum at H13 + k * h_stride
+    const int4* xf;        // this launch's slice of the transform table {chA, chB or -1, set, 0}
+    long long h_stride;    // float2 elements per set
 };
 
 // FAST (CTA-uniform): the whole window lies inside this call's samples and does not wrap around the ring, and
@@ -412,16 +417,17 @@ __device__ __forceinline__ void inv_pass1(const C2<float>* a, const Tw<float>& W
     }
 }
 
-template <bool FAST>
-__device__ __forceinline__ void transform(C2<float>* a, const Tw<float>& W, const FftArgs& g, const float* rowA, const float* rowB,
-                                          float* outA, float* outB, bool hasB, int wb, int lim, int t) {
+// PC: the spectrum of tap set `set` (per-channel impulse responses); otherwise `set` is unused
+template <bool FAST, bool PC>
+__device__ __forceinline__ void transform(C2<float>* a, const Tw<float>& W, const FftArgs& g, int set, const float* rowA,
+                                          const float* rowB, float* outA, float* outB, bool hasB, int wb, int lim, int t) {
     fwd_pass1<FAST>(a, W, rowA, rowB, wb, g.u_ring, lim, t);
     __syncthreads();
     fwd_pass8<kF / 8>(a, W, t);
     __syncthreads();
     fwd_pass8<kF / 64>(a, W, t);
     __syncthreads();
-    mid_pass16(a, reinterpret_cast<const C2<float>*>(g.H13), t);
+    mid_pass16(a, reinterpret_cast<const C2<float>*>(PC ? g.H13 + set * g.h_stride : g.H13), t);
     __syncthreads();
     inv_pass8<kF / 64>(a, W, t);
     __syncthreads();
@@ -430,6 +436,8 @@ __device__ __forceinline__ void transform(C2<float>* a, const Tw<float>& W, cons
     inv_pass1<FAST>(a, W, outA, outB, hasB, g.hist, lim, g.divisor, g.post_nf, t);
 }
 
+// PC: per-channel impulse responses (see FftArgs::xf); PC = false is the shared-taps kernel.
+template <bool PC>
 __global__ void __launch_bounds__(kNT, 3)
 fir_fft_kernel(const __grid_constant__ FftArgs g) {
     extern __shared__ float2 smem_f2[];
@@ -445,8 +453,9 @@ fir_fft_kernel(const __grid_constant__ FftArgs g) {
         const int item = s_item;
         if (item >= g.n_items) break;
         const int pr = item / g.n13, sg = item - pr * g.n13;
-        const int chA = g.c_begin + 2 * pr, chB = chA + 1;
-        const bool hasB = chB < g.c_end;
+        const int4 x = PC ? g.xf[pr] : int4{};   // per-channel taps: {chA, chB or -1, set} of transform pr
+        const int chA = PC ? x.x : g.c_begin + 2 * pr, chB = PC ? x.y : chA + 1;
+        const bool hasB = PC ? chB >= 0 : chB < g.c_end;
         const long long s0 = g.single_base + (long long)sg * V13;
         const long long w0 = s0 - g.hist;                      // call-relative index of window sample 0 (>= -hist)
         const long long lim_ll = g.T - w0;                     // window samples >= lim lie beyond this call's input: zeros
@@ -457,9 +466,9 @@ fir_fft_kernel(const __grid_constant__ FftArgs g) {
         float* outA = g.Y + (long long)chA * g.y_stride + w0;
         float* outB = g.Y + (long long)(hasB ? chB : chA) * g.y_stride + w0;
         if (g.hist == kF / 2 && lim == kF && wb + kF <= g.u_ring)
-            transform<true>(a, W, g, rowA, rowB, outA, outB, hasB, wb, lim, t);
+            transform<true, PC>(a, W, g, x.z, rowA, rowB, outA, outB, hasB, wb, lim, t);
         else
-            transform<false>(a, W, g, rowA, rowB, outA, outB, hasB, wb, lim, t);
+            transform<false, PC>(a, W, g, x.z, rowA, rowB, outA, outB, hasB, wb, lim, t);
     }
     // the last CTA out re-arms the work counter for the next launch on this lane (stream-ordered behind this one)
     if (t == 0) {
@@ -506,8 +515,11 @@ struct WideArgs {
     int n14;               // double segments per channel pair (all lie fully inside the call)
     int n_items;           // pairs * n14
     unsigned* work;        // [2] next item, [3] CTAs done  (slots 0 / 1 belong to fir_fft_kernel on the same lane)
+    const int4* xf;        // PC = true: transform table slice, set k's table at Hw + k * h_stride / 2 (see FftArgs)
+    long long h_stride;
 };
 
+template <bool PC>
 __global__ void __launch_bounds__(kNTW, 1)
 fir_fft_wide_kernel(const __grid_constant__ WideArgs g) {
     extern __shared__ float2 smem_f2[];
@@ -530,8 +542,9 @@ fir_fft_wide_kernel(const __grid_constant__ WideArgs g) {
         if (item >= g.n_items) break;
         if (t == 0) s_item[(it + 1) & 1] = (int)atomicAdd(g.work + 2, 1u);  // the next item: known one item ahead (L2 prefetch)
         const int pr = item / g.n14, sg = item - pr * g.n14;
-        const int chA = g.c_begin + 2 * pr, chB = chA + 1;
-        const bool hasB = chB < g.c_end;
+        const int4 x = PC ? g.xf[pr] : int4{};   // per-channel taps: {chA, chB or -1, set} of transform pr
+        const int chA = PC ? x.x : g.c_begin + 2 * pr, chB = PC ? x.y : chA + 1;
+        const bool hasB = PC ? chB >= 0 : chB < g.c_end;
         const long long w0 = (long long)sg * V14 - g.hist;          // call-relative index of window sample 0
         const int wb = ring_slot(g.u_pos, (int)w0, g.u_ring);       // its ring slot; the window holds kN2 <= u_ring samples
         const float* rowA = g.U + (long long)chA * g.u_stride;
@@ -574,14 +587,15 @@ fir_fft_wide_kernel(const __grid_constant__ WideArgs g) {
             const int nxt = s_item[(it + 1) & 1];
             if (nxt < g.n_items) {
                 const int npr = nxt / g.n14, nsg = nxt - npr * g.n14;
-                const int nA = g.c_begin + 2 * npr;
+                const int4 nx = PC ? g.xf[npr] : int4{};   // per-channel taps: the next item's table entry
+                const int nA = PC ? nx.x : g.c_begin + 2 * npr;
                 const int nwb = ring_slot(g.u_pos, (int)((long long)nsg * V14 - g.hist), g.u_ring);
                 // 2 rows x 16384 floats = 1024 lines of 128 bytes: two per thread
                 const int line = t & 511;
                 int sl = nwb + line * 32;
                 if (sl >= g.u_ring) sl -= g.u_ring;
                 const float* q0 = g.U + (long long)nA * g.u_stride + sl;
-                const float* q1 = g.U + (long long)(nA + 1 < g.c_end ? nA + 1 : nA) * g.u_stride + sl;
+                const float* q1 = g.U + (long long)(PC ? (nx.y >= 0 ? nx.y : nA) : (nA + 1 < g.c_end ? nA + 1 : nA)) * g.u_stride + sl;
                 asm volatile("prefetch.global.L2 [%0];" ::"l"(q0));
                 asm volatile("prefetch.global.L2 [%0];" ::"l"(q1));
             }
@@ -605,7 +619,7 @@ fir_fft_wide_kernel(const __grid_constant__ WideArgs g) {
         // ---- middle: radix 32 on contiguous points . spectrum . inverse radix 32
         {
             float4* p4 = reinterpret_cast<float4*>(a + padw(32 * t));   // 32 contiguous points, no pad inside, 16-byte aligned
-            const float4* h4 = g.Hw + t;
+            const float4* h4 = (PC ? g.Hw + x.z * (g.h_stride / 2) : g.Hw) + t;
             C2<float> v[32];
 #pragma unroll
             for (int q = 0; q < 16; q++) {
@@ -680,9 +694,12 @@ fir_fft_wide_kernel(const __grid_constant__ WideArgs g) {
 // Spectrum for the wide kernel: H16384[f] / 16384 by direct f64 summation (exact argument reduction), stored where the
 // middle pass of thread u finds it: float4 [q * 512 + u] = (H[f(32 u + 2 q)], H[f(32 u + 2 q + 1)]),
 // f(p) = k1 + 16 k2 + 512 bitrev5(s) for p = k1 * 1024 + k2 * 32 + s.
-__global__ void fir_spectrum_wide_kernel(const double* __restrict__ taps_rev, int N, float2* __restrict__ Hout) {
+// blockIdx.y: tap set (taps_rev + set * N, Hout + set * stride), here and in the other spectrum kernels.
+__global__ void fir_spectrum_wide_kernel(const double* __restrict__ taps_rev, int N, float2* __restrict__ Hout, long long stride) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= kN2) return;
+    taps_rev += (long long)blockIdx.y * N;
+    Hout += blockIdx.y * stride;
     const int k1 = p >> 10, k2 = (p >> 5) & 31, sreg = p & 31;
     const int f = k1 + 16 * k2 + 512 * bitrev5(sreg);
     double re = 0.0, im = 0.0;
@@ -733,9 +750,12 @@ struct UpcArgs {
     int c_begin, c_end;
     int P, n_blocks, prime;
     long long b0;          // running block counter of the call's first block (FDL slot = counter mod P)
-    int pair0;             // first channel pair of this launch inside the FDL
+    int pair0;             // first channel pair (PC: first transform of the slice) of this launch inside the FDL
+    const int4* xf;        // PC = true: transform table slice, set k's partitions at H + k * h_stride / 2 (see FftArgs)
+    long long h_stride;
 };
 
+template <bool PC>
 __global__ void __launch_bounds__(kUNT, 8)
 fir_upc_kernel(const __grid_constant__ UpcArgs g) {
     extern __shared__ float2 smem_f2[];
@@ -751,8 +771,9 @@ fir_upc_kernel(const __grid_constant__ UpcArgs g) {
     const Tw<float> W{tabs, tabs + kCoarse, nullptr};
     const C2<float>* T2 = tabs + kCoarse + kFine;
     const int pr = blockIdx.x;
-    const int chA = g.c_begin + 2 * pr, chB = chA + 1;
-    const bool hasB = chB < g.c_end;
+    const int4 x = PC ? g.xf[pr] : int4{};   // per-channel taps: {chA, chB or -1, set} of transform pr
+    const int chA = PC ? x.x : g.c_begin + 2 * pr, chB = PC ? x.y : chA + 1;
+    const bool hasB = PC ? chB >= 0 : chB < g.c_end;
     const float* rowA = g.U + (long long)chA * g.u_stride;
     const float* rowB = g.U + (long long)(hasB ? chB : chA) * g.u_stride;
     float4* fdl = g.fdl + (size_t)(g.pair0 + pr) * g.P * 1024;
@@ -826,7 +847,7 @@ fir_upc_kernel(const __grid_constant__ UpcArgs g) {
             if (blk < 0) continue;   // prime block: only its spectrum is needed
             C2<float> acc[8];
             {
-                const float4* h = g.H + ((size_t)(0 * 2 + q) * 4) * kUNT + t;
+                const float4* h = (PC ? g.H + x.z * (g.h_stride / 2) : g.H) + ((size_t)(0 * 2 + q) * 4) * kUNT + t;
 #pragma unroll
                 for (int s2 = 0; s2 < 4; s2++) {
                     const float4 hh = __ldg(h + s2 * kUNT);
@@ -837,7 +858,7 @@ fir_upc_kernel(const __grid_constant__ UpcArgs g) {
             for (int pp = 1; pp < g.P; pp++) {
                 const int sl2 = (int)((((bidx - pp) % g.P) + g.P) % g.P);
                 const float4* xo = fdl + ((size_t)(sl2 * 2 + q) * 4) * kUNT + t;
-                const float4* h = g.H + ((size_t)(pp * 2 + q) * 4) * kUNT + t;
+                const float4* h = (PC ? g.H + x.z * (g.h_stride / 2) : g.H) + ((size_t)(pp * 2 + q) * 4) * kUNT + t;
 #pragma unroll
                 for (int s2 = 0; s2 < 4; s2++) {
                     const float4 x = __ldcg(xo + s2 * kUNT);
@@ -892,9 +913,11 @@ fir_upc_kernel(const __grid_constant__ UpcArgs g) {
 
 // Partition spectra for the UPC kernel, by direct f64 summation, in the middle pass's order:
 // float4 [((p * 2 + q) * 4 + s2) * 128 + t] = (H_p[f(8 u + 2 s2)], H_p[f(8 u + 2 s2 + 1)]), u = t + 128 q.
-__global__ void fir_spectrum_upc_kernel(const double* __restrict__ taps_rev, int N, int P, float2* __restrict__ Hout) {
+__global__ void fir_spectrum_upc_kernel(const double* __restrict__ taps_rev, int N, int P, float2* __restrict__ Hout, long long stride) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= P * kUF) return;
+    taps_rev += (long long)blockIdx.y * N;
+    Hout += blockIdx.y * stride;
     const int p = idx / kUF, pos = idx % kUF;
     const int k1 = pos >> 7, k2 = (pos >> 3) & 15, sreg = pos & 7;
     const int f = k1 + 16 * k2 + 256 * bitrev3(sreg);
@@ -1191,9 +1214,11 @@ fir_fft_packed_kernel(const float* __restrict__ U, long long u_stride, int hist_
 // argument reduction: f n mod F is an integer), scaled by 1/F, stored where pass 3 of the packed kernel finds
 // it: float4 [(k * 8 + s) * 256 + t] = (H[2 f'].re, H[2 f' + 1].re, H[2 f'].im, H[2 f' + 1].im) with
 // f' = d3 + 8 d2 + 64 d1 + 512 d0, (d3, d2, d1) the base-8 digits of u = t + 256 k, d0 = bitrev3(s).
-__global__ void fir_spectrum_packed_kernel(const double* __restrict__ taps_rev, int N, float4* __restrict__ Hout) {
+__global__ void fir_spectrum_packed_kernel(const double* __restrict__ taps_rev, int N, float4* __restrict__ Hout, long long stride4) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;  // [k][s][t]
     if (idx >= kH2) return;
+    taps_rev += (long long)blockIdx.y * N;
+    Hout += blockIdx.y * stride4;
     const int tt = idx % kNT, s = (idx / kNT) % 8, k = idx / (8 * kNT);
     const int u = tt + kNT * k;
     const int d3 = u / 64, d2 = (u / 8) % 8, d1 = u % 8, d0 = bitrev3(s);
@@ -1219,8 +1244,10 @@ __global__ void fir_spectrum_packed_kernel(const double* __restrict__ taps_rev, 
 // ---- spectrum of h in the transform's own output order (f64) -----------------------------------------------
 // FFT8192(h) / 8192: the bins of an 8192-point segment, in the order mid_pass16 reads them.
 __global__ void __launch_bounds__(kNT, 1)
-fir_spectrum_kernel(const double* __restrict__ taps_rev, int N, const double2* __restrict__ Wd, float2* __restrict__ Hout) {
+fir_spectrum_kernel(const double* __restrict__ taps_rev, int N, const double2* __restrict__ Wd, float2* __restrict__ Hout, long long stride) {
     extern __shared__ double2 smem_d2[];
+    taps_rev += (long long)blockIdx.y * N;
+    Hout += blockIdx.y * stride;
     C2<double>* a = reinterpret_cast<C2<double>*>(smem_d2);
     const int t = threadIdx.x;
     const Tw<double> W = load_tables<double>(a + kPadded, Wd, t);
@@ -1295,7 +1322,7 @@ int fir_fft_max_taps() { return kF / 2 + 1; }
 // H13 (F) | packed-kernel order (F) | wide (2 F) | UPC partitions (4 x 2048 = F)
 size_t fir_fft_spectrum_bytes() { return (size_t)5 * kF * sizeof(float2); }
 int fir_upc_partitions(int n_taps) { return n_taps <= kUMaxP * kUB ? (n_taps + kUB - 1) / kUB : 0; }
-size_t fir_upc_fdl_bytes(int n_taps, int channels) { return (size_t)((channels + 1) / 2) * fir_upc_partitions(n_taps) * kUF * sizeof(float2); }
+size_t fir_upc_fdl_bytes(int n_taps, int transforms) { return (size_t)transforms * fir_upc_partitions(n_taps) * kUF * sizeof(float2); }
 // [0] next item, [1] CTAs done of fir_fft_kernel; [2], [3] the same for fir_fft_wide_kernel
 size_t fir_fft_work_bytes() { return 4 * sizeof(unsigned); }
 static int effective_taps(int n) { return (n - 1 + 3) / 4 * 4 + 1; }  // Ne - 1 multiple of 4
@@ -1321,6 +1348,7 @@ int launch_fir_fft(const FirPlan& fp, const float* U, int64_t u_stride, float* Y
     int rc = ensure_tables();
     if (rc) return rc;
     if (fp.mode == FIR_FFT_PACKED) {  // opt-in: measured 5 % slower than the scalar kernel (see the comment above VF)
+        if (fp.xf) return (int)cudaErrorInvalidValue;  // shared taps only
         static std::atomic<bool> configured2_dev[kMaxDevices];
         std::atomic<bool>& configured2 = configured2_dev[current_device_slot()];
         const int smem2 = (kH2 + kCoarse + kFineP) * (int)sizeof(float4);
@@ -1341,11 +1369,13 @@ int launch_fir_fft(const FirPlan& fp, const float* U, int64_t u_stride, float* Y
         return (int)cudaGetLastError();
     }
     if (!fp.fft_work) return (int)cudaErrorInvalidValue;
-    static std::atomic<bool> configured_dev[kMaxDevices];
-    std::atomic<bool>& configured = configured_dev[current_device_slot()];
+    const bool pc = fp.xf != nullptr;
+    auto narrow = pc ? fir_fft_kernel<true> : fir_fft_kernel<false>;
+    static std::atomic<bool> configured_dev[kMaxDevices][2];
+    std::atomic<bool>& configured = configured_dev[current_device_slot()][pc];
     const int smem = (kPadded + kTwEntries) * (int)sizeof(float2);
     if (!configured.load(std::memory_order_acquire)) {
-        cudaError_t e = cudaFuncSetAttribute(fir_fft_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaError_t e = cudaFuncSetAttribute(narrow, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return (int)e;
         configured.store(true, std::memory_order_release);
     }
@@ -1364,17 +1394,20 @@ int launch_fir_fft(const FirPlan& fp, const float* U, int64_t u_stride, float* Y
     g.post_nf = fp.post_nf;
     g.c_begin = c_begin;
     g.c_end = c_end;
+    g.xf = fp.xf;
+    g.h_stride = fp.h_stride;
     int n14 = 0;
     segment_plan(g.hist, T, &n14, &g.n13);
-    const long long pairs = (c_end - c_begin + 1) / 2;
+    const long long pairs = pc ? fp.n_xf : (c_end - c_begin + 1) / 2;  // per-channel taps: the table slice's transforms
     g.single_base = (long long)n14 * (2 * kF - g.hist);
     g.work = reinterpret_cast<unsigned*>(fp.fft_work);
     if (n14 > 0) {
-        static std::atomic<bool> wconf_dev[kMaxDevices];
-        std::atomic<bool>& wconf = wconf_dev[current_device_slot()];
+        auto wide = pc ? fir_fft_wide_kernel<true> : fir_fft_wide_kernel<false>;
+        static std::atomic<bool> wconf_dev[kMaxDevices][2];
+        std::atomic<bool>& wconf = wconf_dev[current_device_slot()][pc];
         const int wsmem = (kPadW + kTwW) * (int)sizeof(float2);
         if (!wconf.load(std::memory_order_acquire)) {
-            cudaError_t e = cudaFuncSetAttribute(fir_fft_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, wsmem);
+            cudaError_t e = cudaFuncSetAttribute(wide, cudaFuncAttributeMaxDynamicSharedMemorySize, wsmem);
             if (e != cudaSuccess) return (int)e;
             wconf.store(true, std::memory_order_release);
         }
@@ -1386,12 +1419,14 @@ int launch_fir_fft(const FirPlan& fp, const float* U, int64_t u_stride, float* Y
         w.divisor = fp.divisor; w.post_nf = fp.post_nf;
         w.c_begin = c_begin; w.c_end = c_end;
         w.n14 = n14;
+        w.xf = fp.xf;
+        w.h_stride = fp.h_stride;
         const long long wi = pairs * n14;
         if (wi > (1ll << 30)) return (int)cudaErrorInvalidValue;
         w.n_items = (int)wi;
         w.work = g.work;
         const int wgrid = (int)std::min<long long>(wi, g_tab.n_sm);
-        fir_fft_wide_kernel<<<wgrid, kNTW, wsmem, st>>>(w);
+        wide<<<wgrid, kNTW, wsmem, st>>>(w);
         if (n_launches) *n_launches += 1;
     }
     if (g.n13 > 0) {
@@ -1399,7 +1434,7 @@ int launch_fir_fft(const FirPlan& fp, const float* U, int64_t u_stride, float* Y
         if (n_items > (1ll << 30)) return (int)cudaErrorInvalidValue;
         g.n_items = (int)n_items;
         const int grid = (int)std::min<long long>(n_items, 3 * g_tab.n_sm);
-        fir_fft_kernel<<<grid, kNT, smem, st>>>(g);
+        narrow<<<grid, kNT, smem, st>>>(g);
         if (n_launches) *n_launches += 1;
     }
     return (int)cudaGetLastError();
@@ -1412,11 +1447,13 @@ int launch_fir_upc(const FirPlan& fp, const float* U, int64_t u_stride, float* Y
     if (!P || T % kUB || !fp.upc_fdl || fp.hist_pad < P * kUB || fp.hist_pad + T > fp.u_ring) return (int)cudaErrorInvalidValue;
     int rc = ensure_tables();
     if (rc) return rc;
-    static std::atomic<bool> conf_dev[kMaxDevices];
-    std::atomic<bool>& conf = conf_dev[current_device_slot()];
+    const bool pc = fp.xf != nullptr;
+    auto kernel = pc ? fir_upc_kernel<true> : fir_upc_kernel<false>;
+    static std::atomic<bool> conf_dev[kMaxDevices][2];
+    std::atomic<bool>& conf = conf_dev[current_device_slot()][pc];
     const int smem = (kUPad + kUTw) * (int)sizeof(float2);
     if (!conf.load(std::memory_order_acquire)) {
-        cudaError_t e = cudaFuncSetAttribute(fir_upc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return (int)e;
         conf.store(true, std::memory_order_release);
     }
@@ -1430,26 +1467,35 @@ int launch_fir_upc(const FirPlan& fp, const float* U, int64_t u_stride, float* Y
     g.c_begin = c_begin; g.c_end = c_end;
     g.P = P; g.n_blocks = (int)(T / kUB); g.prime = fp.upc_prime;
     g.b0 = fp.upc_block0;
-    g.pair0 = c_begin / 2;
-    const int pairs = (c_end - c_begin + 1) / 2;
-    fir_upc_kernel<<<pairs, kUNT, smem, st>>>(g);
+    g.pair0 = pc ? fp.xf0 : c_begin / 2;   // per-channel taps: delay-line slot = transform index
+    g.xf = fp.xf;
+    g.h_stride = fp.h_stride;
+    const int pairs = pc ? fp.n_xf : (c_end - c_begin + 1) / 2;
+    if (pairs <= 0) return 0;
+    kernel<<<pairs, kUNT, smem, st>>>(g);
     if (n_launches) *n_launches += 1;
     return (int)cudaGetLastError();
 }
 
-int fir_prepare_spectrum(int log2F, const double* taps_rev_dev, int n_taps, float2* H_dev, void* stream) {
-    if (log2F != kLog2F || n_taps > fir_fft_max_taps()) return (int)cudaErrorInvalidValue;
+int fir_prepare_spectrum(int log2F, const double* taps_rev_dev, int n_taps, int n_sets, float2* H_dev, void* stream) {
+    if (log2F != kLog2F || n_taps > fir_fft_max_taps() || n_sets < 1) return (int)cudaErrorInvalidValue;
     int rc = ensure_tables();
     if (rc) return rc;
     const int smem = (kPadded + kTwEntries) * (int)sizeof(double2);
     cudaError_t e = cudaFuncSetAttribute(fir_spectrum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return (int)e;
     cudaStream_t st = (cudaStream_t)stream;
-    fir_spectrum_kernel<<<1, kNT, smem, st>>>(taps_rev_dev, n_taps, g_tab.Wd, H_dev);
-    fir_spectrum_packed_kernel<<<kH2 / 128, 128, 0, st>>>(taps_rev_dev, n_taps, reinterpret_cast<float4*>(H_dev + kF));
-    fir_spectrum_wide_kernel<<<kN2 / 128, 128, 0, st>>>(taps_rev_dev, n_taps, H_dev + 2 * kF);
-    if (const int P = fir_upc_partitions(n_taps))
-        fir_spectrum_upc_kernel<<<(P * kUF + 127) / 128, 128, 0, st>>>(taps_rev_dev, n_taps, P, H_dev + 4 * kF);
+    const long long S = 5 * kF;   // float2 elements per set: fir_fft_spectrum_bytes()
+    for (int k0 = 0; k0 < n_sets; k0 += 65535) {  // gridDim.y limit: one launch per table kind and 65535 sets
+        const unsigned ns = (unsigned)std::min(65535, n_sets - k0);
+        const double* tr = taps_rev_dev + (size_t)k0 * n_taps;
+        float2* H = H_dev + k0 * S;
+        fir_spectrum_kernel<<<dim3(1, ns), kNT, smem, st>>>(tr, n_taps, g_tab.Wd, H, S);
+        fir_spectrum_packed_kernel<<<dim3(kH2 / 128, ns), 128, 0, st>>>(tr, n_taps, reinterpret_cast<float4*>(H + kF), S / 2);
+        fir_spectrum_wide_kernel<<<dim3(kN2 / 128, ns), 128, 0, st>>>(tr, n_taps, H + 2 * kF, S);
+        if (const int P = fir_upc_partitions(n_taps))
+            fir_spectrum_upc_kernel<<<dim3((P * kUF + 127) / 128, ns), 128, 0, st>>>(tr, n_taps, P, H + 4 * kF, S);
+    }
     return (int)cudaGetLastError();
 }
 

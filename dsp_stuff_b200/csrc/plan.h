@@ -191,18 +191,27 @@ struct FirPlan {
     const void* toep_tiles = nullptr;
     void* toep_split = nullptr;
     int64_t toep_max_samples = 0;
+    // Per-channel impulse responses (dspb_node_set_taps_channels), FIR_FFT and FIR_DIRECT only; all null / zero when the
+    // taps are shared.  Set k's spectra start at H + k * h_stride and its reversed taps at taps + k * n_taps.
+    const int* set_index = nullptr;  // [C] set of each (absolute) channel: the direct kernel
+    const int4* xf = nullptr;        // this launch's slice of the transform table: {chA, chB or -1, set, 0} per transform
+    int n_xf = 0;                    // transforms in the slice (channels [c_begin, c_end) are exactly theirs)
+    int xf0 = 0;                     // index of the slice's first transform in the whole table (UPC delay-line slot)
+    int64_t h_stride = 0;            // float2 elements per set in H (fir_fft_spectrum_bytes() / 8)
 };
 // U: [C x u_ring] input rings (see FirPlan::u_ring / u_pos), u_stride = row pitch; Y: [C x T] output.
 // started = samples seen before this call.
 int launch_fir(const FirPlan& fp, const float* U, int64_t u_stride, float* Y, int64_t y_stride, int c_begin, int c_end,
                int64_t T, int64_t started, void* stream, int* n_launches);
-// Computes H from the (device-resident, reversed, f64) taps with the kernel's own forward passes in f64.
-int fir_prepare_spectrum(int log2F, const double* taps_rev_dev, int n_taps, float2* H_dev, void* stream);
+// Computes H from the (device-resident, reversed, f64) taps with the kernel's own forward passes in f64.  n_sets tap sets
+// stored one after the other ([n_sets x n_taps]) give n_sets spectra, set k at H_dev + k * fir_fft_spectrum_bytes() / 8,
+// in one launch per table kind.
+int fir_prepare_spectrum(int log2F, const double* taps_rev_dev, int n_taps, int n_sets, float2* H_dev, void* stream);
 int fir_fft_max_taps();
 size_t fir_fft_spectrum_bytes();   // H buffer of one tap set (all spectrum tables of the FFT kernels)
 size_t fir_fft_work_bytes();       // one launch lane's work area (the persistent kernels' work counters, zeroed once)
 int fir_upc_partitions(int n_taps);                      // 1024-tap partitions of the UPC kernel, 0 = impulse response too long
-size_t fir_upc_fdl_bytes(int n_taps, int channels);
+size_t fir_upc_fdl_bytes(int n_taps, int transforms);     // delay line of `transforms` channel pairs (shared taps: ceil(C / 2))
 constexpr int kUpcBlock = 1024;
 // device-boundary format steps (boundary.cu): stereo fold a + b, mono -> stereo duplicate; flat [C * n] streams
 int launch_fold_stereo(const float* interleaved, float* mono, long long total_mono, cudaStream_t st);

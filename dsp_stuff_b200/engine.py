@@ -56,6 +56,7 @@ ABI_SYMBOLS = [
     "dspb_load_graph_json", "dspb_compile", "dspb_process", "dspb_node_process", "dspb_reset_state",
     "dspb_node_get_i64", "dspb_node_port_index", "dspb_describe_plan", "dspb_profile_enable", "dspb_profile_read",
     "dspb_fold_stereo", "dspb_dup_stereo", "dspb_resample_dup_stereo", "dspb_sync", "dspb_node_set_f32_channels",
+    "dspb_node_set_taps_channels", "dspb_node_set_impulse_response_channels",
 ]
 
 _lib = None
@@ -81,6 +82,8 @@ def load_library(path: Optional[str] = None):
     L.dspb_node_set_enum.argtypes = [vp, i64, cp, cp]
     L.dspb_node_set_taps.argtypes = [vp, i64, vp, i64]
     L.dspb_node_set_impulse_response.argtypes = [vp, i64, vp, i64]
+    L.dspb_node_set_taps_channels.argtypes = [vp, i64, vp, i64, i64, vp, i64]
+    L.dspb_node_set_impulse_response_channels.argtypes = [vp, i64, vp, i64, i64, vp, i64]
     L.dspb_link.argtypes = [vp, i64, cp, i64, cp]
     L.dspb_load_graph_json.argtypes = [vp, cp]
     L.dspb_compile.argtypes = [vp]
@@ -162,6 +165,23 @@ class Engine:
     def set_impulse_response(self, node_id: int, h):
         t = np.ascontiguousarray(h, dtype=np.float64)
         self._ck(self._L.dspb_node_set_impulse_response(self._h, node_id, t.ctypes.data, t.size))
+
+    def set_taps_channels(self, node_id: int, bank, set_index):
+        """Per-channel impulse responses: bank [K, N] float64 (rows reversed like set_taps), set_index [channels] int32.
+        Channel c runs as if set_taps(bank[set_index[c]]) had been called on an engine holding only channel c.  Identical
+        rows are one set; all channels alike = set_taps(row).  A later set_taps / set_impulse_response makes it shared."""
+        self._set_bank(self._L.dspb_node_set_taps_channels, node_id, bank, set_index)
+
+    def set_impulse_response_channels(self, node_id: int, bank, set_index):
+        """Same as set_taps_channels with impulse responses in time order (each row reversed like set_impulse_response)."""
+        self._set_bank(self._L.dspb_node_set_impulse_response_channels, node_id, bank, set_index)
+
+    def _set_bank(self, fn, node_id, bank, set_index):
+        b = np.ascontiguousarray(bank, dtype=np.float64)
+        if b.ndim == 1:
+            b = b.reshape(1, -1)
+        s = np.ascontiguousarray(set_index, dtype=np.int32).reshape(-1)
+        self._ck(fn(self._h, node_id, b.ctypes.data, b.shape[0], b.shape[1], s.ctypes.data, s.size))
 
     def link(self, src: int, out_port: str, dst: int, in_port: str):
         self._ck(self._L.dspb_link(self._h, src, out_port.encode(), dst, in_port.encode()))

@@ -1,7 +1,9 @@
 """Channel sharding across ranks (SURVEY.md section 8e): every channel owns its state, shared parameters are
 replicated and per-channel ones (Engine.set_f32_channels) are sliced: rank r's engine gets values[lo:hi] with
-(lo, hi) = channel_range(r, ...).  So the path partitions with no data-path collective.  The only collective is the
-optional gather of output blocks to rank 0."""
+(lo, hi) = channel_range(r, ...).  Per-channel impulse responses (Engine.set_taps_channels) pass the whole bank with
+set_index[lo:hi].  So the path partitions with no data-path collective.  The only collective is the optional gather of
+output blocks to rank 0.  The FFT FIR pairs channels of one impulse response inside aligned groups of 32 channels, so a
+shard whose lo is a multiple of 32 reproduces the whole run bit for bit; other boundaries agree within rounding."""
 from __future__ import annotations
 
 from typing import Optional, Tuple

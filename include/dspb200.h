@@ -12,8 +12,9 @@
  *   streams.  All audio is f32, laid out channel-major: buffer[c * n + i] is
  *   sample i of channel c ("[C x n] SoA rows").  Filter/delay/FIR state is per
  *   channel.  Parameters are shared by all channels unless a field is given one
- *   value per channel (dspb_node_set_f32_channels); FIR taps, enum fields and
- *   reverb.seconds are always shared.
+ *   value per channel (dspb_node_set_f32_channels) or a FIR node one impulse
+ *   response per channel (dspb_node_set_taps_channels); enum fields,
+ *   reverb.seconds and the FIR tap count are always shared.
  *
  * Threading: one caller thread per engine handle at a time; setters are legal
  * between dspb_process calls and take effect at the next call (the reference
@@ -136,6 +137,34 @@ int dspb_node_set_enum(dspb_engine* e, int64_t node_id, const char* field, const
 int dspb_node_set_taps(dspb_engine* e, int64_t node_id, const double* taps, int64_t n);
 /* Convenience for callers holding an impulse response h[0..n): reverses like the WAV loader. */
 int dspb_node_set_impulse_response(dspb_engine* e, int64_t node_id, const double* h, int64_t n);
+
+/* Per-channel impulse responses.  taps: [n_sets x n_taps] f64, row k stored REVERSED like dspb_node_set_taps;
+ * set_index: [n_channels] int32, channel c runs FIR node `node_id` as if dspb_node_set_taps(taps + set_index[c] * n_taps,
+ * n_taps) had been called on a one-channel engine holding only channel c.  Host pointers.
+ *   - A bank plus an index: 4096 streams sharing 8 impulse responses pass 8 rows.  Bit-identical rows (memcmp over the
+ *     8 * n_taps bytes) count as one set; rows no channel uses are dropped.
+ *   - Every used row bit-identical: exactly dspb_node_set_taps(row), same plan, kernels and outputs.  This holds in every
+ *     fir_mode (the check comes before the fir_mode check below).
+ *   - Side effects are those of dspb_node_set_taps: the node's history is cleared for every channel, and the change takes
+ *     effect at the next dspb_process.  A later dspb_node_set_taps / dspb_node_set_impulse_response makes the node shared again.
+ *   - One tap count for all channels: the Average divisor 1/n_taps and the warm-up length (n_taps - 1 samples) are one value
+ *     per node.
+ *   - Cost (fir_mode 0): two channels share one complex transform only when they use the same set.  Channels are paired
+ *     inside each aligned group of 32 channels; a set with an odd number of channels in a group leaves one channel that runs
+ *     alone.  So a bank whose sets hold an even number of channels in every group runs as many transforms as shared taps,
+ *     and fully distinct impulse responses run one channel per transform, about twice the FFT work.  Each set keeps its own
+ *     320 KiB of spectra on the device.
+ *   - Errors: DSPB_ERR_UNKNOWN_NODE (node id); DSPB_ERR_INVALID (not a fir node, null pointer, n_sets < 1, n_taps < 1,
+ *     n_channels != channels, a set_index outside [0, n_sets), distinct sets on an engine with fir_mode 2 or 3: per-channel
+ *     taps need fir_mode 0 or 1).
+ *   - Planning engines (device -1) accept the call; dspb_describe_plan adds ", per-channel taps: K sets, X transforms
+ *     (Y single-channel)" to the fir step line (", per-channel taps: K sets" on the direct path).
+ *   - Not stored in saved-graph JSON (one taps array per node there).  dspb_node_process carries them over. */
+int dspb_node_set_taps_channels(dspb_engine* e, int64_t node_id, const double* taps, int64_t n_sets, int64_t n_taps,
+                                const int32_t* set_index, int64_t n_channels);
+/* Same with impulse responses h (each row h[0..n_taps) in time order, reversed per row like dspb_node_set_impulse_response). */
+int dspb_node_set_impulse_response_channels(dspb_engine* e, int64_t node_id, const double* h, int64_t n_sets, int64_t n_taps,
+                                            const int32_t* set_index, int64_t n_channels);
 
 /* Replaces: UiContext::add_link (runtime.rs:125-134): lhs = (producer node, output port),
  * rhs = (consumer node, input port); ports by name (node.rs:87-89).  Several links may leave one
