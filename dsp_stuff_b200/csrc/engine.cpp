@@ -308,34 +308,46 @@ int port_index(const std::vector<const char*>& v, const char* name) {
 
 int64_t round_up(int64_t n, int64_t g) { return g <= 1 ? n : (n + g - 1) / g * g; }
 
-// Host side of exact_math.cuh's div_const.  The 3-instruction sequence is NOT exact for every divisor
-// (measured: 0.3, 29.99, ... have millions of wrong quotients), so a divisor gets the fast path only
-// after the device has enumerated all 2^32 dividends against IEEE division with zero mismatches
-// (verify_const_div, a few ms, cached per process).  Everything else takes __fdiv_rn.
-bool div_const_ok(float b, bool plan_only) {
-    if (!(b > 0.0f) || !std::isfinite(b) || b < 1e-30f || b > 1e30f) return false;
-    if (plan_only) return true;  // nothing runs in planning-only mode; show the optimistic schedule
+// Host side of exact_math.cuh's constant divisions.  Neither fast form is exact for every divisor (measured: 0.3, 29.99,
+// ... have millions of wrong quotients under div_const), so a divisor gets one only after the device has enumerated all
+// 2^32 dividends against IEEE division, under exactly the acceptance rule the kernels use, with zero mismatches
+// (verify_const_div2 / verify_const_div, a few ms each, cached per process).  Tiers, first passing one wins: the
+// two-instruction div_const2 (only for divisors in [2^-20, 2^20], the range its |a|-only guard assumes), Markstein's
+// div_const, and __fdiv_rn for everything else.
+float recip_lo(float b, float zh) { return (float)(1.0 / (double)b - (double)zh); }  // zl = RN(1/b - zh), formed in double
+int div_tier(float b, bool plan_only) {
+    if (!(b > 0.0f) || !std::isfinite(b) || b < 1e-30f || b > 1e30f) return DIV_IEEE;
+    const bool mulfma_range = b >= 0x1p-20f && b <= 0x1p20f;
+    // nothing runs in planning-only mode: show the optimistic schedule
+    if (plan_only) return mulfma_range ? DIV_MULFMA : DIV_MARKSTEIN;
     // the verdict is IEEE arithmetic, identical on every device: one process-wide cache, serialised (engines on
     // different threads compile concurrently; the enumeration itself runs on the calling engine's device)
     static std::mutex mu;
-    static std::map<uint32_t, bool> cache;
+    static std::map<uint32_t, int> cache;
     uint32_t bits;
     memcpy(&bits, &b, 4);
     std::lock_guard<std::mutex> lk(mu);
     auto it = cache.find(bits);
     if (it != cache.end()) return it->second;
-    bool ok = false;
+    int tier = DIV_IEEE;
     unsigned long long mism = 1;
-    if (verify_const_div(b, 1.0f / b, &mism) == 0) ok = mism == 0;
-    cache[bits] = ok;
-    return ok;
+    const float zh = 1.0f / b;
+    if (mulfma_range && verify_const_div2(b, zh, recip_lo(b, zh), &mism) == 0 && mism == 0) tier = DIV_MULFMA;
+    mism = 1;
+    if (tier == DIV_IEEE && verify_const_div(b, zh, &mism) == 0 && mism == 0) tier = DIV_MARKSTEIN;
+    cache[bits] = tier;
+    return tier;
 }
-void set_const_div(Op& op, int p_b, int p_r, float b, bool plan_only) {
-    const bool ok = div_const_ok(b, plan_only);
+// op.p[p_b] = b, p[p_b + 1] (and p[p_b + 2]) = what the tier's kernel code reads; op.pad = the tier (plan.h DivTier)
+void set_const_div(Op& op, int p_b, float b, bool plan_only) {
+    const int tier = div_tier(b, plan_only);
+    const float zh = 1.0f / b;
     op.p[p_b] = b;
-    op.p[p_r] = ok ? 1.0f / b : 0.0f;
-    op.pad = ok ? 1 : 0;
+    op.p[p_b + 1] = tier != DIV_IEEE ? zh : 0.0f;
+    op.p[p_b + 2] = tier == DIV_MULFMA ? recip_lo(b, zh) : 0.0f;
+    op.pad = (uint8_t)tier;
 }
+const char* div_tier_name(int tier) { return tier == DIV_MULFMA ? "mul-fma" : tier == DIV_MARKSTEIN ? "markstein" : "ieee"; }
 
 // ---- opt-in time-parallel recurrences (dspb_config::iir_mode = 1) ---------------------------------------------------
 // ScanTab for y[n] = p[n] - a1 y[n-1] - a2 y[n-2]: powers of A = [[-a1, -a2], [1, 0]] in f64, rounded to f32.
@@ -556,7 +568,7 @@ struct Lowerer {
         }
         if (e.raw_ports) return true;  // dspb_node_process: inputs are already averaged (node.rs:217-222)
         Op d = mk(OP_DIVC);
-        set_const_div(d, 0, 1, nf, e.plan_only);
+        set_const_div(d, 0, nf, e.plan_only);
         char b[96];
         snprintf(b, sizeof b, "acc /= %.9g           ; fan-in average of %zu link(s)", nf, ls.size());
         emit(d, b);
@@ -606,7 +618,7 @@ struct Lowerer {
             op_values(nd.type, which, f.data(), v);
             for (int q = 0; q < k; q++) pc_cols[col + q][c] = v[q];
         }
-        op.pad = (uint8_t)((op.pad & 1) | ((col + 1) << 1));
+        op.pad = (uint8_t)((op.pad & 3) | ((col + 1) << 2));
         return " per-channel[" + names + "]";
     }
     void close_fused();
@@ -655,8 +667,8 @@ int Lowerer::finish_vregs(Step& st, std::vector<Op>& o, std::vector<std::string>
         size_t k = i;
         if (o[k].code == OP_LOADV && o[k].vreg == 0xFF) { pre |= 1; k++; }
         if (k < o.size() && o[k].code == OP_DIVC) {
-            pre |= 2 | (o[k].pad ? 4 : 0);
-            const float nf = o[k].p[0], r = o[k].p[1];
+            pre |= 2 | (op_div_tier(o[k]) << 2);
+            const float nf = o[k].p[0], z1 = o[k].p[1], z2 = o[k].p[2];
             k++;
             Op host;
             std::string host_txt;
@@ -664,7 +676,8 @@ int Lowerer::finish_vregs(Step& st, std::vector<Op>& o, std::vector<std::string>
             else { host = mk(OP_NOP); host_txt = "(fan-in prologue only)"; }
             host.pre = (uint8_t)pre;
             host.p[4] = nf;
-            host.p[5] = r;
+            host.p[5] = z1;
+            host.p[6] = z2;
             char b[64];
             snprintf(b, sizeof b, "[%sacc /= %.9g] ", (pre & 1) ? "acc = 0.0 + acc; " : "", nf);
             o[i] = host;
@@ -847,6 +860,11 @@ void Lowerer::close_fused() {
                 if (o.pflags & (1 << q)) k += snprintf(b + k, sizeof b - k, ":p%d=v%d", q, (int)o.pv[q]);
             if (op_pc_col(o) >= 0) k += snprintf(b + k, sizeof b - k, ":c%d", op_pc_col(o));  // per-channel table column
             if (o.code == OP_LOADG || o.code == OP_ADDG || o.code == OP_COPYG || o.code == OP_STOREG) k += snprintf(b + k, sizeof b - k, ":g%d%s", (int)o.buf, o.aux ? "*" : "");
+            // how each constant division runs: the fan-in divisor and a Distort's scalar level ('?': planning mode, where
+            // nothing is verified and a fast tier is the one the divisor would get if its device check passed)
+            auto tier = [&](int t) { return std::string(div_tier_name(t)) + (e.plan_only && t != DIV_IEEE ? "?" : ""); };
+            if (o.pre & 2) k += snprintf(b + k, sizeof b - k, ":nf=%s", tier(pre_div_tier(o.pre)).c_str());
+            if (o.code == OP_DISTORT && !(o.pflags & 1)) k += snprintf(b + k, sizeof b - k, ":div=%s", tier(op_div_tier(o)).c_str());
             m += b;
         }
         cur.text += m + "\n";
@@ -1102,7 +1120,7 @@ int Lowerer::lower() {
                         ctl_param(op, 0, 0);
                         pcm = per_channel(op, ni, 0, 1u);
                         // the exact fast division is verified per divisor: per-channel levels divide with IEEE division (dv)
-                        if (pcm.empty()) set_const_div(op, 0, 1, nd.f32[0], e.plan_only);
+                        if (pcm.empty()) set_const_div(op, 0, nd.f32[0], e.plan_only);
                         snprintf(b, sizeof b, "acc = distort[%s](acc, %g)%s", nt.enums[0].variants[nd.enums[0]], nd.f32[0], pcm.c_str());
                         break;
                     case T_OVERDRIVE:

@@ -34,4 +34,25 @@ __device__ __forceinline__ float div_const(float a, const ConstDiv d, float& mn_
 }
 __device__ __forceinline__ bool div_const_accept(float mn_q, float mx_a) { return mn_q >= kDivLo && mx_a <= kDivHi; }
 
+// Correctly rounded a / b in two instructions (Brisebarre, Muller, Raina, "Accelerating correctly rounded floating-point
+// division when the divisor is known in advance", IEEE TC 53(8), 2004): zh = RN(1/b), zl = RN(1/b - zh) (formed in double
+// on the host), q = RN(a*zh + RN(a*zl)) with one FMUL and one FFMA.  Like div_const it is exact for many divisors but not
+// all, and it goes wrong where a*zl underflows or q leaves the normal range.  The host enables it only for divisors in
+// [2^-20, 2^20], so a bound on |a| alone bounds |q|: the caller keeps the running min and max of |a| over its chunk and
+// accepts the fast results only if min|a| >= 2^-96 and max|a| <= 2^96 (a chunk with zeros, denormals, huge values or
+// infinities is redone with __fdiv_rn).  Inside an accepted chunk a != 0, so a fan-in prologue's `0.0 + a` is a and can be
+// left to the fallback.  The engine enables this form per divisor only after verify_const_div2() enumerated all 2^32
+// dividends under exactly this acceptance rule with zero mismatches.
+struct ConstDiv2 {
+    float zh, zl;
+};
+constexpr float kDiv2Lo = 0x1p-96f;
+constexpr float kDiv2Hi = 0x1p96f;
+__device__ __forceinline__ float div_const2(float a, const ConstDiv2 d, float& mn_a, float& mx_a) {
+    mn_a = fminf(mn_a, fabsf(a));
+    mx_a = fmaxf(mx_a, fabsf(a));
+    return __fmaf_rn(a, d.zh, __fmul_rn(a, d.zl));
+}
+__device__ __forceinline__ bool div_const2_accept(float mn_a, float mx_a) { return mn_a >= kDiv2Lo && mx_a <= kDiv2Hi; }
+
 }  // namespace dspb

@@ -303,14 +303,31 @@ __device__ __forceinline__ void store16(float4* s, int stride, const float (&v)[
     for (int k = 0; k < kF4; k++) s[k * stride] = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
 }
 
-// acc[i] /= b for a host-known divisor: exact fast path, IEEE division when the chunk holds zeros,
-// denormal-range or huge values (exact_math.cuh)
-__device__ __forceinline__ void div16(float (&acc)[kChunk], const ConstDiv d, bool use_fast) {
-    if (use_fast) {
+// acc[i] = (add0 ? 0.0 + acc[i] : acc[i]) / b for a host-known divisor b, in the tier the host verified for it (plan.h
+// DivTier; z1, z2 = r or zh, zl).  The fast forms are exact wherever their guard accepts the chunk; a chunk with zeros,
+// denormal-range or huge values takes IEEE division.  div_const2 accepts only chunks without zeros, where 0.0 + a == a bit
+// for bit, so the fan-in's zero-add is left to the fallback; the Markstein and IEEE tiers add first, as the reference does.
+__device__ __forceinline__ void div_chunk(float (&acc)[kChunk], float b, float z1, float z2, int tier, bool add0) {
+    if (tier == DIV_MULFMA) {
+        float q[kChunk];
+        float mn = kDiv2Hi, mx = 0.0f;
+#pragma unroll
+        for (int i = 0; i < kChunk; i++) q[i] = div_const2(acc[i], ConstDiv2{z1, z2}, mn, mx);
+        if (div_const2_accept(mn, mx)) {
+#pragma unroll
+            for (int i = 0; i < kChunk; i++) acc[i] = q[i];
+            return;
+        }
+    }
+    if (add0) {
+#pragma unroll
+        for (int i = 0; i < kChunk; i++) acc[i] = add(0.0f, acc[i]);
+    }
+    if (tier == DIV_MARKSTEIN) {
         float q[kChunk];
         float mn = kDivHi, mx = 0.0f;
 #pragma unroll
-        for (int i = 0; i < kChunk; i++) q[i] = div_const(acc[i], d, mn, mx);
+        for (int i = 0; i < kChunk; i++) q[i] = div_const(acc[i], ConstDiv{b, z1}, mn, mx);
         if (div_const_accept(mn, mx)) {
 #pragma unroll
             for (int i = 0; i < kChunk; i++) acc[i] = q[i];
@@ -318,7 +335,16 @@ __device__ __forceinline__ void div16(float (&acc)[kChunk], const ConstDiv d, bo
         }
     }
 #pragma unroll
-    for (int i = 0; i < kChunk; i++) acc[i] = dv(acc[i], d.b);
+    for (int i = 0; i < kChunk; i++) acc[i] = dv(acc[i], b);
+}
+// The fan-in prologue folded into an op (plan.h Op::pre): acc = 0.0 + acc (pre & 1), acc /= p[4] (pre & 2).
+__device__ __forceinline__ void fanin_prologue(float (&acc)[kChunk], int pre, const Op& op) {
+    if (pre & 2) {
+        div_chunk(acc, op.p[4], op.p[5], op.p[6], pre_div_tier(pre), pre & 1);
+    } else if (pre & 1) {
+#pragma unroll
+        for (int i = 0; i < kChunk; i++) acc[i] = add(0.0f, acc[i]);
+    }
 }
 
 // Per-CTA / per-tile context shared by every op.
@@ -398,7 +424,7 @@ struct Pf {
 // One op of the segment program on this thread's 16 samples.  `code`, `mode` and `pre` are
 // compile-time constants in the specialised kernels (the switch folds away) and run-time values in
 // the generic interpreter.  pre & 1: acc = 0.0 + acc (first link of a fan-in sum, node.rs:181-183);
-// pre & 2: acc /= nf (node.rs:189-191) with the divisor in p[4], its reciprocal in p[5].
+// pre & 2: acc /= nf (node.rs:189-191) with the divisor in p[4] and its tier's constants in p[5], p[6] (fanin_prologue).
 // PC: the op may carry per-channel parameters (plan.h Program::pc); false in the compiled specialised chains, whose ops
 // never do (chain_matches), so their code is the shared-parameter code only.
 template <int G, bool PC = false>
@@ -413,7 +439,7 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
     const float* pcr = nullptr;  // the op's first column in row 0 (the recurrence lanes pick their own rows)
     if constexpr (PC) {
         pcv[0] = op.p[0]; pcv[1] = op.p[1]; pcv[2] = op.p[2]; pcv[3] = op.p[3]; pcv[4] = op.a2;
-        if (op.pad >> 1) {
+        if (op_pc_col(op) >= 0) {
             pcr = prog.pc + op_pc_col(op);
             const float* r = pcr + (long long)c.ch * prog.pc_stride;
             const int n = op_pc_cols(code);
@@ -424,11 +450,7 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
         if constexpr (PC) return pcv[i];
         else return i < 4 ? op.p[i] : op.a2;
     };
-    if (pre & 1) {
-#pragma unroll
-        for (int i = 0; i < kChunk; i++) acc[i] = add(0.0f, acc[i]);
-    }
-    if (pre & 2) div16(acc, ConstDiv{op.p[4], op.p[5]}, pre & 4);
+    fanin_prologue(acc, pre, op);
     switch (code) {
         case OP_NOP: break;
         case OP_ZERO: {
@@ -520,25 +542,24 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
         } break;
         case OP_DISTORT: {
             if (!(op.pflags & 1) && mode != Fuzz) {  // scalar level: the common case
-                const float l = prm(0);       // per-channel: the host clears pad bit 0, so the divisions below are IEEE (dv)
+                const float l = prm(0);       // per-channel: the host leaves the tier at DIV_IEEE, so the divisions below are dv
                 if (l < 0.001f) break;  // every shaper returns the sample unchanged (distort.rs:64,...)
-                const ConstDiv dl{l, op.p[1]};
-                const bool fast = op.pad & 1;
+                const int tier = op_div_tier(op);
                 switch (mode) {
                     case HardClip: {
 #pragma unroll
                         for (int i = 0; i < kChunk; i++) acc[i] = clipf(mul(acc[i], l));
-                        div16(acc, dl, fast);
+                        div_chunk(acc, l, op.p[1], op.p[2], tier, false);
                     } break;
                     case SoftClip: {
-                        const ConstDiv d3{3.0f, 0.333333343267440796f};
                         float c3[kChunk];
 #pragma unroll
                         for (int i = 0; i < kChunk; i++) {
                             acc[i] = mul(acc[i], l);
                             c3[i] = mul(mul(acc[i], acc[i]), acc[i]);
                         }
-                        div16(c3, d3, true);
+                        // / 3: zh = RN(1/3), zl = RN(1/3 - zh); tests/test_gpu_const_div2.py enumerates all 2^32 dividends
+                        div_chunk(c3, 3.0f, 0x1.555556p-2f, -0x1.555556p-27f, DIV_MULFMA, false);
 #pragma unroll
                         for (int i = 0; i < kChunk; i++) {
                             float s = acc[i];
@@ -547,7 +568,7 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
                             else s = -2.0f / 3.0f;
                             acc[i] = clipf(s);
                         }
-                        div16(acc, dl, fast);
+                        div_chunk(acc, l, op.p[1], op.p[2], tier, false);
                     } break;
                     case Tanh: {
 #pragma unroll
@@ -851,6 +872,10 @@ __device__ __forceinline__ void exec_op(const int code, const int mode, const in
 // sig(i) packs code | mode << 8 | pre << 16; n = 0 selects the run-time interpreter.
 struct ChainDynamic { static constexpr int n = 0; static constexpr int rec = 0; __host__ __device__ static constexpr int sig(int) { return 0; } __host__ __device__ static constexpr int pf_of(int) { return -1; } };
 #define DSPB_SIG(code, mode, pre) ((code) | ((mode) << 8) | ((pre) << 16))
+// The chains' fan-in prologues (every node of a chain has one link: acc /= 1.0001) are compiled for the mul-fma tier;
+// a program whose divisor got another tier does not match a chain and runs in the interpreter.
+constexpr int kPreDiv = 2 | (DIV_MULFMA << 2);   // acc /= p[4]
+constexpr int kPreAddDiv = 1 | kPreDiv;          // acc = 0.0 + acc; acc /= p[4]
 // PF (template argument of the chains): bit 0 = the input chunk (op 0) is register-prefetched, bit 1 = the
 // comb ring chunk is; pf_of(i) is the compile-time pfc of op i.
 template <int PF>
@@ -859,8 +884,8 @@ struct ChainGDBR {  // src -> gain -> distort(SoftClip) -> biquad -> reverb -> s
     static constexpr int rec = 3;
     __host__ __device__ static constexpr int pf_of(int i) { return i == 0 ? (PF & 1) : i == 4 ? ((PF >> 1) & 1) : i == n - 1 ? 1 : 0; }
     __host__ __device__ static constexpr int sig(int i) {
-        return i == 0 ? DSPB_SIG(OP_LOADG, 0, 0) : i == 1 ? DSPB_SIG(OP_GAIN, 0, 6) : i == 2 ? DSPB_SIG(OP_DISTORT, SoftClip, 7)
-             : i == 3 ? DSPB_SIG(OP_BIQUAD, 0, 7) : i == 4 ? DSPB_SIG(OP_COMB, 0, 7) : DSPB_SIG(OP_STOREG, 0, 7);
+        return i == 0 ? DSPB_SIG(OP_LOADG, 0, 0) : i == 1 ? DSPB_SIG(OP_GAIN, 0, kPreDiv) : i == 2 ? DSPB_SIG(OP_DISTORT, SoftClip, kPreAddDiv)
+             : i == 3 ? DSPB_SIG(OP_BIQUAD, 0, kPreAddDiv) : i == 4 ? DSPB_SIG(OP_COMB, 0, kPreAddDiv) : DSPB_SIG(OP_STOREG, 0, kPreAddDiv);
     }
 };
 template <int PF>
@@ -868,7 +893,7 @@ struct ChainGDBRScan {  // the same chain with the biquad in scan mode (dspb_con
     static constexpr int n = 6;
     [[maybe_unused]] static constexpr int rec = -1;
     __host__ __device__ static constexpr int pf_of(int i) { return ChainGDBR<PF>::pf_of(i); }
-    __host__ __device__ static constexpr int sig(int i) { return i == 3 ? DSPB_SIG(OP_BIQUAD, 1, 7) : ChainGDBR<PF>::sig(i); }
+    __host__ __device__ static constexpr int sig(int i) { return i == 3 ? DSPB_SIG(OP_BIQUAD, 1, kPreAddDiv) : ChainGDBR<PF>::sig(i); }
 };
 template <int PF>
 struct ChainGDR {  // src -> gain -> distort(SoftClip) -> reverb -> store   (config 1)
@@ -876,8 +901,8 @@ struct ChainGDR {  // src -> gain -> distort(SoftClip) -> reverb -> store   (con
     [[maybe_unused]] static constexpr int rec = -1;
     __host__ __device__ static constexpr int pf_of(int i) { return i == 0 ? (PF & 1) : i == 3 ? ((PF >> 1) & 1) : i == n - 1 ? 1 : 0; }
     __host__ __device__ static constexpr int sig(int i) {
-        return i == 0 ? DSPB_SIG(OP_LOADG, 0, 0) : i == 1 ? DSPB_SIG(OP_GAIN, 0, 6) : i == 2 ? DSPB_SIG(OP_DISTORT, SoftClip, 7)
-             : i == 3 ? DSPB_SIG(OP_COMB, 0, 7) : DSPB_SIG(OP_STOREG, 0, 7);
+        return i == 0 ? DSPB_SIG(OP_LOADG, 0, 0) : i == 1 ? DSPB_SIG(OP_GAIN, 0, kPreDiv) : i == 2 ? DSPB_SIG(OP_DISTORT, SoftClip, kPreAddDiv)
+             : i == 3 ? DSPB_SIG(OP_COMB, 0, kPreAddDiv) : DSPB_SIG(OP_STOREG, 0, kPreAddDiv);
     }
 };
 template <int PF>
@@ -886,7 +911,7 @@ struct ChainBB {  // src -> biquad -> biquad -> store   (config 2)
     [[maybe_unused]] static constexpr int rec = -1;
     __host__ __device__ static constexpr int pf_of(int i) { return i == 0 ? (PF & 1) : i == -1 ? ((PF >> 1) & 1) : i == n - 1 ? 1 : 0; }
     __host__ __device__ static constexpr int sig(int i) {
-        return i == 0 ? DSPB_SIG(OP_LOADG, 0, 0) : i == 1 ? DSPB_SIG(OP_BIQUAD, 0, 6) : i == 2 ? DSPB_SIG(OP_BIQUAD, 0, 7) : DSPB_SIG(OP_STOREG, 0, 7);
+        return i == 0 ? DSPB_SIG(OP_LOADG, 0, 0) : i == 1 ? DSPB_SIG(OP_BIQUAD, 0, kPreDiv) : i == 2 ? DSPB_SIG(OP_BIQUAD, 0, kPreAddDiv) : DSPB_SIG(OP_STOREG, 0, kPreAddDiv);
     }
 };
 template <int PF>
@@ -895,7 +920,7 @@ struct ChainLH {  // src -> low_pass -> high_pass -> store   (config 2, one-pole
     [[maybe_unused]] static constexpr int rec = -1;
     __host__ __device__ static constexpr int pf_of(int i) { return i == 0 ? (PF & 1) : i == -1 ? ((PF >> 1) & 1) : i == n - 1 ? 1 : 0; }
     __host__ __device__ static constexpr int sig(int i) {
-        return i == 0 ? DSPB_SIG(OP_LOADG, 0, 0) : i == 1 ? DSPB_SIG(OP_LP1, 0, 6) : i == 2 ? DSPB_SIG(OP_HP1, 0, 7) : DSPB_SIG(OP_STOREG, 0, 7);
+        return i == 0 ? DSPB_SIG(OP_LOADG, 0, 0) : i == 1 ? DSPB_SIG(OP_LP1, 0, kPreDiv) : i == 2 ? DSPB_SIG(OP_HP1, 0, kPreAddDiv) : DSPB_SIG(OP_STOREG, 0, kPreAddDiv);
     }
 };
 template <int PF>
@@ -903,7 +928,7 @@ struct ChainCopy {  // G -> (/nf) -> store   (the segment after a Fir node)
     static constexpr int n = 2;
     [[maybe_unused]] static constexpr int rec = -1;
     __host__ __device__ static constexpr int pf_of(int i) { return i == 0 ? (PF & 1) : i == -1 ? ((PF >> 1) & 1) : i == n - 1 ? 1 : 0; }
-    __host__ __device__ static constexpr int sig(int i) { return i == 0 ? DSPB_SIG(OP_LOADG, 0, 0) : DSPB_SIG(OP_STOREG, 0, 6); }
+    __host__ __device__ static constexpr int sig(int i) { return i == 0 ? DSPB_SIG(OP_LOADG, 0, 0) : DSPB_SIG(OP_STOREG, 0, kPreDiv); }
 };
 
 template <int G, class Chain, int I>
@@ -1214,12 +1239,7 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
             tp1 = clock64();
 #endif
             // the recurrence op's own prologue and feed-forward part
-            const int rpre = Chain::n > 0 ? ((Chain::sig(Chain::rec) >> 16) & 0xff) : rop.pre;
-            if (rpre & 1) {
-#pragma unroll
-                for (int k = 0; k < kChunk; k++) acc[k] = add(0.0f, acc[k]);
-            }
-            if (rpre & 2) div16(acc, ConstDiv{rop.p[4], rop.p[5]}, rpre & 4);
+            fanin_prologue(acc, Chain::n > 0 ? ((Chain::sig(Chain::rec) >> 16) & 0xff) : rop.pre, rop);
             if (rcode == OP_BIQUAD) {
                 float b0 = rop.p[0], b1 = rop.p[1], b2 = rop.p[2];
                 if constexpr (PC) {
@@ -1475,11 +1495,7 @@ fused_kernel_ws2(const __grid_constant__ Program prog, int c_begin, int c_end, l
     };
     // prologue + time-parallel part of recurrence op `rop` (stage st) for the tile set by set_tile(ti), then the hand-off
     auto feed = [&](const Op& rop, int st, int ti, float (&acc)[kChunk]) {
-        if (rop.pre & 1) {
-#pragma unroll
-            for (int k = 0; k < kChunk; k++) acc[k] = add(0.0f, acc[k]);
-        }
-        if (rop.pre & 2) div16(acc, ConstDiv{rop.p[4], rop.p[5]}, rop.pre & 4);
+        fanin_prologue(acc, rop.pre, rop);
         // per-channel parameters: this thread's channel row
         const float* pr = op_pc_col(rop) >= 0 ? prog.pc + op_pc_col(rop) + (long long)c.ch * prog.pc_stride : nullptr;
         if (rop.code == OP_BIQUAD) {
@@ -1827,17 +1843,38 @@ __global__ void div_verify_kernel(float b, float r, unsigned long long* mism) {
     }
     if (m) atomicAdd(mism, m);
 }
-}  // namespace
-
-int verify_const_div(float b, float r, unsigned long long* mismatches) {
+// The same proof for div_const2 (zh, zl) under its own acceptance rule: the engine's first tier.
+__global__ void div2_verify_kernel(float b, float zh, float zl, unsigned long long* mism) {
+    const unsigned long long base = ((unsigned long long)blockIdx.x * blockDim.x + threadIdx.x) * 256ull;
+    unsigned long long m = 0;
+    for (int k = 0; k < 256; k++) {
+        const float a = __uint_as_float((unsigned)(base + k));
+        float mn = kDiv2Hi, mx = 0.0f;
+        const float q = div_const2(a, ConstDiv2{zh, zl}, mn, mx);
+        const float ref = __fdiv_rn(a, b);
+        if (div_const2_accept(mn, mx) && __float_as_uint(q) != __float_as_uint(ref) && !(q != q && ref != ref)) m++;
+    }
+    if (m) atomicAdd(mism, m);
+}
+template <class Launch>
+int count_mismatches(Launch launch, unsigned long long* mismatches) {
     unsigned long long* d = nullptr;
     cudaError_t e = cudaMalloc(&d, 8);
     if (e != cudaSuccess) return (int)e;
     cudaMemset(d, 0, 8);
-    div_verify_kernel<<<65536, 256>>>(b, r, d);
-    e = cudaMemcpy(mismatches, d, 8, cudaMemcpyDeviceToHost);
+    launch(d);
+    e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpy(mismatches, d, 8, cudaMemcpyDeviceToHost);
     cudaFree(d);
     return (int)e;
+}
+}  // namespace
+
+int verify_const_div(float b, float r, unsigned long long* mismatches) {
+    return count_mismatches([&](unsigned long long* d) { div_verify_kernel<<<65536, 256>>>(b, r, d); }, mismatches);
+}
+int verify_const_div2(float b, float zh, float zl, unsigned long long* mismatches) {
+    return count_mismatches([&](unsigned long long* d) { div2_verify_kernel<<<65536, 256>>>(b, zh, zl, d); }, mismatches);
 }
 
 // Probe for one recurrence: the same op in exact and in scan mode over 8 channels x 16384 samples (four of uniform noise,

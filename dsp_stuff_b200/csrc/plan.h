@@ -94,14 +94,20 @@ struct Op {
     uint8_t pv[3];    // vregs of tile-valued parameters
     uint8_t buf;      // global buffer index for LOADG/ADDG/STOREG, prefetch slot + 1 in `aux`
     uint16_t aux;     // ring / state slot, or prefetch slot (0 = none, k+1 = slot k)
-    uint8_t pad;      // bit 0: p[1] holds a verified reciprocal of p[0] (exact_math.cuh div_const);
-                      // bits 1-7: per-channel parameters, 1 + the column of this op's first value in Program::pc (0 = shared)
-    uint8_t pre;      // fan-in prologue folded into this op: 1 = acc = 0.0 + acc; 2 = acc /= p[4]; 4 = p[5] = 1/p[4] usable
-    float p[6];       // p[4], p[5]: fan-in divisor and its reciprocal when pre & 2
+    uint8_t pad;      // bits 0-1: DivTier of the op's own constant divisor p[0] (Distort level): p[1] = RN(1/p[0]) when
+                      // DIV_MARKSTEIN, p[1], p[2] = zh, zl when DIV_MULFMA;
+                      // bits 2-7: per-channel parameters, 1 + the column of this op's first value in Program::pc (0 = shared)
+    uint8_t pre;      // fan-in prologue folded into this op: 1 = acc = 0.0 + acc; 2 = acc /= p[4]; bits 2-3: DivTier of
+                      // that division (4: p[5] = RN(1/p[4]); 8: p[5], p[6] = zh, zl)
+    float p[7];       // p[4], p[5], p[6]: fan-in divisor and its reciprocal or zh, zl when pre & 2
     float a2;         // biquad: a2 (p[0..3] = b0, b1, b2, a1)
 };
+// How a constant division runs (exact_math.cuh); the host picks the first tier whose exhaustive device check passes.
+enum DivTier { DIV_IEEE = 0, DIV_MARKSTEIN = 1, DIV_MULFMA = 2 };
+__host__ __device__ inline int op_div_tier(const Op& o) { return o.pad & 3; }
+__host__ __device__ inline constexpr int pre_div_tier(int pre) { return (pre >> 2) & 3; }
 
-// Per-channel parameters (dspb_node_set_f32_channels).  An op whose `pad >> 1` is k > 0 reads its parameters from row `ch`
+// Per-channel parameters (dspb_node_set_f32_channels).  An op whose `pad >> 2` is k > 0 reads its parameters from row `ch`
 // (the ABSOLUTE channel) of the step's table Program::pc, columns k-1 ... k-2+op_pc_cols(code), in this order: p[0], p[1],
 // ... and, for the biquad, a2 last.  Everything else (fan-in divisor, sample rate, control-port tiles) stays in the Op.
 constexpr int kMaxPcCols = 32;      // columns of one step's table (a segment that needs more is cut)
@@ -110,7 +116,7 @@ __host__ __device__ inline constexpr int op_pc_cols(int code) {
          : (code == OP_LP1 || code == OP_HP1 || code == OP_ENVELOPE || code == OP_SIGGEN) ? 2
          : (code == OP_GAIN || code == OP_DISTORT || code == OP_MIX || code == OP_COMB || code == OP_GATE) ? 1 : 0;
 }
-__host__ __device__ inline int op_pc_col(const Op& o) { return (o.pad >> 1) - 1; }  // -1: shared parameters
+__host__ __device__ inline int op_pc_col(const Op& o) { return (o.pad >> 2) - 1; }  // -1: shared parameters
 
 // Does an op of this code read the shared-memory vreg named by Op::vreg?  (SAVEV writes it; parameter tiles are in pv[].)
 inline constexpr bool op_reads_vreg_field(int code) {
@@ -160,6 +166,8 @@ int launch_fused(const Program& prog, int G, int c_begin, int c_end, int64_t T, 
 int fused_smem_bytes(const Program& prog, int G);
 // Enumerates all 2^32 dividends on the device; *mismatches == 0 proves div_const exact for divisor b.
 int verify_const_div(float b, float r, unsigned long long* mismatches);
+// The same for div_const2 with zh, zl (exact_math.cuh ConstDiv2) under its own acceptance rule.
+int verify_const_div2(float b, float zh, float zl, unsigned long long* mismatches);
 // Runs a one-recurrence probe program in exact and in scan mode on the device (noise + log sweep, 16384 samples) and
 // returns max |scan - exact| / max |exact|: the measured error that gates scan mode for one coefficient set.
 int measure_scan_error(const Op& exact_op, const ScanTab& tab, float* rel_err);
