@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdspb200.so")
 DRIVER = os.path.join(HERE, "dspb_run")
-SOURCES = ["engine.cpp", "fused_chain.cu", "fir.cu", "fir_fft.cu", "fir_toeplitz.cu", "boundary.cu"]
+SOURCES = ["engine.cpp", "fused_chain.cu", "fir.cu", "fir_fft.cu", "fir_toeplitz.cu", "boundary.cu", "reset.cu"]
 HEADERS = ["plan.h", "json_min.h", "exact_math.cuh", "dspb_run.cpp", os.path.join("..", "..", "include", "dspb200.h")]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

@@ -169,6 +169,11 @@ struct Node {
     int fir_xf_single = 0;          // transforms that carry one channel
     DevBuf set_dev, xf_dev;         // fir_set and fir_xf on the device
     bool fir_pc() const { return !fir_set.empty(); }
+    // Channels reset on their own (dspb_reset_channels) that are still in their own warm-up: {channel, samples since its
+    // reset}, ascending channels.  Only channels whose reset came after the node's own (started) are kept: a node-level
+    // restart (fir_dirty, dspb_reset_state) clears the list, since min(started, since reset) is then `started` for every channel.
+    std::vector<int2> warm;
+    const int2* warm_dev = nullptr;  // this call's copy of `warm` on the device
 };
 
 // Transform table of per-channel impulse responses.  Two channels share one complex transform only when they use the same set.
@@ -264,6 +269,10 @@ struct dspb_engine {
     std::vector<ProfRec> prof;
     bool plan_only = false;
     bool host_inflight = false;   // a DSPB_MEM_HOST_ASYNC call may still be running on the internal streams
+    // dspb_reset_channels: channels to reset at the start of the next dspb_process (ascending, no duplicates), and the device
+    // area that call's clear descriptors, channel list and FIR warm-up lists are copied to (sized in ensure_resources)
+    std::vector<int32_t> reset_pending;
+    DevBuf reset_dev;
     int64_t host_last_n = 0;
     // playback-side sample-rate converter (dspb_resample_dup_stereo): dasp Converter state shared by all channels + the
     // last 16 pushed frames of every channel
@@ -452,6 +461,7 @@ int clear_node_state(dspb_engine* e, Node& n) {
     n.u_pos = 0;
     n.fdl_valid = false;
     n.upc_ctr = 0;
+    n.warm.clear();
     (void)e;
     return DSPB_OK;
 }
@@ -1294,8 +1304,21 @@ int ensure_resources(dspb_engine* e) {
             }
             n.started = 0;
             n.u_pos = 0;
+            n.warm.clear();
             n.fir_dirty = false;
         }
+    }
+    // dspb_reset_channels (prepare_channel_resets): one ClearDesc per state buffer, the channel list (padded to 16 bytes) and
+    // one warm-up list per FIR node, at most C entries each
+    size_t descs = 0, firs = 0;
+    for (auto& np : e->nodes) {
+        descs += is_stateful(np->type) || np->type == T_REVERB || np->type == T_FIR;
+        firs += np->type == T_FIR;
+    }
+    const size_t reset_bytes = descs * sizeof(ClearDesc) + round_up((int64_t)C * 4, 16) + firs * C * sizeof(int2);
+    if (e->reset_dev.bytes < reset_bytes) {
+        int r = e->reset_dev.alloc(reset_bytes, false, e->plan_only);
+        if (r) return r;
     }
     return DSPB_OK;
 }
@@ -1470,6 +1493,13 @@ int run_steps(dspb_engine* e, const float* const* d_in, float* const* d_out, int
             fp.u_pos = f.u_pos;
             // work counters of the persistent FFT kernels: lanes run concurrently on their own streams
             fp.fft_work = fp.mode == FIR_FFT ? f.fft_work[lane]->p : nullptr;
+            if (!f.warm.empty()) {  // channels reset on their own, in [c0, c1), still in their warm-up
+                auto lo = std::lower_bound(f.warm.begin(), f.warm.end(), c0, [](const int2& w, int c) { return w.x < c; });
+                auto hi = std::lower_bound(lo, f.warm.end(), c1, [](const int2& w, int c) { return w.x < c; });
+                fp.warm = f.warm_dev + (lo - f.warm.begin());
+                fp.n_warm = (int)(hi - lo);
+                for (auto it = lo; it != hi; ++it) fp.warm_len = std::max(fp.warm_len, (int)f.taps.size() - 1 - it->y);
+            }
             if (f.fir_pc()) {  // per-channel impulse responses: the transform-table slice of channels [c0, c1)
                 if (c0 % 32 || (c1 % 32 && c1 != e->cfg.channels))
                     return fail(DSPB_ERR_INVALID, "per-channel taps: launch range [%d, %d) is not aligned to 32 channels", c0, c1);
@@ -1512,6 +1542,10 @@ void advance_state(dspb_engine* e, int64_t n) {
             nd.fdl_valid = nd.upc_this_call;   // a call through the segment kernels leaves the delay line stale
             if (nd.upc_this_call) nd.upc_ctr += n / kUpcBlock;
             nd.upc_this_call = false;
+            size_t k = 0;  // per-channel warm-ups: advance, and drop the finished ones
+            for (const int2& w : nd.warm)
+                if ((int64_t)w.y + n < (int64_t)nd.taps.size() - 1) nd.warm[k++] = make_int2(w.x, w.y + (int)n);
+            nd.warm.resize(k);
         }
     }
 }
@@ -1523,6 +1557,68 @@ int check_ready(dspb_engine* e, int64_t n) {
     if (!e->lowered) {
         int r = lower_graph(e);
         if (r) return r;
+    }
+    return DSPB_OK;
+}
+
+// Start of a dspb_process, on the stream that orders it, in front of its first kernel: the per-channel resets recorded since
+// the last call (one clear launch for every state buffer and listed channel), and the device copy of every FIR warm-up
+// list.  Nothing recorded and no channel in its own warm-up: nothing is enqueued.
+int prepare_channel_resets(dspb_engine* e, cudaStream_t st) {
+    const std::vector<int32_t>& ch = e->reset_pending;
+    const int n_ch = (int)ch.size();
+    std::vector<ClearDesc> descs;
+    for (auto& np : e->nodes) {
+        Node& n = *np;
+        if (ch.empty()) break;
+        if (n.state.p) descs.push_back({n.state.p, 4, 0, 4, 4});
+        if (n.type == T_REVERB && n.ring.p) descs.push_back({n.ring.p, n.D, 0, n.D, n.D});
+        if (n.type != T_FIR || !n.U.p) continue;
+        // the hist_pad slots behind this call's sample 0; every later slot is written by the step feeding the FIR before
+        // the FIR step reads it
+        descs.push_back({n.U.p, n.u_ring, ring_slot(n.u_pos, -n.hist_pad, n.u_ring), n.hist_pad, n.u_ring});
+        n.fdl_valid = false;  // the UPC delay line holds spectra of the old history: re-prime from the ring
+        const int N = (int)n.taps.size();
+        if (n.started == 0 || N <= 1) continue;  // the node's own warm-up covers them (or there is none)
+        std::vector<int2> merged;  // restart (or start) the warm-up of every listed channel
+        merged.reserve(n.warm.size() + ch.size());
+        size_t i = 0;
+        for (int32_t c : ch) {
+            while (i < n.warm.size() && n.warm[i].x < c) merged.push_back(n.warm[i++]);
+            if (i < n.warm.size() && n.warm[i].x == c) i++;
+            merged.push_back(make_int2(c, 0));
+        }
+        merged.insert(merged.end(), n.warm.begin() + i, n.warm.end());
+        n.warm.swap(merged);
+    }
+    // one copy: [descriptors | channels | warm-up lists]
+    const bool clear = !descs.empty();
+    const size_t ch_off = descs.size() * sizeof(ClearDesc);
+    size_t bytes = clear ? ch_off + round_up((int64_t)ch.size() * 4, 16) : 0;
+    std::vector<char> stage(bytes);
+    if (clear) {
+        memcpy(stage.data(), descs.data(), ch_off);
+        memcpy(stage.data() + ch_off, ch.data(), ch.size() * 4);
+    }
+    char* dev = reinterpret_cast<char*>(e->reset_dev.p);
+    for (auto& np : e->nodes) {
+        Node& n = *np;
+        if (n.type != T_FIR || n.warm.empty()) continue;
+        n.warm_dev = reinterpret_cast<const int2*>(dev + bytes);
+        stage.resize(bytes + n.warm.size() * sizeof(int2));
+        memcpy(stage.data() + bytes, n.warm.data(), n.warm.size() * sizeof(int2));
+        bytes = stage.size();
+    }
+    e->reset_pending.clear();
+    if (bytes == 0) return DSPB_OK;
+    if (bytes > e->reset_dev.bytes) return fail(DSPB_ERR_INVALID, "per-channel reset tables exceed their device area");
+    // pageable source: cudaMemcpyAsync returns once the bytes are staged, so `stage` may go out of scope
+    CUDA_TRY(cudaMemcpyAsync(dev, stage.data(), bytes, cudaMemcpyHostToDevice, st));
+    if (clear) {
+        int rc = launch_clear_rows(reinterpret_cast<const ClearDesc*>(dev), (int)descs.size(),
+                                   reinterpret_cast<const int*>(dev + ch_off), n_ch, st);
+        if (rc) return fail(DSPB_ERR_CUDA, "clear kernel launch: %s", cudaGetErrorString((cudaError_t)rc));
+        e->last_launches++;
     }
     return DSPB_OK;
 }
@@ -1796,11 +1892,29 @@ int dspb_reset_state(dspb_engine* e) {
     CUDA_TRY(cudaSetDevice(e->cfg.device));
     CUDA_TRY(cudaDeviceSynchronize());
     e->host_inflight = false;
+    e->reset_pending.clear();
     for (auto& n : e->nodes) {
         int r = clear_node_state(e, *n);
         if (r) return r;
     }
     e->rs.target_hz = 0.0;  // the next dspb_resample_dup_stereo call builds a fresh converter
+    return DSPB_OK;
+}
+
+int dspb_reset_channels(dspb_engine* e, const int32_t* channels, int64_t n_channels) {
+    if (!e) return fail(DSPB_ERR_INVALID, "null engine");
+    if (n_channels < 0) return fail(DSPB_ERR_INVALID, "n_channels %lld < 0", (long long)n_channels);
+    if (!channels && n_channels > 0) return fail(DSPB_ERR_INVALID, "null channel list");
+    const int C = e->cfg.channels;
+    for (int64_t i = 0; i < n_channels; i++)
+        if (channels[i] < 0 || channels[i] >= C)
+            return fail(DSPB_ERR_INVALID, "channels[%lld] = %d is outside [0, %d)", (long long)i, (int)channels[i], C);
+    if (n_channels == 0) return DSPB_OK;
+    // recorded only: the clear is enqueued by the next dspb_process, in stream order with it
+    auto& p = e->reset_pending;
+    p.insert(p.end(), channels, channels + n_channels);
+    std::sort(p.begin(), p.end());
+    p.erase(std::unique(p.begin(), p.end()), p.end());
     return DSPB_OK;
 }
 
@@ -1827,6 +1941,8 @@ int dspb_process(dspb_engine* e, const float* const* inputs, float* const* outpu
             if ((uintptr_t)inputs[i] & 15) return fail(DSPB_ERR_INVALID, "device buffers must be 16-byte aligned");
         for (size_t i = 0; i < n_out; i++)
             if ((uintptr_t)outputs[i] & 15) return fail(DSPB_ERR_INVALID, "device buffers must be 16-byte aligned");
+        r = prepare_channel_resets(e, (cudaStream_t)stream);  // before the fork: every chunk stream waits for it
+        if (r) return r;
         int chunks = e->dev_chunks;
         if (e->steps.size() < 2 || C < 64 * chunks) chunks = 1;
         if (chunks <= 1) {
@@ -1893,6 +2009,8 @@ int dspb_process(dspb_engine* e, const float* const* inputs, float* const* outpu
     std::vector<float*> dout(n_out);
     for (size_t i = 0; i < n_in; i++) din[i] = e->h_in[i]->p;
     for (size_t i = 0; i < n_out; i++) dout[i] = e->h_out[i]->p;
+    r = prepare_channel_resets(e, e->s_cmp);  // after the previous call's kernels, before this call's first
+    if (r) return r;
     static const int host_chunks = getenv("DSPB_HOST_CHUNKS") ? std::max(1, std::min(64, atoi(getenv("DSPB_HOST_CHUNKS")))) : 16;
     int n_chunks = host_chunks;
     int per = (C + n_chunks - 1) / n_chunks;
@@ -2070,6 +2188,7 @@ int dspb_node_get_i64(dspb_engine* e, int64_t node_id, const char* key, int64_t*
     if (!e || !key || !out) return fail(DSPB_ERR_INVALID, "null argument");
     if (!strcmp(key, "kernel_launches")) { *out = e->last_launches; return DSPB_OK; }
     if (!strcmp(key, "n_segments")) { *out = (int64_t)e->steps.size(); return DSPB_OK; }
+    if (!strcmp(key, "pending_resets")) { *out = (int64_t)e->reset_pending.size(); return DSPB_OK; }
     int i = e->find(node_id);
     if (i < 0) return fail(DSPB_ERR_UNKNOWN_NODE, "unknown node id %lld", (long long)node_id);
     Node& n = *e->nodes[i];

@@ -31,15 +31,23 @@ constexpr int kDirectTile = 256;
 
 // One thread per output sample; the CTA's input window lives in shared memory.
 // PC: per-channel impulse responses, channel ch reads the reversed taps of its set, taps + set_index[ch] * N.
-template <bool PC>
+// LISTED: the warm-up patch of channels reset on their own (dspb_reset_channels): blockIdx.y indexes `warm`, {channel, samples
+// since its reset}, and the CTA recomputes that channel's samples [n_begin, n_end) that fall in its warm-up (`started` and
+// `c_begin` unused).
+template <bool PC, bool LISTED>
 __global__ void __launch_bounds__(kDirectTile)
 fir_direct_kernel(const float* __restrict__ U, long long u_stride, int hist_pad, int u_ring, int u_pos, float* __restrict__ Y, long long y_stride,
                   const double* __restrict__ taps, int N, long long T, long long started, float divisor, float post_nf,
-                  int c_begin, long long n_begin, long long n_end, const int* __restrict__ set_index) {
+                  int c_begin, long long n_begin, long long n_end, const int* __restrict__ set_index, const int2* __restrict__ warm) {
     extern __shared__ float xw[];  // [kDirectTile + N - 1]
-    const int ch = c_begin + blockIdx.y;
+    const int ch = LISTED ? warm[blockIdx.y].x : c_begin + blockIdx.y;
     if constexpr (PC) taps += (long long)set_index[ch] * N;
     const long long tile0 = n_begin + (long long)blockIdx.x * kDirectTile;
+    if constexpr (LISTED) {
+        started = warm[blockIdx.y].y;
+        n_end = min(n_end, (long long)N - 1 - started);
+        if (tile0 >= n_end) return;  // the whole CTA: this channel's warm-up ends before the tile
+    }
     const long long w0 = tile0 - (N - 1);  // call-relative index of xw[0]; >= -hist_pad
     const float* row = U + (long long)ch * u_stride;  // a ring of u_ring samples, call sample n at slot (u_pos + n) mod u_ring
     const int W = kDirectTile + N - 1;
@@ -66,27 +74,29 @@ fir_direct_kernel(const float* __restrict__ U, long long u_stride, int hist_pad,
 
 }  // namespace
 
+// listed: one CTA row per entry of fp.warm instead of per channel of [c_begin, c_end)
 int launch_fir_direct(const FirPlan& fp, const float* U, int64_t u_stride, float* Y, int64_t y_stride, int c_begin, int c_end,
-                      int64_t T, int64_t started, int64_t n_begin, int64_t n_end, cudaStream_t st) {
+                      int64_t T, int64_t started, int64_t n_begin, int64_t n_end, cudaStream_t st, bool listed = false) {
     const int N = fp.n_taps;
     const size_t smem = (size_t)(kDirectTile + N - 1) * 4;
     const bool pc = fp.set_index != nullptr;
-    auto kernel = pc ? fir_direct_kernel<true> : fir_direct_kernel<false>;
+    auto kernel = listed ? (pc ? fir_direct_kernel<true, true> : fir_direct_kernel<false, true>)
+                         : (pc ? fir_direct_kernel<true, false> : fir_direct_kernel<false, false>);
     // per device and instantiation: the opt-in is a per-device function attribute
-    static std::atomic<size_t> configured_dev[kMaxDevices][2];
-    std::atomic<size_t>& configured = configured_dev[current_device_slot()][pc];
+    static std::atomic<size_t> configured_dev[kMaxDevices][4];
+    std::atomic<size_t>& configured = configured_dev[current_device_slot()][pc + 2 * listed];
     if (smem > 48 * 1024 && smem > configured.load(std::memory_order_acquire)) {
         cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
         configured.store(smem, std::memory_order_release);
     }
     if (n_end <= n_begin) return 0;
-    const int C = c_end - c_begin;
+    const int rows = listed ? fp.n_warm : c_end - c_begin;
     const long long tiles = (n_end - n_begin + kDirectTile - 1) / kDirectTile;
-    for (int c = 0; c < C; c += 65535) {  // gridDim.y limit
-        dim3 grid((unsigned)tiles, (unsigned)std::min(65535, C - c));
+    for (int c = 0; c < rows; c += 65535) {  // gridDim.y limit
+        dim3 grid((unsigned)tiles, (unsigned)std::min(65535, rows - c));
         kernel<<<grid, kDirectTile, smem, st>>>(U, u_stride, fp.hist_pad, fp.u_ring, fp.u_pos, Y, y_stride, fp.taps, N, T, started,
-                                               fp.divisor, fp.post_nf, c_begin + c, n_begin, n_end, fp.set_index);
+                                               fp.divisor, fp.post_nf, c_begin + c, n_begin, n_end, fp.set_index, fp.warm + c);
     }
     return (int)cudaGetLastError();
 }
@@ -94,20 +104,27 @@ int launch_fir_direct(const FirPlan& fp, const float* U, int64_t u_stride, float
 int launch_fir(const FirPlan& fp, const float* U, int64_t u_stride, float* Y, int64_t y_stride, int c_begin, int c_end,
                int64_t T, int64_t started, void* stream, int* n_launches) {
     cudaStream_t st = (cudaStream_t)stream;
+    int rc = 0;
     if (fp.mode == FIR_DIRECT) {
         if (n_launches) *n_launches += 1;
-        return launch_fir_direct(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, started, 0, T, st);
-    }
-    if (fp.mode == FIR_TOEPLITZ && fp.set_index) return (int)cudaErrorInvalidValue;  // shared taps only
-    int rc = fp.mode == FIR_TOEPLITZ ? launch_fir_toeplitz(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, st, n_launches)
+        rc = launch_fir_direct(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, started, 0, T, st);
+    } else {
+        if (fp.mode == FIR_TOEPLITZ && fp.set_index) return (int)cudaErrorInvalidValue;  // shared taps only
+        rc = fp.mode == FIR_TOEPLITZ ? launch_fir_toeplitz(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, st, n_launches)
              : (fp.mode == FIR_FFT && fp.upc_fdl) ? launch_fir_upc(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, st, n_launches)
                                                   : launch_fir_fft(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, st, n_launches);
-    if (rc) return rc;
-    // Samples that still belong to the warm-up are recomputed exactly by the direct kernel.
-    const int64_t warm_end = (int64_t)fp.n_taps - 1 - started;  // call-relative
-    if (warm_end > 0) {
+        if (rc) return rc;
+        // Samples that still belong to the warm-up are recomputed exactly by the direct kernel.
+        const int64_t warm_end = (int64_t)fp.n_taps - 1 - started;  // call-relative
+        if (warm_end > 0) {
+            if (n_launches) *n_launches += 1;
+            rc = launch_fir_direct(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, started, 0, std::min<int64_t>(warm_end, T), st);
+        }
+    }
+    // ... and so are those of channels reset on their own, in every mode: their warm-up restarted at their reset.
+    if (rc == 0 && fp.n_warm > 0) {
         if (n_launches) *n_launches += 1;
-        rc = launch_fir_direct(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, started, 0, std::min<int64_t>(warm_end, T), st);
+        rc = launch_fir_direct(fp, U, u_stride, Y, y_stride, c_begin, c_end, T, 0, 0, std::min<int64_t>(fp.warm_len, T), st, true);
     }
     return rc;
 }

@@ -206,6 +206,12 @@ struct FirPlan {
     int n_xf = 0;                    // transforms in the slice (channels [c_begin, c_end) are exactly theirs)
     int xf0 = 0;                     // index of the slice's first transform in the whole table (UPC delay-line slot)
     int64_t h_stride = 0;            // float2 elements per set in H (fir_fft_spectrum_bytes() / 8)
+    // Channels reset by dspb_reset_channels that are still in their own warm-up while the node is past it at their position:
+    // {channel, samples since that channel's reset}, ascending channels, all inside [c_begin, c_end).  The direct kernel
+    // recomputes samples [0, min(T, N - 1 - started)) of each of them after the main launch; warm_len = the longest of those.
+    const int2* warm = nullptr;
+    int n_warm = 0;
+    int warm_len = 0;
 };
 // U: [C x u_ring] input rings (see FirPlan::u_ring / u_pos), u_stride = row pitch; Y: [C x T] output.
 // started = samples seen before this call.
@@ -233,5 +239,15 @@ int fir_toeplitz_max_taps();
 size_t fir_toeplitz_tiles_bytes(int n_taps);
 size_t fir_toeplitz_split_bytes(int n_taps, int channels, int64_t max_samples);
 int fir_toeplitz_prepare(const double* taps_rev_dev, int n_taps, void* tiles_dev, void* stream);
+
+// Per-channel state reset (reset.cu).  One state buffer of the graph: rows of `pitch` f32 from `base`; a listed channel's
+// slots (first + i) mod ring, i in [0, len), are zeroed (a [C x 4] state row or a reverb ring: first 0, len = ring = row).
+struct ClearDesc {
+    float* base;
+    int64_t pitch;
+    int64_t first, len, ring;
+};
+// Zeroes those slots of every (channel, descriptor) pair in one launch; descs and channels are device arrays.
+int launch_clear_rows(const ClearDesc* descs, int n_descs, const int* channels, int n_channels, void* stream);
 
 }  // namespace dspb

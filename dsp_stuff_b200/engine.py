@@ -56,7 +56,7 @@ ABI_SYMBOLS = [
     "dspb_load_graph_json", "dspb_compile", "dspb_process", "dspb_node_process", "dspb_reset_state",
     "dspb_node_get_i64", "dspb_node_port_index", "dspb_describe_plan", "dspb_profile_enable", "dspb_profile_read",
     "dspb_fold_stereo", "dspb_dup_stereo", "dspb_resample_dup_stereo", "dspb_sync", "dspb_node_set_f32_channels",
-    "dspb_node_set_taps_channels", "dspb_node_set_impulse_response_channels",
+    "dspb_node_set_taps_channels", "dspb_node_set_impulse_response_channels", "dspb_reset_channels",
 ]
 
 _lib = None
@@ -90,6 +90,7 @@ def load_library(path: Optional[str] = None):
     L.dspb_process.argtypes = [vp, vp, vp, i64, ctypes.c_int, vp]
     L.dspb_node_process.argtypes = [vp, i64, vp, vp, vp, i64, ctypes.c_int, vp]
     L.dspb_reset_state.argtypes = [vp]
+    L.dspb_reset_channels.argtypes = [vp, vp, i64]
     L.dspb_node_get_i64.argtypes = [vp, i64, cp, ctypes.POINTER(i64)]
     L.dspb_node_port_index.argtypes = [vp, i64, cp, ctypes.c_int, ctypes.POINTER(ctypes.c_int32)]
     L.dspb_profile_enable.argtypes = [vp, ctypes.c_int]
@@ -199,6 +200,12 @@ class Engine:
 
     def reset_state(self):
         self._ck(self._L.dspb_reset_state(self._h))
+
+    def reset_channels(self, channels):
+        """Resets the state of the listed channels (int32 indices) at the next process call, as if each ran alone on an engine
+        fresh from reset_state; the other channels are untouched.  Parameters and per-channel settings are kept."""
+        c = np.ascontiguousarray(channels, dtype=np.int32).reshape(-1)
+        self._ck(self._L.dspb_reset_channels(self._h, c.ctypes.data if c.size else None, c.size))
 
     def get_i64(self, node_id: int, key: str) -> int:
         v = ctypes.c_int64()

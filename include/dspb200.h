@@ -231,14 +231,37 @@ int dspb_dup_stereo(dspb_engine* e, const float* mono, float* interleaved, int64
 int dspb_resample_dup_stereo(dspb_engine* e, const float* mono, float* interleaved, int64_t n_in, int64_t n_out,
                              double target_hz, int mem_kind, void* cuda_stream, int64_t* consumed);
 
-/* Clears all per-channel state (what a fresh NodeStatic::new / restore gives). */
+/* Clears all per-channel state (what a fresh NodeStatic::new / restore gives).  Drops any pending dspb_reset_channels request. */
 int dspb_reset_state(dspb_engine* e);
+
+/* Per-channel state reset: from the next dspb_process on, every listed channel behaves as if dspb_reset_state had been
+ * called on a one-channel engine holding only that channel (same graph, same parameters, same per-channel values and
+ * impulse responses).  Unlisted channels are not touched.  channels: host pointer to n_channels indices in [0, channels).
+ * This is how a service recycles a stream slot: reset the slot, then set its per-channel values.
+ *   - Reset, for each listed channel: the [C x 4] state row of every biquad, low_pass, high_pass, envelope, gate and
+ *     signal_gen node, its reverb ring rows, its FIR input history, and its FIR warm-up (the first n_taps - 1 samples after
+ *     the reset are summed over the samples seen since, as for a fresh node, fir.rs:192-216), which may span several calls.
+ *   - Not reset: parameters, per-channel values and impulse responses, the plan; the dspb_resample_dup_stereo converter,
+ *     whose position is shared by all channels; the sub-engines of dspb_node_process (dspb_reset_state leaves those alone too).
+ *   - The call only records the request; it neither blocks nor synchronises.  Requests accumulate until the next
+ *     dspb_process, which enqueues the clear in front of its first kernel on the stream that orders it (`cuda_stream` for
+ *     DSPB_MEM_DEVICE, the engine's compute stream for the host paths), so a reset recorded between two DSPB_MEM_HOST_ASYNC
+ *     calls falls exactly between them.  Duplicate indices are allowed; resetting a channel again restarts its warm-up.
+ *   - Cost: nothing while no request is pending and no reset channel is in its warm-up.  Otherwise one clear launch for the
+ *     call after the reset, and one direct-kernel launch per FIR step (and channel range) while a reset channel is in its
+ *     warm-up.  A FIR node on the short-call (UPC) path re-primes its delay line once.
+ *   - n_channels == 0 is a no-op (channels may be NULL).  Errors, nothing recorded: DSPB_ERR_INVALID (null engine,
+ *     n_channels < 0, channels NULL with n_channels > 0, an index outside [0, channels)).
+ *   - Planning engines (device -1) accept the call; dspb_node_get_i64(e, 0, "pending_resets") counts the distinct channels
+ *     recorded and not yet consumed. */
+int dspb_reset_channels(dspb_engine* e, const int32_t* channels, int64_t n_channels);
 
 /* ---- introspection (index work that must match the reference bit-exactly) ------------------ */
 
 /* keys: "delay_samples" (reverb: ring length D, nodes/reverb.rs:58-68), "n_taps" (fir),
  *       "n_inputs" / "n_outputs" (port counts), "kernel_launches" (engine, node_id ignored:
- *       kernels launched by the last dspb_process), "n_segments" (engine: fused segments). */
+ *       kernels launched by the last dspb_process), "n_segments" (engine: fused segments),
+ *       "pending_resets" (engine: distinct channels recorded by dspb_reset_channels for the next dspb_process). */
 int dspb_node_get_i64(dspb_engine* e, int64_t node_id, const char* key, int64_t* out);
 /* Port name -> local index, as PortStorage::get_idx on a freshly built node (node.rs:74-89). */
 int dspb_node_port_index(dspb_engine* e, int64_t node_id, const char* port, int is_output, int32_t* out);
