@@ -40,9 +40,8 @@ def build(force: bool = False, verbose: bool = False) -> str:
         obj = os.path.join(bdir, os.path.splitext(src)[0] + ".o")
         cmd = [_nvcc()] + common + ["-c", os.path.join(CSRC, src), "-o", obj]
         if src == "fused_chain.cu":
+            # -fmad=false: belt and braces, parity-critical arithmetic also uses *_rn intrinsics
             cmd += ["-fmad=false", "-diag-suppress", "177"]  # 177: unused `rec` members of chains the ws kernel never takes
-            if os.environ.get("DSPB_WS_TIMING"):
-                cmd += ["-DDSPB_WS_TIMING"]  # belt and braces: parity-critical arithmetic also uses *_rn intrinsics
         if verbose:
             cmd += ["-Xptxas", "-v"]
             print(" ".join(cmd))

@@ -813,8 +813,7 @@ void Lowerer::close_fused() {
     const int S = kTile / G;
     P.n_prefetch = 0;
     for (int k = 0; k < kMaxPrefetch; k++) P.pf_buf[k] = P.pf_ring[k] = -1;
-    static const bool in_prefetch = !(getenv("DSPB_IN_PREFETCH") && atoi(getenv("DSPB_IN_PREFETCH")) == 0);
-    for (int i = 0; i < P.n_ops && in_prefetch; i++)
+    for (int i = 0; i < P.n_ops; i++)
         if (P.ops[i].code == OP_LOADG) {
             // A buffer this very program stores earlier (a source value spilled for a later step AND consumed again in
             // this one) must not be read one tile ahead: the prefetch would see the previous call's scratch.
@@ -833,8 +832,7 @@ void Lowerer::close_fused() {
             P.ops[i].aux = 1;
             break;
         }
-    static const bool ring_prefetch = !(getenv("DSPB_RING_PREFETCH") && atoi(getenv("DSPB_RING_PREFETCH")) == 0);
-    for (int i = 0; i < P.n_ops && ring_prefetch; i++)
+    for (int i = 0; i < P.n_ops; i++)
         if (P.ops[i].code == OP_COMB) {
             const Node& rn = *e.nodes[cur.ring_nodes[P.ops[i].aux & 0xff]];
             if ((rn.D & (kChunk - 1)) == 0 && rn.D >= 2 * (int64_t)S) {
@@ -1242,7 +1240,6 @@ int ensure_resources(dspb_engine* e) {
         }
         if (n.type == T_FIR && (n.fir_dirty || !n.Y.p)) {
             const int N = (int)n.taps.size();
-            const int F = 1 << e->cfg.fir_fft_log2;
             // history kept in front of a call: N-1 samples; the UPC kernel re-primes its delay line from P whole blocks
             const int upc_P = e->cfg.fir_mode == FIR_FFT ? fir_upc_partitions(N) : 0;
             n.hist_pad = (int)round_up(std::max(std::max(N - 1, 4), upc_P * kUpcBlock), 4);
@@ -1258,7 +1255,6 @@ int ensure_resources(dspb_engine* e) {
             const double* taps_host = pc ? n.fir_bank.data() : n.taps.data();
             r = n.H.alloc(K * fir_fft_spectrum_bytes(), false, e->plan_only);  // every spectrum table of the FFT kernels
             if (r) return r;
-            (void)F;
             r = n.taps_dev.alloc((size_t)K * N * 8, false, e->plan_only);
             if (r) return r;
             r = n.set_dev.alloc(pc ? (size_t)C * 4 : 0, false, e->plan_only);
@@ -2011,8 +2007,8 @@ int dspb_process(dspb_engine* e, const float* const* inputs, float* const* outpu
     for (size_t i = 0; i < n_out; i++) dout[i] = e->h_out[i]->p;
     r = prepare_channel_resets(e, e->s_cmp);  // after the previous call's kernels, before this call's first
     if (r) return r;
-    static const int host_chunks = getenv("DSPB_HOST_CHUNKS") ? std::max(1, std::min(64, atoi(getenv("DSPB_HOST_CHUNKS")))) : 16;
-    int n_chunks = host_chunks;
+    constexpr int kHostChunks = 16;  // H2D / kernels / D2H pipeline depth of a host-pointer call
+    int n_chunks = kHostChunks;
     int per = (C + n_chunks - 1) / n_chunks;
     per = (per + 31) / 32 * 32;  // keep CTA channel groups intact
     n_chunks = (C + per - 1) / per;
@@ -2237,9 +2233,6 @@ int dspb_profile_read(dspb_engine* e, double* ms_total, int64_t* rounds, int cap
     e->prof.clear();
     return (int)e->steps.size();
 }
-
-// debug aid (not part of the public header): phase timing of the warp-specialised kernel, see fused_chain.cu
-int dspb_debug_ws_timing(long long* out8, int clear) { return dspb::ws_timing_read(out8, clear != 0); }
 
 int64_t dspb_describe_plan(dspb_engine* e, char* buf, int64_t cap) {
     if (!e) return 0;

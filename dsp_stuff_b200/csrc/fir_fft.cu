@@ -44,32 +44,12 @@ struct __align__(2 * sizeof(T)) C2 {
 };
 __device__ __forceinline__ C2<double> operator+(C2<double> a, C2<double> b) { return {a.x + b.x, a.y + b.y}; }
 __device__ __forceinline__ C2<double> operator-(C2<double> a, C2<double> b) { return {a.x - b.x, a.y - b.y}; }
-// f32 complex add/sub.  Default: two scalar FADDs.  -DDSPB_FIR_FADD2 selects one packed add/sub.f32x2 instead (half the
-// issue slots of two FADDs on paper): compiled both ways the kernel has 2320 (packed) vs 2368 (scalar) SASS
-// instructions -- the packed form needs 256 MOVs to pair registers and blocks the mul+add -> FFMA contraction -- and
-// the packed ops hold the FP32 pipe for two cycles each.  Measured on B200 (config 4, 4096 x 16384): 0.456 ms scalar
-// vs 0.473 ms packed, so scalar is the default.
-__device__ __forceinline__ unsigned long long pack2(C2<float> a) {
-    return (unsigned long long)__float_as_uint(a.x) | ((unsigned long long)__float_as_uint(a.y) << 32);
-}
-__device__ __forceinline__ C2<float> unpack2(unsigned long long r) {
-    return {__uint_as_float((unsigned)r), __uint_as_float((unsigned)(r >> 32))};
-}
-#ifdef DSPB_FIR_FADD2
-__device__ __forceinline__ C2<float> operator+(C2<float> a, C2<float> b) {
-    unsigned long long d;
-    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(pack2(a)), "l"(pack2(b)));
-    return unpack2(d);
-}
-__device__ __forceinline__ C2<float> operator-(C2<float> a, C2<float> b) {
-    unsigned long long d;
-    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(pack2(a)), "l"(pack2(b)));
-    return unpack2(d);
-}
-#else
+// f32 complex add/sub as two scalar FADDs.  A packed add/sub.f32x2 (half the issue slots on paper) was slower: the
+// kernel has 2320 (packed) vs 2368 (scalar) SASS instructions -- the packed form needs 256 MOVs to pair registers and
+// blocks the mul+add -> FFMA contraction -- and the packed ops hold the FP32 pipe for two cycles each.  Measured on
+// B200 (config 4, 4096 x 16384): 0.456 ms scalar vs 0.473 ms packed.
 __device__ __forceinline__ C2<float> operator+(C2<float> a, C2<float> b) { return {a.x + b.x, a.y + b.y}; }
 __device__ __forceinline__ C2<float> operator-(C2<float> a, C2<float> b) { return {a.x - b.x, a.y - b.y}; }
-#endif
 template <typename T> __device__ __forceinline__ C2<T> cmul(C2<T> a, C2<T> w) { return {a.x * w.x - a.y * w.y, a.x * w.y + a.y * w.x}; }
 template <typename T> __device__ __forceinline__ C2<T> cmulc(C2<T> a, C2<T> w) { return {a.x * w.x + a.y * w.y, a.y * w.x - a.x * w.y}; }  // a * conj(w)
 

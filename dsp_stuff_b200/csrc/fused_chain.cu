@@ -1021,29 +1021,23 @@ fused_kernel(const __grid_constant__ Program prog, int c_begin, int c_end, long 
 // for tile i (and hand tile buffer i&1 to R), then the ops after it for tile i-1 (once R is done with it),
 // so the sequential 12-cycle-per-sample chain is hidden behind elementwise work of neighbouring tiles.
 // Hand-offs use named barriers (bar.arrive / bar.sync with the 288-thread count).
-// NR recurrence warps (one per SM sub-partition) split the CTA's channels: each R warp only gets its fair
-// share of its scheduler's issue slots next to the always-ready E warps, so two of them on different
-// sub-partitions advance the recurrences twice as fast.
-// Optional phase timing (build with -DDSPB_WS_TIMING): summed clock64 deltas of CTA 0:
-// [0] R waits for FULL  [1] R loop  [2] E pre-ops  [3] E waits for DONE  [4] E post-ops  [5] E waits EONLY
-__device__ long long g_ws_timing[8];
-constexpr int kNR = 1;
-// Measured (tests/cuda/rec_microbench.cu, DSPB_WS_TIMING): an R warp alone takes 14 cycles per step and 36-50
-// inside this kernel, but it is never the bottleneck -- the elementwise warps are (E never waits for DONE, R
-// idles ~30 % of the time waiting for FULL).  Giving R its own SM sub-partition or a second R warp changed
-// nothing, so the layout stays simple: E warps first, R warp last.
-constexpr int kWsThreads = kThreads + 32 * kNR;
-constexpr int kWsLaunchThreads = kWsThreads;
+// The one R warp serves all channels of the CTA (lane = channel).  With many channels per SM it does not bound the
+// kernel, the E warps do: measured, E never waits for DONE and R idles ~30 % of the time waiting for FULL, and a
+// second R warp splitting the channels changed nothing.  When the recurrence chain does bound the kernel (few channels
+// per SM), the XR layout below gives the R warp a sub-partition of its own.
+constexpr int kWsLaunchThreads = kThreads + 32;
 enum { BAR_FULL0 = 1, BAR_FULL1 = 2, BAR_DONE0 = 3, BAR_DONE1 = 4, BAR_EONLY = 5 };
 __device__ __forceinline__ void bar_sync(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 __device__ __forceinline__ void bar_arrive(int id, int n) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 
+// `lane` is the channel index inside the CTA (or >= G for idle lanes); `row` is its state row, read and written only
+// when `ok`.  A biquad writes back y1, y2 (.z/.w) only: the elementwise warps own x1, x2.
 template <int G, class Core>
-__device__ __forceinline__ void ws_recurrence_warp(Core core, float* tiles, const float4* st_in, float4* st_out, int lane,
-                                                   bool ch_ok, long long n_tiles, long long T, int n_ws) {
-    using Q = Geo<G>;  // `lane` is the channel index inside the CTA (or >= G for idle lanes)
+__device__ __forceinline__ void ws_recurrence_warp(Core core, float* tiles, float4* row, int lane, bool ok, long long n_tiles,
+                                                   long long T, int n_ws, bool biquad) {
+    using Q = Geo<G>;
     float4 s = make_float4(0, 0, 0, 0);
-    if (lane < G && ch_ok) s = *st_in;
+    if (ok) s = *row;
     core.load(s);
     for (long long i = 0; i < n_tiles; i++) {
         const int b = (int)(i & 1);
@@ -1058,9 +1052,11 @@ __device__ __forceinline__ void ws_recurrence_warp(Core core, float* tiles, cons
         __syncwarp();
         bar_arrive(BAR_DONE0 + b, n_ws);
     }
-    if (lane < G && ch_ok) {
+    if (ok) {
         core.save(s);
-        *st_out = s;
+        float* f = reinterpret_cast<float*>(row);
+        if (biquad) { f[2] = s.z; f[3] = s.w; }
+        else *row = s;
     }
 }
 
@@ -1086,7 +1082,7 @@ __global__ void __launch_bounds__(XR ? kXrLaunchThreads : kWsLaunchThreads, XR ?
 fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, long long T, int gc, int rec_index) {
     // gc <= G: channels this CTA really owns.  The launcher trims gc so that the grid is ONE balanced wave (every SM
     // gets the same number of channels); the CTA is launched with only gc * TPC elementwise threads + the R warp.
-    const int n_e = gc * Geo<G>::TPC, n_ws = n_e + 32 * kNR;
+    const int n_e = gc * Geo<G>::TPC, n_ws = n_e + 32;
     using Q = Geo<G>;
     extern __shared__ float4 smem4[];
     int t = threadIdx.x;  // logical index; t < n_e: elementwise thread, else R-warp thread
@@ -1116,53 +1112,24 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
     constexpr bool PC = Chain::n == 0;
     const bool rpc = PC && op_pc_col(rop) >= 0;
 
-    if (t >= n_e) {  // ---------------- R warps ----------------
-        constexpr int GP = (G + kNR - 1) / kNR;  // channels per R warp
-        const int rw = (t - n_e) >> 5, rl = t & 31;
-        const int lane = (rl < GP && rw * GP + rl < gc) ? rw * GP + rl : G;  // channel inside the CTA; G = idle lane
+    if (t >= n_e) {  // ---------------- R warp ----------------
+        const int rl = t & 31;
+        const int lane = rl < gc ? rl : G;  // channel inside the CTA; G = idle lane
         const int ch = c_begin + blockIdx.x * gc + lane;
         const bool ok = lane < G && ch < c_end;
-        const float4* sin = reinterpret_cast<const float4*>(stp) + (ok ? ch : 0);
-        float4* sout = reinterpret_cast<float4*>(stp) + (ok ? ch : 0);
+        float4* row = reinterpret_cast<float4*>(stp) + (ok ? ch : 0);
         if (rcode == OP_BIQUAD) {
             DF1Core core; core.a1 = rop.p[3]; core.a2 = rop.a2;
             if (PC && rpc && ok) core.from_row(prog.pc + op_pc_col(rop) + (long long)ch * prog.pc_stride);
-            // y1, y2 live in .z/.w; the E warps own .x/.y (x1, x2) and write them separately at the end
-            float4 s = make_float4(0, 0, 0, 0);
-            if (ok) s = *sin;
-            core.load(s);
-            using QQ = Geo<G>;
-            for (long long i = 0; i < n_tiles; i++) {
-                const int b = (int)(i & 1);
-                const long long rem = T - i * QQ::S;
-                const int valid_f4 = (int)((rem < QQ::S ? rem : QQ::S) / 4);
-#ifdef DSPB_WS_TIMING
-                long long tq0 = clock64();
-#endif
-                bar_sync(BAR_FULL0 + b, n_ws);
-#ifdef DSPB_WS_TIMING
-                long long tq1 = clock64();
-#endif
-                if (lane < G) {
-                    float4* r = reinterpret_cast<float4*>(tiles + b * (G * QQ::ROW) + lane * QQ::ROW);
-                    recurrence_row(core, r, valid_f4);
-                }
-#ifdef DSPB_WS_TIMING
-                if (blockIdx.x == 0 && t == n_e) { long long tq2 = clock64(); g_ws_timing[0] += tq1 - tq0; g_ws_timing[1] += tq2 - tq1; }
-#endif
-                __threadfence_block();
-                __syncwarp();
-                bar_arrive(BAR_DONE0 + b, n_ws);
-            }
-            if (ok) { float* f = reinterpret_cast<float*>(sout); f[2] = core.y1; f[3] = core.y2; }
+            ws_recurrence_warp<G>(core, tiles, row, lane, ok, n_tiles, T, n_ws, true);
         } else if (rcode == OP_LP1 || rcode == OP_HP1) {
             OnePoleCore core; core.r = rop.p[0];
             if (PC && rpc && ok) core.from_row(prog.pc + op_pc_col(rop) + (long long)ch * prog.pc_stride);
-            ws_recurrence_warp<G>(core, tiles, sin, sout, lane, ok, n_tiles, T, n_ws);
+            ws_recurrence_warp<G>(core, tiles, row, lane, ok, n_tiles, T, n_ws, false);
         } else {
             EnvCore core; core.ga = rop.p[0]; core.gr = rop.p[1];
             if (PC && rpc && ok) core.from_row(prog.pc + op_pc_col(rop) + (long long)ch * prog.pc_stride);
-            ws_recurrence_warp<G>(core, tiles, sin, sout, lane, ok, n_tiles, T, n_ws);
+            ws_recurrence_warp<G>(core, tiles, row, lane, ok, n_tiles, T, n_ws, false);
         }
         return;
     }
@@ -1214,20 +1181,10 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
 
     const int nt = (int)n_tiles;
     for (int i = 0; i <= nt; i++) {
-#ifdef DSPB_WS_TIMING
-        long long tb0 = clock64();
-        long long tp1 = 0, tp2 = 0;
-#endif
         // edge[] is rewritten below: from i = 2 on, the BAR_DONE sync of the previous iteration already orders
         // that behind every thread's reads (and the ring stores of tile i-2 before the loads of tile i-1)
         if (i <= 1) bar_sync(BAR_EONLY, n_e);
-#ifdef DSPB_WS_TIMING
-        if (blockIdx.x == 0 && t == 0) g_ws_timing[5] += clock64() - tb0;
-#endif
         float acc[kChunk];
-#ifdef DSPB_WS_TIMING
-        long long te0 = clock64(), te1 = te0, te2 = te0;
-#endif
         if (i < nt) {  // ---- ops before the recurrence, tile i ----
             set_tile(i);
 #pragma unroll
@@ -1235,9 +1192,6 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
             if constexpr (Chain::n > 0) run_static_range<G, Chain, 0, Chain::rec>(prog, c, acc, pf);
             else
                 for (int ip = 0; ip < rec_index; ip++) exec_op<G, true>(prog.ops[ip].code, prog.ops[ip].mode, prog.ops[ip].pre, -1, prog.ops[ip], c, acc, pf);
-#ifdef DSPB_WS_TIMING
-            tp1 = clock64();
-#endif
             // the recurrence op's own prologue and feed-forward part
             fanin_prologue(acc, Chain::n > 0 ? ((Chain::sig(Chain::rec) >> 16) & 0xff) : rop.pre, rop);
             if (rcode == OP_BIQUAD) {
@@ -1262,9 +1216,6 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
                     if (c.j == 0) { const float2 s2 = xstate[(i & 1) * 32 + c.g]; xm1 = s2.x; xm2 = s2.y; }
                     else { const float2 e = edge[t - 1]; xm2 = e.x; xm1 = e.y; }
                 }
-#ifdef DSPB_WS_TIMING
-                tp2 = clock64();
-#endif
                 float pm1 = acc[0], pm2;
                 acc[0] = add(add(mul(b0, acc[0]), mul(b1, xm1)), mul(b2, xm2));
                 pm2 = pm1; pm1 = acc[1];
@@ -1302,15 +1253,9 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
             __threadfence_block();
             bar_arrive(BAR_FULL0 + (int)(i & 1), n_ws);
         }
-#ifdef DSPB_WS_TIMING
-        te1 = clock64();
-#endif
         if (i >= 1) {  // ---- ops after the recurrence, tile i-1 ----
             const int b = (int)((i - 1) & 1);
             bar_sync(BAR_DONE0 + b, n_ws);
-#ifdef DSPB_WS_TIMING
-            te2 = clock64();
-#endif
             set_tile(i - 1);
             const float4* row = reinterpret_cast<const float4*>(tiles + b * (G * Q::ROW) + c.g * Q::ROW);
 #pragma unroll
@@ -1331,10 +1276,6 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
             else
                 for (int ip = rec_index + 1; ip < prog.n_ops; ip++) exec_op<G, true>(prog.ops[ip].code, prog.ops[ip].mode, prog.ops[ip].pre, -1, prog.ops[ip], c, acc, pf);
         }
-#ifdef DSPB_WS_TIMING
-        if (blockIdx.x == 0 && t == 0) { long long te3 = clock64(); g_ws_timing[2] += te1 - te0; g_ws_timing[3] += te2 - te1; g_ws_timing[4] += te3 - te2;
-            if (tp1) { g_ws_timing[6] += tp1 - te0; g_ws_timing[7] += tp2 - tp1; } }
-#endif
     }
     bar_sync(BAR_EONLY, n_e);
     if constexpr (Q::TPC <= 32) {
@@ -1354,7 +1295,6 @@ fused_kernel_ws(const __grid_constant__ Program prog, int c_begin, int c_end, lo
 // barriers FULL / DONE per stage and tile parity), same XR layout (R1 = physical warp 3, R2 = warp 7: both on
 // sub-partition 3, where two dependent chains interleave without slowing each other down).
 enum { BAR2_FULL = 1, BAR2_DONE = 5, BAR2_EONLY = 9 };  // FULL/DONE: + 2 * stage + parity
-constexpr int kWs2LaunchThreads = kThreads + 64;
 
 template <int G>
 struct Ws2Smem {
@@ -1389,8 +1329,8 @@ __device__ __forceinline__ void ws2_rec_loop(Core core, float* tiles, float* stp
     }
 }
 
-template <int G, bool XR>
-__global__ void __launch_bounds__(XR ? kXrLaunchThreads : kWs2LaunchThreads, XR ? 1 : 2)
+template <int G>
+__global__ void __launch_bounds__(kXrLaunchThreads, 1)
 fused_kernel_ws2(const __grid_constant__ Program prog, int c_begin, int c_end, long long T64, int r1, int r2) {
     using Q = Geo<G>;
     constexpr int n_e = kThreads, n_ws = kThreads + 32;
@@ -1402,17 +1342,13 @@ fused_kernel_ws2(const __grid_constant__ Program prog, int c_begin, int c_end, l
     const int T = (int)T64;
     const int nt = (T + Q::S - 1) / Q::S;
     int t = threadIdx.x, role = 0;  // 0 = elementwise, 1 = R1, 2 = R2
-    if constexpr (XR) {
-        const int pw = t >> 5;
-        if ((pw & 3) == 3) {
-            if (pw > 7) return;
-            role = pw == 3 ? 1 : 2;
-        } else {
-            t = (pw - (pw >> 2)) * 32 + (t & 31);
-            if (t >= n_e) return;
-        }
-    } else if (t >= n_e) {
-        role = 1 + ((t - n_e) >> 5);
+    const int pw = t >> 5;
+    if ((pw & 3) == 3) {
+        if (pw > 7) return;
+        role = pw == 3 ? 1 : 2;
+    } else {
+        t = (pw - (pw >> 2)) * 32 + (t & 31);
+        if (t >= n_e) return;
     }
     const Op& rop1 = prog.ops[r1];
     const Op& rop2 = prog.ops[r2];
@@ -1626,30 +1562,20 @@ bool ws2_rec_indices(const Program& p, int* r1, int* r2) {
     return true;
 }
 
-template <int G, bool XR>
+template <int G>
 int launch_ws2(const Program& prog, int c_begin, int c_end, int64_t T, int r1, int r2, cudaStream_t st) {
     const int smem = Ws2Smem<G>::bytes;
     static std::atomic<bool> configured_dev[kMaxDevices];
     std::atomic<bool>& configured = configured_dev[current_device_slot()];
     if (!configured.load(std::memory_order_acquire)) {
-        cudaError_t e = cudaFuncSetAttribute(fused_kernel_ws2<G, XR>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaError_t e = cudaFuncSetAttribute(fused_kernel_ws2<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return (int)e;
         configured.store(true, std::memory_order_release);
     }
     const int n_cta = (c_end - c_begin + G - 1) / G;
-    fused_kernel_ws2<G, XR><<<n_cta, XR ? kXrLaunchThreads : kWs2LaunchThreads, smem, st>>>(prog, c_begin, c_end, (long long)T, r1, r2);
+    fused_kernel_ws2<G><<<n_cta, kXrLaunchThreads, smem, st>>>(prog, c_begin, c_end, (long long)T, r1, r2);
     return (int)cudaGetLastError();
 }
-}  // namespace
-int ws_timing_read(long long* out, bool clear) {
-    cudaError_t e = cudaMemcpyFromSymbol(out, g_ws_timing, 8 * sizeof(long long));
-    if (e == cudaSuccess && clear) {
-        long long z[8] = {0};
-        e = cudaMemcpyToSymbol(g_ws_timing, z, sizeof z);
-    }
-    return (int)e;
-}
-namespace {
 int ws_smem_bytes(const Program& prog, int G) {
     const int S = kTile / G;
     bool hp = false;
@@ -1711,34 +1637,28 @@ int launch_ws(const Program& prog, int c_begin, int c_end, int64_t T, int rec_in
     }
     if (XR) {
         const int n_cta = (c_end - c_begin + G - 1) / G;
-        static bool said = false;
-        if (!said && getenv("DSPB_DEBUG")) { fprintf(stderr, "[dspb] fused_kernel_ws XR: G=%d n_cta=%d regs=%d smem=%d\n", G, n_cta, regs, smem); said = true; }
         fused_kernel_ws<G, Chain, true><<<n_cta, kXrLaunchThreads, smem, st>>>(prog, c_begin, c_end, (long long)T, G, rec_index);
         return (int)cudaGetLastError();
     }
     // Channels per CTA: G, or a smaller power of two when a channel is one warp (TPC == 32): smaller CTAs (8 channels
     // = 9 warps, 4 resident per SM) balance better and measured 0.344 ms against 0.368 ms for the config-3 chain at
     // 4096 channels.  The grid has to stay ONE wave, and the capacity that counts is not n_sm x CTAs-per-SM:
-    // measured on B200 (DSPB_GC sweep, profiles/r01s3_fused_gc_sweep.txt), CTAs are dealt evenly to the 8 GPCs
+    // measured on B200 (a sweep over gc, profiles/r01s3_fused_gc_sweep.txt), CTAs are dealt evenly to the 8 GPCs
     // and the smallest GPC has 16 SMs, so a grid runs in one wave only while n_cta / 8 <= 16 x CTAs-per-SM.
     // 293 CTAs of 14 channels (a "perfectly balanced" 2 per SM on paper) took 2.1x as long: the CTAs that did not
     // fit their GPC started when the first ones had finished (ncu: sm__cycles_active min 437 K / max 1506 K).
     int gc = G;
-    static const bool no_balance = getenv("DSPB_NO_BALANCE") != nullptr;
-    if (Geo<G>::TPC == 32 && regs > 0 && !no_balance) {
+    if (Geo<G>::TPC == 32 && regs > 0) {
         const int n = c_end - c_begin;
         for (int g = G / 2; g >= 8; g >>= 1) {
-            const int warps = g + kNR;
+            const int warps = g + 1;  // one elementwise warp per channel, and the R warp
             const int cps = std::min(65536 / (regs * 32 * warps), (227 * 1024) / (smem + 1024));
             const int n_cta = (n + g - 1) / g;
             if (cps >= 1 && (n_cta + 7) / 8 <= 16 * cps) gc = g;
         }
     }
-    if (const char* f = getenv("DSPB_GC")) { const int v = atoi(f); if (v >= 1 && v <= G && Geo<G>::TPC == 32) gc = v; }
     const int n_cta = (c_end - c_begin + gc - 1) / gc;
-    static bool said = false;
-    if (!said && getenv("DSPB_DEBUG")) { fprintf(stderr, "[dspb] fused_kernel_ws: G=%d gc=%d n_cta=%d regs=%d smem=%d\n", G, gc, n_cta, regs, smem); said = true; }
-    fused_kernel_ws<G, Chain, false><<<n_cta, gc * Geo<G>::TPC + 32 * kNR, smem, st>>>(prog, c_begin, c_end, (long long)T, gc, rec_index);
+    fused_kernel_ws<G, Chain, false><<<n_cta, gc * Geo<G>::TPC + 32, smem, st>>>(prog, c_begin, c_end, (long long)T, gc, rec_index);
     return (int)cudaGetLastError();
 }
 
@@ -1788,42 +1708,36 @@ int launch_gc(const Program& prog, int c_begin, int c_end, int64_t T, int n_stat
 
 template <int G>
 int launch_g(const Program& prog, int c_begin, int c_end, int64_t T, int n_states, cudaStream_t st) {
-    static const bool no_static = getenv("DSPB_NO_STATIC") != nullptr;
-    static const bool no_ws_env = getenv("DSPB_NO_WS") != nullptr;
     // a recurrence in scan mode has no sequential part to hide: such programs take the plain kernel
-    const bool no_ws = no_ws_env || prog.n_scan > 0;
+    const bool no_ws = prog.n_scan > 0;
     {   // two recurrences in series: pipelined over two recurrence warps
-        static const bool no_ws2 = getenv("DSPB_NO_WS2") != nullptr;
         int r1 = -1, r2 = -1;
-        if (!no_ws && !no_ws2 && G <= 16 && ws2_rec_indices(prog, &r1, &r2) && Ws2Smem<G>::bytes <= 200 * 1024) {
+        if (!no_ws && G <= 16 && ws2_rec_indices(prog, &r1, &r2) && Ws2Smem<G>::bytes <= 200 * 1024) {
             // only the chain-bound regime (one CTA per SM, one wave) has a variant: with many channels per SM the
             // elementwise work dominates and the plain kernel below is as good
-            if ((c_end - c_begin + G - 1) / G <= 128) return launch_ws2<G, true>(prog, c_begin, c_end, T, r1, r2, st);
+            if ((c_end - c_begin + G - 1) / G <= 128) return launch_ws2<G>(prog, c_begin, c_end, T, r1, r2, st);
         }
     }
     const int rec = (G <= 32 && !no_ws) ? ws_rec_index(prog) : -1;
     if (rec >= 0 && ws_smem_bytes(prog, G) <= 200 * 1024) {
         // chain-bound launches (at most one CTA per SM and one wave: n_cta <= 8 GPCs x 16 SMs) give the recurrence
         // warp a sub-partition of its own
-        static const bool no_xr = getenv("DSPB_NO_XR") != nullptr;
-        const bool xr = !no_xr && (c_end - c_begin + G - 1) / G <= 128 && prog.n_vregs == 0 && prog.n_ops <= 8;
+        const bool xr = (c_end - c_begin + G - 1) / G <= 128 && prog.n_vregs == 0 && prog.n_ops <= 8;
         if (xr) {
-            if (!no_static && chain_matches<ChainGDBR<3>>(prog)) return launch_ws<G, ChainGDBR<3>, true>(prog, c_begin, c_end, T, rec, st);
+            if (chain_matches<ChainGDBR<3>>(prog)) return launch_ws<G, ChainGDBR<3>, true>(prog, c_begin, c_end, T, rec, st);
             return launch_ws<G, ChainDynamic, true>(prog, c_begin, c_end, T, rec, st);
         }
-        if (!no_static && chain_matches<ChainGDBR<3>>(prog)) return launch_ws<G, ChainGDBR<3>, false>(prog, c_begin, c_end, T, rec, st);
-        if (!no_static && chain_matches<ChainGDBR<1>>(prog)) return launch_ws<G, ChainGDBR<1>, false>(prog, c_begin, c_end, T, rec, st);
+        if (chain_matches<ChainGDBR<3>>(prog)) return launch_ws<G, ChainGDBR<3>, false>(prog, c_begin, c_end, T, rec, st);
+        if (chain_matches<ChainGDBR<1>>(prog)) return launch_ws<G, ChainGDBR<1>, false>(prog, c_begin, c_end, T, rec, st);
         return launch_ws<G, ChainDynamic, false>(prog, c_begin, c_end, T, rec, st);
     }
-    if (!no_static) {
-        if (chain_matches<ChainGDBR<3>>(prog)) return launch_gc<G, ChainGDBR<3>>(prog, c_begin, c_end, T, n_states, st);
-        if (chain_matches<ChainGDBRScan<3>>(prog)) return launch_gc<G, ChainGDBRScan<3>>(prog, c_begin, c_end, T, n_states, st);
-        if (chain_matches<ChainGDR<3>>(prog)) return launch_gc<G, ChainGDR<3>>(prog, c_begin, c_end, T, n_states, st);
-        if (chain_matches<ChainGDR<1>>(prog)) return launch_gc<G, ChainGDR<1>>(prog, c_begin, c_end, T, n_states, st);
-        if (chain_matches<ChainBB<1>>(prog)) return launch_gc<G, ChainBB<1>>(prog, c_begin, c_end, T, n_states, st);
-        if (chain_matches<ChainLH<1>>(prog)) return launch_gc<G, ChainLH<1>>(prog, c_begin, c_end, T, n_states, st);
-        if (chain_matches<ChainCopy<1>>(prog)) return launch_gc<G, ChainCopy<1>>(prog, c_begin, c_end, T, n_states, st);
-    }
+    if (chain_matches<ChainGDBR<3>>(prog)) return launch_gc<G, ChainGDBR<3>>(prog, c_begin, c_end, T, n_states, st);
+    if (chain_matches<ChainGDBRScan<3>>(prog)) return launch_gc<G, ChainGDBRScan<3>>(prog, c_begin, c_end, T, n_states, st);
+    if (chain_matches<ChainGDR<3>>(prog)) return launch_gc<G, ChainGDR<3>>(prog, c_begin, c_end, T, n_states, st);
+    if (chain_matches<ChainGDR<1>>(prog)) return launch_gc<G, ChainGDR<1>>(prog, c_begin, c_end, T, n_states, st);
+    if (chain_matches<ChainBB<1>>(prog)) return launch_gc<G, ChainBB<1>>(prog, c_begin, c_end, T, n_states, st);
+    if (chain_matches<ChainLH<1>>(prog)) return launch_gc<G, ChainLH<1>>(prog, c_begin, c_end, T, n_states, st);
+    if (chain_matches<ChainCopy<1>>(prog)) return launch_gc<G, ChainCopy<1>>(prog, c_begin, c_end, T, n_states, st);
     return launch_gc<G, ChainDynamic>(prog, c_begin, c_end, T, n_states, st);
 }
 

@@ -171,8 +171,6 @@ int verify_const_div2(float b, float zh, float zl, unsigned long long* mismatche
 // Runs a one-recurrence probe program in exact and in scan mode on the device (noise + log sweep, 16384 samples) and
 // returns max |scan - exact| / max |exact|: the measured error that gates scan mode for one coefficient set.
 int measure_scan_error(const Op& exact_op, const ScanTab& tab, float* rel_err);
-// debug: summed clock64 phase timings of the warp-specialised kernel (only with -DDSPB_WS_TIMING)
-int ws_timing_read(long long* out8, bool clear);
 
 enum FirMode { FIR_FFT = 0, FIR_DIRECT = 1, FIR_TOEPLITZ = 2, FIR_FFT_PACKED = 3 };
 struct FirPlan {
